@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the fused warp+paste compositing path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic frame-sets.  Default workload: 8 x 1080p
 cameras into one panorama - the geometry north_star's 70 % target is quoted on - with 5 launches of 64
@@ -22,6 +22,12 @@ Rank 0 prints ONE JSON line:
 
 ``--impl reference`` times only that CPU chain (all host threads) and prints
 the same line shape with ``"impl": "reference"``.
+
+``--dump-outputs DIR`` (rank 0) writes what the timed paths computed in their last step, for comparing two builds
+output for output (the synthetic inputs are seeded, so the same arguments give the same inputs):
+``panoramas.npy`` from the timed launches (or the CPU chain with ``--impl reference``) and ``e2e_panoramas.npy``
+from the end-to-end leg.  Each is a seeded sample of pixels, ``[K, C]`` float32, with their (frame, row, column)
+in ``<name>_pixels.npy``, ``[K, 3]`` float32.
 
 With N > 1 (torchrun, one rank per GPU) the sequence shards by frame range:
 every rank composites its own batch, there is no data-path collective
@@ -51,6 +57,7 @@ WORKLOADS = {
 DEFAULT_WORKLOAD = "ns_8x1080p"
 LAUNCHES_PER_STEP = 5
 FALLBACK_HBM_GBS = 6650.0
+DUMP_PIXELS = 1 << 20   # pixels sampled per dumped output: 2 x 12 MB with their positions, two outputs < 64 MB
 
 
 def build_chain(name):
@@ -87,6 +94,24 @@ def measured_peak():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return FALLBACK_HBM_GBS, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def dump_outputs(out_dir, name, panos, seed=0):
+    """Writes a fixed, seeded sample of the pixels of ``panos`` ([F, H, W(, C)] uint8, numpy or torch on any device)
+    as ``out_dir/<name>.npy`` and their (frame, row, column) as ``out_dir/<name>_pixels.npy``, both float32."""
+    shape = tuple(int(v) for v in panos.shape[:3])
+    n = int(np.prod(shape))
+    flat = np.arange(n) if n <= DUMP_PIXELS else np.unique(np.random.default_rng(seed).integers(0, n, DUMP_PIXELS))
+    f, y, x = np.unravel_index(flat, shape)
+    if isinstance(panos, np.ndarray):
+        vals = panos[f, y, x]
+    else:
+        import torch
+        f_t, y_t, x_t = (torch.from_numpy(a).to(panos.device) for a in (f, y, x))
+        vals = panos[f_t, y_t, x_t].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, name + "_pixels.npy"), np.stack([f, y, x], axis=1).astype(np.float32))
 
 
 # ---------------------------------------------------------------------------
@@ -224,11 +249,16 @@ def run_reference(args, rank, world):
     for _ in range(args.warmup):
         for i in range(per_step):
             run(frame_sets[i % 4])
+    last = []
     t0 = time.perf_counter()
-    for _ in range(args.steps):
+    for step in range(args.steps):
         for i in range(per_step):
-            run(frame_sets[i % 4])
+            pano = run(frame_sets[i % 4])
+            if args.dump_outputs and step == args.steps - 1:
+                last.append(pano)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "panoramas", np.stack(last))
     pps = args.steps * per_step / dt
     line = {
         "impl": "reference", "metric": "panoramas_per_sec", "value": pps, "unit": "panoramas/s",
@@ -300,13 +330,16 @@ class Resident(object):
         torch.cuda.empty_cache()
 
 
-def time_resident(w, ctx, steps, warmup, launches_per_step, sampler=None):
-    """CUDA-event time of ``steps`` steps of ``launches_per_step`` launches, max over ranks."""
+def time_resident(w, ctx, steps, warmup, launches_per_step, sampler=None, clear_out=False):
+    """CUDA-event time of ``steps`` steps of ``launches_per_step`` launches, max over ranks.  ``clear_out`` zeroes the
+    output after the warm-up (untimed), so that what it holds afterwards was written by the timed launches."""
     import torch
     from multicamera_stitching_b200 import _cabi
     for _ in range(warmup):
         for _ in range(launches_per_step):
             w.launch()
+    if clear_out:
+        w.out.zero_()
     ctx.barrier()
     if sampler is not None:
         sampler.start()
@@ -604,8 +637,10 @@ def run_ours(args, rank, local_rank, world):
     # ---- kernel-resident timing ------------------------------------------------
     lps = args.launches_per_step
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    ms_total, launches = time_resident(w, ctx, args.steps, args.warmup, lps, sampler)
+    ms_total, launches = time_resident(w, ctx, args.steps, args.warmup, lps, sampler, clear_out=bool(args.dump_outputs))
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, "panoramas", w.out)   # every launch of the last step wrote w.out
     ms_step = ms_total / args.steps
     pps = world * batch * lps * args.steps / (ms_total * 1e-3)
     launch_ms = ms_total / max(launches, 1)
@@ -642,7 +677,9 @@ def run_ours(args, rank, local_rank, world):
         d = np.abs(got.astype(np.int16) - ref.astype(np.int16))
         if int(d.max()) > 1:
             raise SystemExit("bench.py: e2e panorama differs from the cv2 chain")
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
+    if args.dump_outputs:
+        host_out.zero_()   # untimed: the dump must come from the timed steps, not from the warm-up
     sampler2 = ClockSampler(local_rank)
     if rank == 0:
         sampler2.start()
@@ -660,6 +697,8 @@ def run_ours(args, rank, local_rank, world):
         sampler2.stop()
         clocks = ClockSampler.merged(sampler, sampler2)   # both timed regions
     e2e_pps = world * e2e_batch * e2e_steps / (e2e_ms * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, "e2e_panoramas", host_out)   # the last step filled every slot of the ring
     del pipe, host_frames, host_out
     # what the box's host<->device path can carry with all ranks copying at once, and the panorama rate it allows
     up_gbs, dn_gbs = host_ceiling(ctx, device)
@@ -756,6 +795,8 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="kernel experiments: skip the end-to-end leg and the extras")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra records (configs 2-5)")
     ap.add_argument("--ref-panos-per-step", type=int, default=4)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's panoramas to DIR/*.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))

@@ -1,5 +1,6 @@
 import sys, os
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import numpy as np, torch
 from helpers import synthetic_chain
 from oracle import stitcher_ref

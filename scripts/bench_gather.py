@@ -1,4 +1,6 @@
-import sys; sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import numpy as np, torch
 from helpers import synthetic_chain
 dev = torch.device('cuda', 0)

@@ -4,8 +4,9 @@
 logging module and a byte copy of the reference's ``Utils.py``) is a build output that travels with the repository
 snapshot; the reference tree itself does not.  Where that output is present, the reference class is calibrated by
 its own ``calibrate_stitcher`` with the stage homographies of the synthetic rigs and its ``stitch(images_dic)`` is
-held against the product's, bit for bit.  (Where it is absent the committed fixture tests/golden/chain_ref.npz,
-made by the same classes, carries the pin: tests/test_golden.py.)"""
+held against the product's, bit for bit.  Where it is absent (a clean checkout: the repository does not ship the
+reference) these tests skip; what remains checked against the reference there is the committed fixture
+tests/golden/chain_ref.npz (tests/test_golden.py), the panoramas of three chains, not the cases below."""
 import numpy as np
 import pytest
 

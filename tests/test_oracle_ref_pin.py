@@ -6,8 +6,11 @@ feature detector) and imports the reference's ``Utils.py`` unchanged.  Every fun
 the reference method it restates (SURVEY.md section 8 rows a1-a5, a7), on the seeded synthetic inputs of the other
 tests: same state fields, same panoramas, same match lists, bit for bit.
 
-CPU only; skipped where the reference tree is absent (the GPU box) - there the committed fixture
-``tests/golden/chain_ref.npz``, generated from the reference classes by ``scripts/make_golden.py``, carries the pin.
+CPU only.  A test that needs the reference's class is skipped where neither the reference tree nor its build output
+``oracle/_ref`` is present (a clean checkout): the repository does not ship the reference.  What runs there of it is
+the committed fixture ``tests/golden/chain_ref.npz`` (tests/test_golden.py), generated from the reference classes by
+``scripts/make_golden.py``: the panoramas and canvas geometry of three chains, not the other comparisons made here.
+The product-side halves of the fallback checks below need no reference and always run.
 """
 import os
 import pickle
@@ -20,15 +23,22 @@ from helpers import synthetic_chain
 from multicamera_stitching_b200 import synthetic
 from oracle import build_ref, stitcher_ref
 
-pytestmark = pytest.mark.skipif(not build_ref.available(), reason="reference tree not present")
 
 FIELDS = ("cachedAH", "cachedAINVH", "cachedBH", "cachedBINVH", "Bpts", "Apts", "ABSize", "x_limits", "y_limits",
           "AimgSize", "BimgSize")
 
 
 @pytest.fixture(scope="module")
-def ref():
+def ref_or_none():
+    """The reference module, or None where neither the reference tree nor oracle/_ref is present."""
     return build_ref.load()
+
+
+@pytest.fixture(scope="module")
+def ref(ref_or_none):
+    if ref_or_none is None:
+        pytest.skip("reference not present (neither the reference tree nor oracle/_ref)")
+    return ref_or_none
 
 
 def inject_homography(sb, H):
@@ -127,10 +137,12 @@ def test_stitch_pair_equals_reference(ref, super_mode, kind):
         assert want.shape == got.shape and np.array_equal(want, got)
 
 
-def test_uncalibrated_pair_returns_image_b(ref):
+def test_uncalibrated_pair_returns_image_b(ref_or_none):
+    """An uncalibrated pair hands image B back (:255-256); the reference's side is checked where it is present."""
     imageB = synthetic.make_frame(40, 50, 3, 0, 0, "noise")
     imageA = synthetic.make_frame(40, 50, 3, 1, 0, "noise")
-    assert ref.StitcherBase().stitch((imageB, imageA)) is imageB
+    if ref_or_none is not None:
+        assert ref_or_none.StitcherBase().stitch((imageB, imageA)) is imageB
     assert stitcher_ref.stitch_pair(stitcher_ref.new_state(), (imageB, imageA)) is imageB
 
 
@@ -313,6 +325,7 @@ def test_per_stage_overlays_equal_the_reference(ref, n, super_mode):
     assert got.shape == want.shape and np.array_equal(got, want)
 
 
+@pytest.mark.skipif(not build_ref.available(), reason="reference tree not present")
 def test_prebuilt_reference_runs_without_the_reference_tree(tmp_path):
     """The build output (oracle/_ref: the patched class, the logging stand-in, a byte copy of the reference's
     Utils.py) is all the GPU box has: with the reference tree out of reach, ``build_ref.load()`` falls back to it
@@ -374,24 +387,27 @@ def test_product_lifecycle_equals_reference(ref):
         assert str(a) == str(b)
 
 
-def test_product_fallbacks_equal_reference(ref):
+def test_product_fallbacks_equal_reference(ref_or_none):
     """The frame path never raises (SURVEY section 8 b): an uncalibrated chain hands the first image through
     (:255-256), a dictionary with fewer images than labels hands back the last label's image (:124-128) - the
-    product returns the very objects the reference returns, without touching a device."""
+    product returns the very objects the reference returns, without touching a device.  The product's side always
+    runs; the reference's side where it is present."""
     from multicamera_stitching_b200 import Stitcher
     images = synthetic.make_frames(3, 48, 64, 3, frame_index=0, kind="noise")
-    rs, ours = ref.Stitcher(images, super_mode=False), Stitcher(images)
-    labels = list(rs.img_labels)
-    assert rs.stitch(images) is images[labels[0]] and ours.stitch(images) is images[labels[0]]
-    short = {l: images[l] for l in labels[1:]}                     # one image missing: the last label's image comes back
-    assert rs.stitch(short) is images[labels[-1]] and ours.stitch(short) is images[labels[-1]]
-    short = {l: images[l] for l in labels[:2]}                     # the last label itself missing: both look it up
-    with pytest.raises(KeyError):
-        rs.stitch(short)
-    with pytest.raises(KeyError):
-        ours.stitch(short)
-    short = {labels[-1]: images[labels[-1]]}
-    assert rs.stitch(short) is images[labels[-1]] and ours.stitch(short) is images[labels[-1]]
-    pair_r, pair_o = rs.stitchers[0], ours.stitchers[0]
-    b, a = images[labels[0]], images[labels[1]]
-    assert pair_r.stitch((b, a)) is b and pair_o.stitch((b, a)) is b
+    ours = Stitcher(images)
+    rs = None if ref_or_none is None else ref_or_none.Stitcher(images, super_mode=False)
+    sides = [ours] if rs is None else [rs, ours]
+    labels = list(ours.img_labels)
+    if rs is not None:
+        assert list(rs.img_labels) == labels
+    for side in sides:
+        assert side.stitch(images) is images[labels[0]]
+        short = {l: images[l] for l in labels[1:]}                 # one image missing: the last label's image comes back
+        assert side.stitch(short) is images[labels[-1]]
+        short = {l: images[l] for l in labels[:2]}                 # the last label itself missing: both look it up
+        with pytest.raises(KeyError):
+            side.stitch(short)
+        short = {labels[-1]: images[labels[-1]]}
+        assert side.stitch(short) is images[labels[-1]]
+        b, a = images[labels[0]], images[labels[1]]
+        assert side.stitchers[0].stitch((b, a)) is b
