@@ -169,7 +169,7 @@ extern "C" int mcs_match_hamming_top2(const uint8_t* q, const int32_t* nq, int n
 // Layout: a CTA owns 32 queries and sweeps the train set in chunks of 128; both tiles sit in shared memory
 // with a row pitch of DIM + 1 floats (conflict-free column walks).  Thread (ty, lane) accumulates the 4 x 4
 // distances between queries 4 ty .. 4 ty + 3 and trains lane, lane + 32, lane + 64, lane + 96 of the chunk,
-// keeps a running top-2 per query (packed key: distance bits << 32 | train index, which orders
+// keeps a running top-2 per query (packed key: sqrtf(sum) bits << 32 | train index, which orders
 // non-negative floats numerically and breaks ties toward the lower index), and the 32 lanes merge by
 // shuffles at the end.
 #define L2_QB 32
@@ -235,13 +235,17 @@ mcs_match_l2_kernel(const float* __restrict__ q, const int32_t* __restrict__ nq_
                     acc[a][b] = __fadd_rn(acc[a][b], __fmul_rn(d, d));   // like the reference build: no contraction
                 }
         }
+        // Rank by the rooted distance, as cv2's batchDistance does: sqrtf maps neighbouring sums to one float
+        // (e.g. 4200782 and 4200783), and among equal distances the lower train index must win, whichever
+        // sum was smaller.
 #pragma unroll
         for (int a = 0; a < 4; ++a)
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
                 const int j = lane + 32 * b;
                 if (j < cn)
-                    top2_insert64(((unsigned long long)__float_as_uint(acc[a][b]) << 32) | (unsigned)(c0 + j), b0[a], b1[a]);
+                    top2_insert64(((unsigned long long)__float_as_uint(sqrtf(acc[a][b])) << 32) | (unsigned)(c0 + j),
+                                  b0[a], b1[a]);
             }
     }
 #pragma unroll
@@ -261,7 +265,7 @@ mcs_match_l2_kernel(const float* __restrict__ q, const int32_t* __restrict__ nq_
             const size_t o = (size_t)pair * nq_max + qidx;
             const bool valid_q = qidx < nq;
             const bool h0 = valid_q && k0 != none, h1 = valid_q && k1 != none;
-            const float d0 = sqrtf(__uint_as_float((unsigned)(k0 >> 32))), d1 = sqrtf(__uint_as_float((unsigned)(k1 >> 32)));
+            const float d0 = __uint_as_float((unsigned)(k0 >> 32)), d1 = __uint_as_float((unsigned)(k1 >> 32));
             idx2[2 * o] = h0 ? (int)(unsigned)k0 : -1;
             idx2[2 * o + 1] = h1 ? (int)(unsigned)k1 : -1;
             dist2[2 * o] = h0 ? d0 : -1.0f;
