@@ -9,7 +9,7 @@ import os
 import numpy as np
 
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
-# $MCS_B200_LIB points the binding at another build of the same library (kernel experiments)
+# $MCS_B200_LIB points the binding at another build of the same library (comparisons between builds)
 LIB_PATH = os.environ.get("MCS_B200_LIB") or os.path.join(_PKG_DIR, "libmcs_b200.so")
 
 MCS_OK = 0

@@ -69,9 +69,7 @@ struct McsTile {
 };
 static_assert(sizeof(McsTile) == 32, "McsTile must stay 32 bytes");
 
-#ifndef MCS_TILED_WARPS
 #define MCS_TILED_WARPS 8   // resampling warps of the tiled kernel; each owns two rows of a cell
-#endif
 #define MCS_CELL_W 128
 #define MCS_CELL_H (2 * MCS_TILED_WARPS)
 
@@ -98,14 +96,9 @@ static_assert(sizeof(McsTile) == 32, "McsTile must stay 32 bytes");
 #define MCS_FAST_PASS_BYTES (MCS_TILED_WARPS * 32 * 8)
 #define MCS_FAST_MAX_PASSES 2
 
-// gather-variant launch geometry (64 x 16 pixel blocks)
-#define MCS_TILE_W 64
-#define MCS_TILE_H 16
-
 #define MCS_BOX_BYTES_MAX (40 * 1024)   // per staged source box
 
 #define MCS_FRAME_BLOCK_DEFAULT 64
-#define MCS_SCHED_MAX_GRID 2047
 
 struct mcs_plan {
     int n_layers;

@@ -40,6 +40,14 @@ __device__ __forceinline__ void fixed_coords(double m0, double m3, double m6, co
 // saturate_cast<short> of the integer part of a 1/32-px coordinate
 __device__ __forceinline__ int sat16(int v) { return max(-32768, min(32767, v)); }
 
+// Some of the four bilinear taps at 1/32-px (X, Y) lies inside the layer's source (otherwise the
+// sample is BORDER_CONSTANT 0 and the layer does not touch the pixel).
+__device__ __forceinline__ bool some_tap_inside(const McsLayer& g, int X, int Y) {
+    const int sx = sat16(X >> 5), sy = sat16(Y >> 5);
+    return ((unsigned)sx < (unsigned)g.src_w || (unsigned)(sx + 1) < (unsigned)g.src_w) &&
+           ((unsigned)sy < (unsigned)g.src_h || (unsigned)(sy + 1) < (unsigned)g.src_h);
+}
+
 // 1/32-px source coordinates of pixel (xl, yl) of a layer's own canvas frame: the homography
 // recipe above for WARP layers, the plan's fixed-point map (cv2.remap with CV_16SC2 + CV_16UC1
 // maps: X = 32 * map_x + fx, Y = 32 * map_y + fy) for REMAP layers.

@@ -43,8 +43,8 @@ __device__ __forceinline__ void load_px(const uint8_t* __restrict__ p, int (&v)[
     for (int c = 0; c < C; ++c) v[c] = __ldg(p + c);
 }
 
-// Fixed-point bilinear sample of `src` at (X, Y) in 1/32 px.  `touched` reports whether any tap
-// was inside the source (used by the ownership statistics).
+// Fixed-point bilinear sample of `src` at (X, Y) in 1/32 px.  Returns whether any tap was inside
+// the source.
 template <int C>
 __device__ __forceinline__ bool sample_u8(const uint8_t* __restrict__ src, long long pitch, int src_w,
                                           int src_h, int X, int Y, int (&out)[C]) {
@@ -81,106 +81,17 @@ __device__ __forceinline__ int find_owner(const StitchArgs& a, int x, int y) {
 }
 
 // --------------------------------------------------------------------------------------------
-// Variant 1 ("gather"): one thread per 4 consecutive output pixels, source taps fetched straight
-// from global memory.  Handles every layout (any pitch / alignment / homography); it is the
-// fallback of the tiled variant, never of a CPU path.
-//
-// STATS = true turns the kernel into the ownership counter behind mcs_plan_owned_pixels.
-template <int C, bool STATS>
-__global__ void __launch_bounds__(256)
-mcs_stitch_gather_kernel(const __grid_constant__ StitchArgs a, unsigned long long* __restrict__ owned) {
-    const int x_first = blockIdx.x * MCS_TILE_W + threadIdx.x * 4;
-    const int y = blockIdx.y * MCS_TILE_H + threadIdx.y;
-    const bool inside = y < a.out_h && x_first < a.out_w;
-    if (!STATS && !inside) return;   // the counter keeps whole warps alive for its warp-level merge
-    const int frame = blockIdx.z;
-
-    int prev_owner = -2, prev_xb = 0;
-    RowBlock rb = {0.0, 0.0, 0.0};
-    uint8_t px[4 * C];
-    const int n_px = inside ? min(4, a.out_w - x_first) : 0;
-
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        int v[C];
-#pragma unroll
-        for (int c = 0; c < C; ++c) v[c] = 0;
-        const int x = x_first + i;
-        int counted = -1;   // STATS: layer this pixel is counted for
-        if (i < n_px) {
-            const int k = find_owner(a, x, y);
-            if (k >= 0) {
-                const LayerArgs& L = a.L[k];
-                const int xl = x - L.g.ox, yl = y - L.g.oy;
-                const uint8_t* src = L.src + (long long)frame * L.frame_stride;
-                bool touched = true;
-                if (L.g.kind == MCS_LAYER_COPY) {
-                    if (!STATS) load_px<C>(src + (long long)yl * L.pitch + (long long)xl * C, v);
-                } else {
-                    int X, Y;
-                    if (L.g.kind == MCS_LAYER_REMAP) {
-                        layer_coords(L.g, xl, yl, X, Y);
-                    } else {
-                        const int xb = xl & ~63;
-                        if (k != prev_owner || xb != prev_xb) {
-                            rb = row_block(L.g.mi, xb, yl);
-                            prev_owner = k;
-                            prev_xb = xb;
-                        }
-                        fixed_coords(L.g.mi[0], L.g.mi[3], L.g.mi[6], rb, xl & 63, X, Y);
-                    }
-                    if (STATS) {
-                        const int sx = max(-32768, min(32767, X >> 5)), sy = max(-32768, min(32767, Y >> 5));
-                        touched = ((unsigned)sx < (unsigned)L.g.src_w || (unsigned)(sx + 1) < (unsigned)L.g.src_w) &&
-                                  ((unsigned)sy < (unsigned)L.g.src_h || (unsigned)(sy + 1) < (unsigned)L.g.src_h);
-                    } else {
-                        sample_u8<C>(src, L.pitch, L.g.src_w, L.g.src_h, X, Y, v);
-                    }
-                }
-                if (STATS && touched) counted = k;
-            }
-        }
-        if (STATS) {   // one atomic per (warp, layer) instead of one per pixel
-            const unsigned peers = __match_any_sync(0xffffffffu, counted);
-            if (counted >= 0 && (threadIdx.y * blockDim.x + threadIdx.x) % 32 == __ffs(peers) - 1)
-                atomicAdd(owned + counted, (unsigned long long)__popc(peers));
-        }
-#pragma unroll
-        for (int c = 0; c < C; ++c) px[i * C + c] = (uint8_t)v[c];
-    }
-    if (STATS) return;
-
-    uint8_t* out = a.dst + (long long)frame * a.dst_frame_stride + (long long)y * a.dst_pitch +
-                   (long long)x_first * C;
-    const bool aligned4 = ((reinterpret_cast<uintptr_t>(out) & 3) == 0);
-    if (n_px == 4 && aligned4) {
-        uint32_t* o32 = reinterpret_cast<uint32_t*>(out);
-#pragma unroll
-        for (int wd = 0; wd < C; ++wd)
-            o32[wd] = (uint32_t)px[4 * wd] | ((uint32_t)px[4 * wd + 1] << 8) |
-                      ((uint32_t)px[4 * wd + 2] << 16) | ((uint32_t)px[4 * wd + 3] << 24);
-    } else {
-        for (int b = 0; b < n_px * C; ++b) out[b] = px[b];
-    }
-}
-
-// --------------------------------------------------------------------------------------------
-// Variant 1 as launched by mcs_stitch_u8: one thread per output pixel, consecutive lanes on
-// consecutive pixels, the frames of the launch looped INSIDE the thread.  Owner search and the
-// float64 coordinate recipe run once per pixel and launch, not once per pixel and frame; what is
-// left per frame is the twelve tap bytes (neighbouring lanes share their cache lines: a warp's 32
-// pixels read ~110 contiguous bytes per source row), the integer blend and C byte stores.  Same
-// arithmetic as sample_u8, byte loads and byte stores only: any pitch, any alignment.
-#ifndef MCS_GATHER_BX
+// Variant 1 ("gather"): one thread per output pixel, consecutive lanes on consecutive pixels, the
+// frames of the launch looped INSIDE the thread, source taps fetched straight from global memory.
+// Handles every layout (any pitch / alignment / homography); it is the fallback of the tiled
+// variant, never of a CPU path.  Owner search and the float64 coordinate recipe run once per pixel
+// and launch, not once per pixel and frame; what is left per frame is the twelve tap bytes
+// (neighbouring lanes share their cache lines: a warp's 32 pixels read ~110 contiguous bytes per
+// source row), the integer blend and C byte stores.  Same arithmetic as sample_u8, byte loads and
+// byte stores only: any pitch, any alignment.
 #define MCS_GATHER_BX 64
 #define MCS_GATHER_BY 4
-#endif
-#ifndef MCS_GATHER_FRAMES
 #define MCS_GATHER_FRAMES 16   // frames per thread (grid.z covers the rest)
-#endif
-#ifndef MCS_GATHER_UNROLL
-#define MCS_GATHER_UNROLL 1
-#endif
 
 // WORDS: every source base, pitch and frame stride is a multiple of 4 bytes (checked by the launcher).  A pixel
 // whose four taps are inside the source, with another source row below them, then fetches its taps as aligned
@@ -257,8 +168,7 @@ mcs_stitch_gather_frames_kernel(const __grid_constant__ StitchArgs a) {
         }
         return;
     }
-    constexpr int kUnroll = MCS_GATHER_UNROLL;
-#pragma unroll kUnroll
+#pragma unroll 1
     for (int f = 0; f < n_fr; ++f, r0 += fs, out += a.dst_frame_stride) {
         int p00[C], p01[C], p10[C], p11[C];
 #pragma unroll
@@ -271,6 +181,29 @@ mcs_stitch_gather_frames_kernel(const __grid_constant__ StitchArgs a) {
         for (int c = 0; c < C; ++c)
             out[c] = (uint8_t)((w00 * p00[c] + w01 * p01[c] + w10 * p10[c] + w11 * p11[c] + 16384) >> 15);
     }
+}
+
+// The ownership counter behind mcs_plan_owned_pixels: per layer, the output pixels it owns and
+// samples from its source (COPY layers: every one; otherwise some tap must be inside the source).
+// Blocks of 32 x 16 pixels; whole warps stay alive for the warp-level merge.
+__global__ void __launch_bounds__(512)
+mcs_owned_pixels_kernel(const __grid_constant__ StitchArgs a, unsigned long long* __restrict__ owned) {
+    const int x = blockIdx.x * 32 + threadIdx.x, y = blockIdx.y * 16 + threadIdx.y;
+    const int k = x < a.out_w && y < a.out_h ? find_owner(a, x, y) : -1;
+    int counted = -1;   // layer this pixel is counted for
+    if (k >= 0) {
+        const McsLayer& g = a.L[k].g;
+        bool touched = true;
+        if (g.kind != MCS_LAYER_COPY) {
+            int X, Y;
+            layer_coords(g, x - g.ox, y - g.oy, X, Y);
+            touched = some_tap_inside(g, X, Y);
+        }
+        if (touched) counted = k;
+    }
+    // one atomic per (warp, layer) instead of one per pixel
+    const unsigned peers = __match_any_sync(0xffffffffu, counted);
+    if (counted >= 0 && (int)threadIdx.x == __ffs(peers) - 1) atomicAdd(owned + counted, (unsigned long long)__popc(peers));
 }
 
 // --------------------------------------------------------------------------------------------
@@ -395,9 +328,7 @@ mcs_feather_table_kernel(const __grid_constant__ StitchArgs a, const int4* __res
                 Y = yl * 32;
             } else {
                 layer_coords(g, xl, yl, X, Y);
-                const int sx = sat16(X >> 5), sy = sat16(Y >> 5);
-                touched = ((unsigned)sx < (unsigned)g.src_w || (unsigned)(sx + 1) < (unsigned)g.src_w) &&
-                          ((unsigned)sy < (unsigned)g.src_h || (unsigned)(sy + 1) < (unsigned)g.src_h);
+                touched = some_tap_inside(g, X, Y);
             }
             if (k == m || touched) band_ent[(size_t)n++ * total + i] = make_int4(X, Y, k, d);
         }
@@ -487,21 +418,6 @@ static cudaError_t launch_gather_frames(const mcs_plan* plan, const StitchArgs& 
     return cudaGetLastError();
 }
 
-template <bool STATS>
-static cudaError_t launch_gather(const mcs_plan* plan, const StitchArgs& a, unsigned long long* owned,
-                                 cudaStream_t stream) {
-    dim3 block(MCS_TILE_W / 4, MCS_TILE_H, 1);
-    dim3 grid((plan->out_w + MCS_TILE_W - 1) / MCS_TILE_W, (plan->out_h + MCS_TILE_H - 1) / MCS_TILE_H,
-              a.n_frames);
-    switch (plan->channels) {
-        case 1: mcs_stitch_gather_kernel<1, STATS><<<grid, block, 0, stream>>>(a, owned); break;
-        case 3: mcs_stitch_gather_kernel<3, STATS><<<grid, block, 0, stream>>>(a, owned); break;
-        default: mcs_stitch_gather_kernel<4, STATS><<<grid, block, 0, stream>>>(a, owned); break;
-    }
-    mcs_count_launch(1);
-    return cudaGetLastError();
-}
-
 extern "C" int mcs_stitch_u8(const mcs_plan* plan_c, const uint8_t* const* src,
                              const int64_t* src_pitch_bytes, const int64_t* src_frame_stride,
                              int n_frames, uint8_t* dst, int64_t dst_pitch_bytes,
@@ -537,10 +453,7 @@ extern "C" int mcs_stitch_u8(const mcs_plan* plan_c, const uint8_t* const* src,
     } else {
         fill_args(plan, a, src, src_pitch_bytes, src_frame_stride, n_frames, dst, dst_pitch_bytes,
                   dst_frame_stride);
-        if (getenv("MCS_GATHER_LEGACY"))   // the four-pixels-per-thread, frame-per-CTA form (experiments)
-            MCS_CHECK_CUDA(launch_gather<false>(plan, a, nullptr, stream));
-        else
-            MCS_CHECK_CUDA(launch_gather_frames(plan, a, stream));
+        MCS_CHECK_CUDA(launch_gather_frames(plan, a, stream));
         plan->last_variant = 1;
     }
     if (plan->band_fused && plan->last_variant == 2) {
@@ -592,7 +505,10 @@ extern "C" int mcs_plan_owned_pixels(const mcs_plan* plan, int64_t* owned_host, 
     if (e == cudaSuccess && plan->out_w > 0 && plan->out_h > 0) {
         StitchArgs a;
         fill_args(plan, a, nullptr, nullptr, nullptr, 1, nullptr, 0, 0);
-        e = launch_gather<true>(plan, a, d, stream);
+        const dim3 grid((plan->out_w + 31) / 32, (plan->out_h + 15) / 16, 1);
+        mcs_owned_pixels_kernel<<<grid, dim3(32, 16, 1), 0, stream>>>(a, d);
+        mcs_count_launch(1);
+        e = cudaGetLastError();
     }
     unsigned long long h[MCS_MAX_LAYERS];
     if (e == cudaSuccess) e = cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, stream);

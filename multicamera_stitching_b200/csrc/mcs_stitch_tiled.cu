@@ -35,22 +35,13 @@
 #include <cuda.h>   // CUtensorMap
 #include <string.h>
 #include <stdlib.h>
-#include <vector>
 
 #define TILED_WARPS MCS_TILED_WARPS
 #define TILED_THREADS (32 * TILED_WARPS)
-#ifndef TILED_MIN_CTAS
 #define TILED_MIN_CTAS 2
-#endif
-#ifndef TILED_PX_BATCH
-#define TILED_PX_BATCH 4   // pixels whose loads are issued before the first store (1, 2, 4, 8)
-#endif
-#ifndef TILED_SMEM_BUDGET_KB
-#define TILED_SMEM_BUDGET_KB (TILED_MIN_CTAS == 2 ? 113 : 73)
-#endif
-#ifndef TILED_MAX_STAGES
+#define TILED_PX_BATCH 4   // pixels whose loads are issued before the first store
+#define TILED_SMEM_BUDGET_KB 113   // per CTA, so that TILED_MIN_CTAS CTAs fit an SM
 #define TILED_MAX_STAGES 8
-#endif
 #define TILED_LOOKAHEAD_SLACK 2   // boxes are issued `stages - TILED_LOOKAHEAD_SLACK` units ahead
 
 struct TiledArgs {
@@ -91,7 +82,6 @@ struct TiledArgs {
     const uint8_t* fast;
     int fast_stride;
     int fast_passes;
-    unsigned long long* timeline;       // experiments (-DTILED_TIMELINE): per CTA 8 x globaltimer, see the kernel
     int use_fast;                       // 0: this launch's output alignment rules the group path out; FAST
                                         // tiles are then resampled through their per-pixel descriptors
     // feather mode, fused form: BAND tiles (tiles [0, class_first[1])) blend with up to MCS_BAND_MAX_OVERLAYS outer
@@ -100,7 +90,6 @@ struct TiledArgs {
     const uint32_t* band_desc;          // [n_band][MCS_BAND_MAX_OVERLAYS][2048] overlay descriptors
     int feather_log2;
     int ov_bytes;                       // shared-memory bytes of the overlay-descriptor buffer (0: no BAND tiles)
-    int band_every, band_zone_end;      // sweep order of the BAND tiles, see decode_chunk
 };
 
 // ---- PTX wrappers ----------------------------------------------------------------------------
@@ -304,7 +293,6 @@ __device__ __forceinline__ void issuer_init(SchedMem* sm, Issuer& c, bool writer
 // resampled tiles (FAST, WARP: bound by the SM) evenly with the COPY and ZERO tiles (bound by DRAM): with the
 // classes one after the other every CTA is in the same regime at the same time and the launch costs the sum of
 // a compute-bound and a memory-bound phase; interleaved, the copies fill the DRAM time the resampling leaves idle.
-template <bool BANDS>
 __device__ __forceinline__ void decode_chunk(const TiledArgs& a, int id, int& blk, int& t, int& f0, int& f1) {
     blk = a.n_blocks > 1 ? id / a.chunks_per_block : 0;
     const int p = id - blk * a.chunks_per_block;
@@ -329,13 +317,6 @@ __device__ __forceinline__ void decode_chunk(const TiledArgs& a, int id, int& bl
     }
     if (j < a.split_first) {
         t = j;
-        if (BANDS && j < a.band_zone_end) {
-            // BAND tiles (the first tiles of the table) are spread over the sweep, one after every band_every - 1 other
-            // resampled tiles: with all of them up front every CTA runs its slowest, most latency-bound units at the
-            // same time; spread out, a CTA in a BAND chunk shares its SM with one in an ordinary chunk
-            const int g = j / a.band_every;
-            t = j - g * a.band_every == a.band_every - 1 ? g : a.class_first[1] + (j - g);
-        }
     } else {
         const int q = (j - a.split_first) / a.split, part = (j - a.split_first) - q * a.split;
         t = a.split_first + q;
@@ -352,7 +333,6 @@ __device__ __forceinline__ int tile_class(const TiledArgs& a, int t) {
 // Make sure sequence numbers below `upto` are published (or the end marker is).  Scheduler thread.  One claim
 // is kept in flight: the atomic is issued when the previous claim is published and its result read at the
 // next call, a chunk later, so the round trip to the counter is not on the thread's critical path.
-template <bool BANDS>
 __device__ __forceinline__ void sched_ensure(const TiledArgs& a, SchedMem* sm, Issuer& c, int upto) {
     while (!c.ended && c.claimed < upto) {
         unsigned g0;
@@ -365,7 +345,7 @@ __device__ __forceinline__ void sched_ensure(const TiledArgs& a, SchedMem* sm, I
         for (int i = 0; i < a.claim && !c.ended; ++i) {
             const bool more = g0 + (unsigned)i < (unsigned)a.n_chunks;
             int4 e = make_int4(-1, 0, 0, 0);
-            if (more) decode_chunk<BANDS>(a, (int)(g0 + (unsigned)i), e.y, e.x, e.z, e.w);
+            if (more) decode_chunk(a, (int)(g0 + (unsigned)i), e.y, e.x, e.z, e.w);
             sm->chunk[c.claimed % TILED_QD] = e;
             ++c.claimed;
             c.ended = more ? 0 : 1;
@@ -401,7 +381,7 @@ __device__ __forceinline__ void issuer_step(const TiledArgs& a, SchedMem* sm, Is
         // through a run of ZERO chunks the issuer only keeps pace with the consumers: claiming ahead there
         // would just take cheap chunks away from CTAs that have nothing else left
         if (kn > k_cons + (c.zero ? 1 : TILED_SCHED_LEAD)) return;
-        sched_ensure<BANDS>(a, sm, c, kn + 1);
+        sched_ensure(a, sm, c, kn + 1);
         if (kn >= c.claimed) return;                 // past the end marker
         const int4 e = sm->chunk[kn % TILED_QD];
         if (e.x < 0) return;
@@ -431,10 +411,6 @@ __device__ __forceinline__ void issuer_step(const TiledArgs& a, SchedMem* sm, Is
         if (BANDS && INBAND) {
             sm->nl = 1 + ((rec.w >> 24) & 15);
             sm->li0 = (rec.w >> 28) & 1;   // zero-base BAND tile: no box of the owner, the unit starts at its first overlay
-#if defined(TILED_BAND_ABL) && TILED_BAND_ABL == 2   // ablation (wrong output): BAND tiles without their overlays
-            sm->nl = 1;
-            sm->li0 = 0;
-#endif
             sm->li = sm->li0;
             if ((rec.w >> 24) & 15) {   // BAND tile: the records of its overlay boxes
 #pragma unroll
@@ -469,12 +445,8 @@ __device__ __forceinline__ void issuer_step(const TiledArgs& a, SchedMem* sm, Is
         }
     }
     mbar_wait(s_empty + 8 * c.slot, c.phase ^ 1, __LINE__);   // first trip round the ring: passes at once
-#ifdef TILED_ABL_NOTMA   // ablation: the box is never loaded, consumers resample stale shared memory
-    mbar_arrive(s_full + 8 * c.slot);
-#else
     mbar_expect_tx(s_full + 8 * c.slot, bytes);
     tma_load_3d(s_base + c.slot * a.box_bytes, &a.tmap[layer], bx, by, c.frame0 + c.f, s_full + 8 * c.slot);
-#endif
     if (BANDS && INBAND) {
         if (++li == sm->nl) {
             li = sm->li0;
@@ -618,10 +590,6 @@ __device__ __forceinline__ RowOut row_split(uint32_t s_first, uint32_t g_first, 
 __device__ __forceinline__ void write_out(const RowOut& r0, const RowOut& r1, bool ragged, uint8_t* frame) {
     const uint4 v0 = lds128(r0.s_chunk);
     const uint4 v1 = lds128(r1.s_chunk);
-#ifdef TILED_ABL_NOSTORE   // ablation (benchmark experiments only): keep the loads, drop the global stores
-    if (v0.x == 0x12345678u && v1.y == 0x9abcdef0u) frame[r0.g_byte] = 1;
-    return;
-#endif
     if (r0.do_chunk) MCS_STG128(reinterpret_cast<uint4*>(frame + r0.g_chunk), v0);
     if (r1.do_chunk) MCS_STG128(reinterpret_cast<uint4*>(frame + r1.g_chunk), v1);
     if (ragged) {
@@ -748,9 +716,6 @@ __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d
                 const uint32_t w = lds32(sm.ov + (uint32_t)o * (MCS_CELL_W * MCS_CELL_H * 4) + ((j * TILED_WARPS + warp) * 32 + lane) * 4);
                 if (__any_sync(0xffffffffu, (w >> 26) != 0u)) ov_slots |= 1u << (8 * o + j);
             }
-#if defined(TILED_BAND_ABL) && TILED_BAND_ABL == 1   // ablation (wrong output): overlay boxes staged, nothing blended
-        ov_slots = 0;
-#endif
     }
     constexpr int OUT_PITCH = MCS_CELL_W * C + 16;
     const int stages = a.stages;
@@ -805,11 +770,7 @@ __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d
         } else {
         mbar_wait(sm.full + 8 * ring.slot, ring.phase, __LINE__);
         const uint32_t box = order_after_wait(sm.base + ring.slot * a.box_bytes);
-#ifdef TILED_ABL_NOCOMPUTE   // ablation: no resampling, staging rows keep whatever they hold
-        if (false) {
-#else
         if (groups == 0xffu) {
-#endif
             // All tap loads and arithmetic of a batch of pixels come before its first staging
             // store: ptxas cannot prove that a store does not alias a later load, so stores in
             // between would serialise the pixels' (long) dependency chains.
@@ -825,7 +786,6 @@ __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d
                 }
             }
         } else {
-#ifndef TILED_ABL_NOCOMPUTE
 #pragma unroll 1
             for (int jj = 0; jj < 4; ++jj) {   // pairs (row 0, row 1) of one column group
                 if (!(groups & (0x11u << jj))) continue;
@@ -838,7 +798,6 @@ __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d
                 stage_px<C>(o16_0 + g, o8_0 + g, t0);
                 stage_px<C>(o16_1 + g, o8_1 + g, t1);
             }
-#endif
         }
         __syncwarp();   // every lane has consumed its box reads and staged its pixels
         if (lane == 0) mbar_arrive(sm.empty + 8 * ring.slot);
@@ -1071,18 +1030,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
     asm volatile("" : "+r"(sm.base), "+r"(sm.full), "+r"(sm.empty), "+r"(sm.out));
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-#ifdef TILED_TIMELINE
-#define TILED_STAMP(i_)                                                                        \
-    if (tid == 0 && a.timeline) {                                                              \
-        unsigned long long now_;                                                               \
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now_));                               \
-        a.timeline[(size_t)blockIdx.x * 8 + (i_)] = now_;                                      \
-    }
-    int stamped_cls = -1;
-#else
-#define TILED_STAMP(i_)
-#endif
-    TILED_STAMP(0)
     Issuer issuer;
     issuer_init(sm.issuer, issuer, tid == 0);
     if (tid == 0) {
@@ -1105,7 +1052,7 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
 
     if (tid == 0) {
         // the first chunks, the record of the very first one, the first boxes
-        sched_ensure<BANDS>(a, sm.issuer, issuer, 2);
+        sched_ensure(a, sm.issuer, issuer, 2);
         const int4 e0 = sm.issuer->chunk[0];
         if (e0.x >= 0) prefetch_chunk(a, sm, 0, e0);
         // (BAND-aware: the prologue may enter chunk 0 whatever it is, but not run ahead into a BAND chunk 1 - the
@@ -1117,14 +1064,13 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
     RingPos ring{0, 0u, 0};
     if (BANDS && lane == 0) sts32(sm.ov + a.ov_bytes + 16 + 4 * warp, 0u);   // BAND chunks this warp has processed (phase of the overlay buffer's barriers; own warp only)
     const uint32_t s_published = smem_u32(&sm.issuer->published), s_ids = smem_u32(&sm.issuer->chunk[0]);
-    TILED_STAMP(1)
     for (int k_cons = 0;; ++k_cons) {
         // ---- chunk record: start the copy of the next chunk's, wait for this chunk's ----
         const int cb = k_cons & 1;
         const uint32_t rec = sm.dbuf + cb * TILED_DESC_BUF_BYTES;
         const uint32_t rec_release = sm.dbar + 16 + 8 * cb;
         if (tid == 0) {
-            sched_ensure<BANDS>(a, sm.issuer, issuer, k_cons + 2);
+            sched_ensure(a, sm.issuer, issuer, k_cons + 2);
             int4 e2 = make_int4(-1, 0, 0, 0);
             if (k_cons + 1 < issuer.claimed) e2 = sm.issuer->chunk[(k_cons + 1) % TILED_QD];
             if (e2.x >= 0) {
@@ -1144,9 +1090,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
         mbar_wait(sm.dbar + 8 * cb, (uint32_t)((k_cons >> 1) & 1), __LINE__);
         const uint4 info = lds128(sm.dbar + 32 + 16 * cb);
         const int blk = (int)info.x, f0 = (int)info.y, f1 = (int)info.z;
-#ifdef TILED_ABL_NODESC
-        const int t = id;
-#endif
         McsTile tile;
         {
             const uint4 q0 = lds128(rec), q1 = lds128(rec + 16);
@@ -1162,12 +1105,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             tile.by = (int)q1.z;
             tile.reserved = (int)q1.w;
         }
-#ifdef TILED_TIMELINE
-        if (tile.cls != stamped_cls) {   // first chunk of each class: FAST 2, WARP 3, COPY 4, ZERO 5
-            stamped_cls = tile.cls;
-            TILED_STAMP(2 + (MCS_N_CLASSES - 1 - tile.cls))
-        }
-#endif
         const int c0 = tile.c0, c1 = tile.c1, h = tile.h;
         const int nbytes = (c1 - c0) * C;
         const int n_fr = f1 - f0;
@@ -1262,9 +1199,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             mbar_wait(ov_full, (uint32_t)(band_seq & 1), __LINE__);
             __syncwarp();
             if (lane == 0) sts32(ov_full + 16 + 4 * warp, (uint32_t)(band_seq + 1));
-#if defined(TILED_BAND_ABL) && TILED_BAND_ABL == 2
-            n_ov = 0;
-#endif
         }
         if (C == 3 && tile.cls == MCS_TILE_FAST && a.use_fast) {
             // ---- FAST cell: this thread's two group descriptors and its share of the warp's general list ----
@@ -1303,13 +1237,7 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             const uint32_t dp = rec + MCS_FAST_HEADER_BYTES + (warp * 32 + lane) * 4;
             uint32_t w[8];
 #pragma unroll
-#ifdef TILED_ABL_NODESC   // ablation: no descriptor loads (wrong output)
-            for (int j = 0; j < 8; ++j)
-                w[j] = (uint32_t)((lane + 32 * (j & 3)) * 3 + (warp + 8 * (j >> 2)) * 512) | ((uint32_t)((lane + j) & 31) << 16) |
-                       ((uint32_t)((lane * 3 + t) & 31) << 21);
-#else
             for (int j = 0; j < 8; ++j) w[j] = lds32(dp + j * (TILED_WARPS * 32 * 4));
-#endif
             __syncwarp();
             if (lane == 0) mbar_arrive(rec_release);
 #pragma unroll
@@ -1321,15 +1249,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             const int row = warp + TILED_WARPS * (j >> 2), g0c = 32 * (j & 3);
             if (row < h && g0c < c1 && g0c + 32 > c0) groups |= 1u << j;
         }
-#ifdef TILED_ABL_W0HALF   // ablation (wrong output): warp 0 resamples only its first row
-        if (warp == 0) groups &= 0x0fu;
-#endif
-#ifdef TILED_ABL_W0NONE   // ablation (wrong output): warp 0 resamples nothing
-        if (warp == 0) groups = 0u;
-#endif
-#ifdef TILED_ABL_ALLHALF  // ablation (wrong output): every warp resamples only its first row
-        groups &= 0x0fu;
-#endif
         // the common box pitch of this channel count at compile time (128 columns at about unit scale), any other at run time
         constexpr int SP_MAIN = C == 1 ? 256 : C == 3 ? 512 : 640;
 #define MCS_WARP_FRAMES(SP_, ISS_, BAND_)                                                                           \
@@ -1346,7 +1265,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
         }
 #undef MCS_WARP_FRAMES
     }
-    TILED_STAMP(7)
     // every CTA ends on a claim past the last chunk; the last CTA out rewinds the counters for the next launch
     if (tid == 0) {
         __threadfence();
@@ -1379,8 +1297,6 @@ static EncodeTiledFn get_encode_fn() {
 
 // Overlay-descriptor buffer of the BAND tiles (feather mode, fused form); 0 when the plan has none.
 static size_t tiled_ov_bytes(const mcs_plan* plan) {
-    static const bool force = getenv("MCS_TILED_FORCE_BANDS") != nullptr;   // experiments: the BAND-aware instantiation on any plan
-    if (force) return (size_t)MCS_BAND_MAX_OVERLAYS * MCS_CELL_W * MCS_CELL_H * 4;
     return plan->band_fused && plan->n_band > 0 ? (size_t)plan->band_max_ov * MCS_CELL_W * MCS_CELL_H * 4 : 0;
 }
 
@@ -1513,12 +1429,10 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
     // split the last resampled tiles of the sweep (about two per CTA) into four chunks each
     a.split_end = plan->class_first[MCS_SEG(MCS_TILE_COPY)];   // BAND, FAST and WARP tiles are the resampled ones
     a.split = fb >= 16 ? 4 : 1;
-    int split_tiles = 2 * (int)grid;
+    const int split_tiles = 2 * (int)grid;
     {
-        const char* env = getenv("MCS_TILED_SPLIT");         // experiments: split factor (0 / 1 = no split)
+        const char* env = getenv("MCS_TILED_SPLIT");   // tests: split factor (0 / 1 = no split)
         if (env) a.split = atoi(env) > 1 && fb >= atoi(env) ? atoi(env) : 1;
-        const char* env2 = getenv("MCS_TILED_SPLIT_TILES");  // experiments: split tiles per CTA
-        if (env2) split_tiles = atoi(env2) * (int)grid;
     }
     // A last frame block shorter than the split factor would cut its split tiles into chunks WITHOUT frames.  The box
     // issuer spends one of its calls on stepping over such a chunk and its consumers make none in it, so every one of
@@ -1534,8 +1448,6 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
         if (a.light_every < 2) a.light_every = 2;
         int zone = n_light < n_heavy / (a.light_every - 1) ? n_light : n_heavy / (a.light_every - 1);   // light tiles placed
         a.light_end = zone * a.light_every;
-        const char* env = getenv("MCS_TILED_INTERLEAVE");   // experiments: 0 = class after class
-        if (env && atoi(env) == 0) a.light_end = 0;
         a.heavy_end = n_heavy + a.light_end / a.light_every;
     }
     if ((long long)a.n_blocks * a.chunks_per_block >= (1ll << 30)) {
@@ -1551,8 +1463,6 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
         const long long fair = a.n_chunks / (4 * grid);
         if (claim > fair) claim = (int)fair;
         a.claim = claim < 1 ? 1 : claim > 8 ? 8 : claim;
-        const char* env = getenv("MCS_TILED_CLAIM");   // experiments
-        if (env && atoi(env) >= 1 && atoi(env) <= 8) a.claim = atoi(env);
     }
     a.work = plan->d_work;
     for (int c = 0; c <= MCS_N_CLASSES; ++c) a.class_first[c] = plan->class_first[c];
@@ -1560,16 +1470,6 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
     a.band_desc = plan->d_band_desc;
     a.feather_log2 = plan->feather_log2;
     a.ov_bytes = (int)tiled_ov_bytes(plan);
-    {
-        const int n_band = plan->class_first[1];
-        a.band_every = n_band > 0 ? a.split_first / n_band : 0;
-        // measured (8 x 1080p, F = 8): 4.88 ms per step spread against 4.78 ms with the BAND tiles first, so the
-        // spread order is an experiment ($MCS_TILED_BAND_SPREAD=1) and a test of the issuer's entry rule
-        const char* env = getenv("MCS_TILED_BAND_SPREAD");
-        if (!(env && atoi(env) == 1)) a.band_every = 0;
-        if (a.band_every < 2) a.band_every = 0;
-        a.band_zone_end = n_band * a.band_every;
-    }
     a.fast = plan->d_fast;
     a.fast_stride = plan->fast_stride;
     a.fast_passes = plan->fast_passes;
@@ -1577,27 +1477,7 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
     // output rows: every output row of every frame must start on a 4-byte boundary
     a.use_fast = plan->d_fast != nullptr && (reinterpret_cast<uintptr_t>(dst) & 3) == 0 && (dst_pitch & 3) == 0 &&
                  (n_frames == 1 || (dst_frame_stride & 3) == 0);
-#ifdef TILED_TIMELINE
-    static unsigned long long* d_timeline = nullptr;
-    const char* tl_path = getenv("MCS_TILED_TIMELINE");
-    if (tl_path && !d_timeline) cudaMalloc(&d_timeline, sizeof(unsigned long long) * 8 * (MCS_SCHED_MAX_GRID + 1));
-    if (tl_path) cudaMemsetAsync(d_timeline, 0, sizeof(unsigned long long) * 8 * (size_t)grid, stream);
-    a.timeline = tl_path ? d_timeline : nullptr;
-#endif
     kern<<<(unsigned)grid, TILED_THREADS, smem, stream>>>(a);
-#ifdef TILED_TIMELINE
-    if (tl_path) {   // debugging aid: synchronous dump of the last launch
-        std::vector<unsigned long long> h(8 * (size_t)grid);
-        cudaMemcpy(h.data(), d_timeline, sizeof(unsigned long long) * h.size(), cudaMemcpyDeviceToHost);
-        if (FILE* f = fopen(tl_path, "w")) {
-            for (long long b = 0; b < grid; ++b) {
-                for (int i = 0; i < 8; ++i) fprintf(f, "%llu ", h[8 * b + i]);
-                fprintf(f, "\n");
-            }
-            fclose(f);
-        }
-    }
-#endif
     mcs_count_launch(1);
     MCS_CHECK_CUDA(cudaGetLastError());
     return MCS_OK;

@@ -477,7 +477,7 @@ void mcs_plan_build_tiles(mcs_plan* plan) {
     for (int k = 0; k < MCS_MAX_LAYERS; ++k) maps.wmap[k] = plan->d_wmap[k];
     bool fused = false;
     {
-        const char* env = getenv("MCS_TILED_BAND");   // "0": keep the two-pass band path (tests, experiments)
+        const char* env = getenv("MCS_TILED_BAND");   // "0": keep the two-pass band path (tests)
         const bool want = (plan->feather_log2 > 0 || plan->blend_custom) && plan->feather_log2 <= MCS_BAND_MAX_LOG2 && plan->n_layers > 1 &&
                           !(env && atoi(env) == 0);
         if (want) {
@@ -597,7 +597,7 @@ void mcs_plan_build_tiles(mcs_plan* plan) {
         // box pitch a multiple of 128 bytes (32 banks): when the lanes of a warp straddle two
         // source rows their words still fall into disjoint shared-memory banks
         {
-            const char* env = getenv("MCS_TILED_PITCH_WORDS");   // experiments: box pitch granularity
+            const char* env = getenv("MCS_TILED_PITCH_WORDS");   // tests: box pitch granularity
             const int g = env && atoi(env) >= 4 ? atoi(env) : 32;
             bw4[k] = (bw4[k] + g - 1) / g * g;
         }
@@ -615,17 +615,10 @@ void mcs_plan_build_tiles(mcs_plan* plan) {
     for (int i = 0; i < n_tiles; ++i) tiles[i].reserved = i;   // the tile's index in `binfo` through the sorts below
     // Work split: tiles grouped by class (each class keeps its layer / row / column order, so a
     // CTA's range covers neighbouring cells), costs prefix-summed for the launch-time cut.
-    // Inside a class the tiles run in bands of $MCS_TILED_ORDER cell rows over the whole panorama width; inside a band
-    // layer by layer, each layer's cells in raster order (0 = no bands: layer by layer).
-    const char* env_order = getenv("MCS_TILED_ORDER");
-    const int band = env_order ? atoi(env_order) : 1;
-    auto by_class = [band](const McsTile& a, const McsTile& b) {
+    // Inside a class the tiles run cell row by cell row over the whole panorama width, each row left to right.
+    auto by_class = [](const McsTile& a, const McsTile& b) {
         if (a.cls != b.cls) return a.cls > b.cls;
-        if (band <= 0) return false;
-        const int ba = a.y0 / (MCS_CELL_H * band), bb = b.y0 / (MCS_CELL_H * band);
-        if (ba != bb) return ba < bb;
-        if (band > 1 && a.layer != b.layer) return a.layer < b.layer;
-        if (a.y0 / MCS_CELL_H != b.y0 / MCS_CELL_H) return a.y0 < b.y0;
+        if (a.y0 / MCS_CELL_H != b.y0 / MCS_CELL_H) return a.y0 / MCS_CELL_H < b.y0 / MCS_CELL_H;
         return a.cx0 < b.cx0;
     };
     std::stable_sort(tiles.begin(), tiles.end(), by_class);
@@ -643,8 +636,8 @@ void mcs_plan_build_tiles(mcs_plan* plan) {
     std::vector<uint8_t> tile_passes(n_tiles, 0);
     int fast_passes = 0, n_fast = 0;
     {
-        const char* env = getenv("MCS_TILED_FAST");   // experiments: 0 = per-pixel descriptors only
-        const bool want = !(env && atoi(env) == 0) && C == 3 && MCS_TILED_WARPS == 8;
+        const char* env = getenv("MCS_TILED_FAST");   // tests: 0 = per-pixel descriptors only
+        const bool want = !(env && atoi(env) == 0) && C == 3;
         if (want && e == cudaSuccess && n_warp_tiles > 0) {
             uint8_t* d_counts = nullptr;
             std::vector<uint8_t> counts(8 * (size_t)n_warp_tiles);
@@ -663,7 +656,7 @@ void mcs_plan_build_tiles(mcs_plan* plan) {
                 // template (two passes, 86 % of the tiles) 0.877 ms per 64 panoramas against 0.833 ms for the
                 // per-pixel path, with up to 32 (one pass, 20 % of the tiles) 0.837 against 0.821.  The group path
                 // is therefore kept for tiles that are really at unit scale: at most 12 pixels per warp (5 %) off.
-                const char* env_max = getenv("MCS_TILED_FAST_MAX");   // experiments
+                const char* env_max = getenv("MCS_TILED_FAST_MAX");   // tests
                 int limit = env_max ? atoi(env_max) : 12;
                 limit = std::max(0, std::min(limit, 32 * MCS_FAST_MAX_PASSES));
                 for (int i = 0; i < n_warp_tiles; ++i) {
@@ -781,7 +774,7 @@ void mcs_plan_build_tiles(mcs_plan* plan) {
     plan->fast_passes = fast_passes;
     plan->d_desc = d_desc;
     {
-        // frames per sweep of the tile table; $MCS_TILED_FRAME_BLOCK overrides (experiments)
+        // frames per sweep of the tile table; $MCS_TILED_FRAME_BLOCK overrides (tests)
         const char* env = getenv("MCS_TILED_FRAME_BLOCK");
         const int v = env ? atoi(env) : 0;
         plan->frame_block = v > 0 ? v : MCS_FRAME_BLOCK_DEFAULT;

@@ -9,11 +9,7 @@ only its own output goes back to the host (SURVEY.md section 8 row e).
 """
 import torch
 
-import os
-
 from . import _cabi
-
-_NO_KERNEL = bool(os.environ.get("MCS_SEQ_NO_KERNEL"))   # experiments: copies only (wrong panoramas)
 
 
 def shard_range(n_frames, world_size, rank):
@@ -160,9 +156,8 @@ class SequencePipeline(object):
             self.s_k.wait_event(slot["ev_in"])
             if slot["used"]:
                 self.s_k.wait_event(slot["ev_out"])     # previous D2H done reading dst
-            if not _NO_KERNEL:
-                self.plan.run([t[:n] for t in slot["src"]], out=slot["dst"][:n], n_frames=n,
-                              stream=self.s_k)
+            self.plan.run([t[:n] for t in slot["src"]], out=slot["dst"][:n], n_frames=n,
+                          stream=self.s_k)
             slot["ev_k"].record(self.s_k)
         with torch.cuda.stream(self.s_out):
             self.s_out.wait_event(slot["ev_k"])

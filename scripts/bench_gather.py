@@ -9,13 +9,11 @@ F = 32
 batch = {l: torch.from_numpy(np.stack([images[l]] * F)).to(dev) for l in labels}
 plan = st.plan([images[l].shape for l in labels], dev)
 out = plan.new_output(F, pitch_align=128)
-import os
-for v, legacy in ((2, ''), (1, ''), (1, 'MCS_GATHER_BYTES'), (1, 'MCS_GATHER_LEGACY')):
+for v, mode in ((2, ''), (1, ''), (1, 'MCS_GATHER_BYTES')):
     plan.handle.force_variant(v)
-    os.environ.pop('MCS_GATHER_LEGACY', None)
     os.environ.pop('MCS_GATHER_BYTES', None)
-    if legacy:
-        os.environ[legacy] = '1'   # read by the library at every call
+    if mode:
+        os.environ[mode] = '1'   # read by the library at every call
     st.stitch_batch(batch, out=out); torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for _ in range(3): st.stitch_batch(batch, out=out)
@@ -24,4 +22,4 @@ for v, legacy in ((2, ''), (1, ''), (1, 'MCS_GATHER_BYTES'), (1, 'MCS_GATHER_LEG
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 10
     ab = plan.algorithmic_bytes()
-    print('variant=%d mode=%s ms=%.3f frac=%.3f' % (plan.handle.last_variant(), legacy, ms, ab * F / ms / 1e6 / 6533.5))
+    print('variant=%d mode=%s ms=%.3f frac=%.3f' % (plan.handle.last_variant(), mode, ms, ab * F / ms / 1e6 / 6533.5))

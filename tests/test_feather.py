@@ -260,14 +260,11 @@ def test_feather_ramp_in_super_mode(cuda_device, n, h, w, c, log2):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("spread", ["0", "1"])
-def test_fused_bands_over_several_frame_blocks(cuda_device, monkeypatch, spread):
-    """BAND chunks of frame block b + 1 follow the COPY / ZERO chunks of block b in the sweep, and with
-    $MCS_TILED_BAND_SPREAD they are spread between the ordinary resampled chunks: either way the box issuer
+def test_fused_bands_over_several_frame_blocks(cuda_device, monkeypatch):
+    """BAND chunks of frame block b + 1 follow the COPY / ZERO chunks of block b in the sweep: the box issuer
     enters a BAND chunk only when the consumers get there.  11 frames in blocks of 4."""
     import torch
     monkeypatch.setenv("MCS_TILED_FRAME_BLOCK", "4")
-    monkeypatch.setenv("MCS_TILED_BAND_SPREAD", spread)
     n, h, w, c, log2 = 5, 270, 480, 3, 3
     st, states, labels, images = synthetic_chain(n, h, w, c, kind="noise", xoffset=2, yoffset=7)
     st.feather_log2 = log2

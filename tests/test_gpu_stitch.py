@@ -459,8 +459,8 @@ def test_frame_counts_whose_last_block_is_shorter_than_the_split(cuda_device, n_
 def test_gather_variant_batches(cuda_device, monkeypatch, n, h, w, c, super_mode):
     """The fallback kernel loops the frames of a launch inside its threads (16 per thread, the rest through
     grid.z): batches around that block size, frame by frame against the cv2 chain - with rows that are and are
-    not multiples of four bytes (aligned word loads or byte loads for the taps), with the byte loads forced
-    ($MCS_GATHER_BYTES), and through the older frame-per-CTA form kept behind $MCS_GATHER_LEGACY."""
+    not multiples of four bytes (aligned word loads or byte loads for the taps), and with the byte loads forced
+    ($MCS_GATHER_BYTES)."""
     st, states, labels, images = synthetic_chain(n, h, w, c, kind="noise", super_mode=super_mode)
     plan = st.plan([images[l].shape for l in labels], cuda_device)
     try:
@@ -469,9 +469,8 @@ def test_gather_variant_batches(cuda_device, monkeypatch, n, h, w, c, super_mode
             sets = [synthetic_chain(n, h, w, c, kind="noise", super_mode=super_mode, frame_index=f % 5)[3] for f in range(F)]
             batch = {l: torch.from_numpy(np.stack([s[l] for s in sets])).to(cuda_device) for l in labels}
             refs = [stitcher_ref.stitch_chain(states, labels, sets[f]) for f in range(min(F, 5))]
-            for mode in ("", "MCS_GATHER_BYTES", "MCS_GATHER_LEGACY"):
-                for k in ("MCS_GATHER_LEGACY", "MCS_GATHER_BYTES"):
-                    monkeypatch.delenv(k, raising=False)
+            for mode in ("", "MCS_GATHER_BYTES"):
+                monkeypatch.delenv("MCS_GATHER_BYTES", raising=False)
                 if mode:
                     monkeypatch.setenv(mode, "1")
                 # dense panorama rows, and rows padded to a multiple of four bytes
