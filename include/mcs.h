@@ -126,7 +126,8 @@ int mcs_plan_destroy(mcs_plan* plan);
 /*
  * mcs_plan_owned_pixels - per-layer count of output pixels whose value is
  * taken from that layer and has at least one bilinear tap inside the source
- * (for COPY layers: every pixel of the visible rectangle).  Host array
+ * (for COPY layers: every pixel of the visible rectangle); with camera weights
+ * (mcs_plan_set_camera_weights) the pixels the layer contributes to.  Host array
  * owned[n_layers].  This is the `owned_k` of SURVEY.md section 8(d):
  *   algorithmic bytes / panorama = out_w*out_h*C + C * sum_k owned_k.
  * Synchronous (runs a counting kernel on `cuda_stream` and waits).
@@ -139,7 +140,7 @@ int mcs_plan_owned_pixels(const mcs_plan* plan, int64_t* owned_host, void* cuda_
  * the window cannot influence the panorama - they belong to the part of the camera that the
  * reference's paste (StitcherClass.py:240-241) overwrites - so a host-facing caller needs to
  * bring only the window onto the device.  Whole frames when the windows are not known (no tile
- * table, feather mode).
+ * table, feather mode, camera weights).
  */
 int mcs_plan_source_windows(const mcs_plan* plan, int32_t* xyxy);
 
@@ -239,9 +240,39 @@ int mcs_plan_set_feather(mcs_plan* plan, int feather_log2);
 int mcs_plan_set_blend(mcs_plan* plan, int feather_log2, const int32_t* paste_xyxy,
                        const uint8_t* const* weight_maps, const int64_t* map_pitch);
 
+/*
+ * mcs_plan_set_camera_weights - the camera-weighted blend: every camera that sees an output pixel
+ * contributes, weighted by its own per-pixel weight map and normalised by the summed weights (the
+ * blend of OpenCV's FeatherBlender, in integers).  For output pixel p and layer k:
+ *   v_k  what the layer produces at p in overwrite mode (COPY: the source pixel; WARP / REMAP: the
+ *        fixed-point bilinear sample, BORDER_CONSTANT 0)
+ *   w_k  the same sample (same coordinates, taps and rounding) of the layer's weight map, i.e.
+ *        cv2.warpPerspective(map, cachedAH, ABSize) placed like the camera's image
+ *   the contributors are the layers whose visible rectangle contains p and whose w_k > 0, S = sum w_k;
+ *   out = (sum w_k * v_k + S / 2) / S per channel (integer division), 0 where S == 0.
+ * One contributor gives v_k exactly.  Unlike the overwrite, the zero background of an inner canvas
+ * does not hide the outer cameras.  Extension with no reference counterpart; specification in
+ * oracle/camera_weight_model.py.
+ *
+ *   weight_maps  host [n_layers] pointers: weight_maps[k] is a uint8 map of layer k's SOURCE frame
+ *                (src_h rows of src_w values, map_pitch[k] bytes apart), one value per camera pixel,
+ *                so it survives recalibration; a NULL entry means 255 everywhere.
+ *                weight_maps == NULL switches the mode off (the plan is the overwrite again).
+ *   map_pitch    host [n_layers]
+ * The maps are copied; a counting kernel then records what each layer contributes (reported by
+ * mcs_plan_owned_pixels: algorithmic bytes = out_w*out_h*C + C * sum_k contributions_k) and the most
+ * contributors any pixel has.  More than 4 fails with MCS_ERR_UNSUPPORTED and leaves the plan in
+ * overwrite mode.  The mode excludes the stage-wise blend of mcs_plan_set_blend: setting either while
+ * the other is on fails with MCS_ERR_INVALID.  mcs_stitch_u8 runs a kernel of its own for it (variant
+ * 5; forcing the tiled variant fails with MCS_ERR_UNSUPPORTED), and mcs_plan_source_windows / _spans
+ * report whole frames.  Synchronous.
+ */
+int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_maps, const int64_t* map_pitch);
+
 /* Which kernel variant the last mcs_stitch_u8 on this plan launched
  * (diagnostics for tests / bench): 0 = none yet, 1 = gather, 2 = tiled, 3 = overwrite pass +
- * feather band pass, 4 = tiled with the seam bands blended in the same launch. */
+ * feather band pass, 4 = tiled with the seam bands blended in the same launch, 5 = camera-weighted
+ * blend (mcs_plan_set_camera_weights). */
 int mcs_plan_last_variant(const mcs_plan* plan);
 
 /* Pin the kernel variant of a plan: 0 = automatic (tiled when the plan and the buffers allow

@@ -63,6 +63,12 @@ class Stitcher(Debugger):
     # stage, None or a uint8 array of the shape of that stage's imageB (the running canvas) holding the canvas'
     # weight in units of 1 / 2**feather_log2; None everywhere = the distance ramp of feather_log2.
     blend_weights = None
+    # Optional camera-weighted blend (extension, include/mcs.h mcs_plan_set_camera_weights): a dict
+    # {label: None or a uint8 array of that camera's calibrated (h, w)} - every camera that sees a pixel
+    # contributes, weighted by its own map and normalised by the summed weights; None = 255 everywhere, a
+    # missing label likewise.  None (the default) keeps the reference's overwrite.  ``edge_ramp`` gives the
+    # FeatherBlender-style map.
+    camera_weights = None
 
     def __init__(self, images_dic, super_mode=False):
         # labels sorted like np.sort(images_dic.keys()) (reference :61)
@@ -141,7 +147,8 @@ class Stitcher(Debugger):
             return images_dic[self.img_labels[-1]]
         frames = [images_dic[label] for label in self.img_labels]
         out = _composite(self._engine_(), self.stitchers, frames, batched=False, debugger=self,
-                         feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights)
+                         feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
+                         camera_weights=self._camera_weight_list())
         if draw_descriptors and not _is_tensor(out):
             out = self._draw_overlays(out, frames)
         return out
@@ -184,12 +191,40 @@ class Stitcher(Debugger):
         tensor ``[F, H_out, W_out, C]``.  Extension of the reference API."""
         frames = [frames_dic[label] for label in self.img_labels]
         return _composite(self._engine_(), self.stitchers, frames, batched=True, out=out, debugger=self,
-                          feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights)
+                          feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
+                          camera_weights=self._camera_weight_list())
 
     def plan(self, img_shapes, device=None):
         """Compiled plan (``engine.CompiledPlan``) for frames of these shapes."""
         return self._engine_().plan_for(self.stitchers, [tuple(s) for s in img_shapes], device,
-                                        feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights)
+                                        feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
+                                        camera_weights=self._camera_weight_list())
+
+    def _camera_weight_list(self):
+        """``camera_weights`` checked and as a list in camera order, or None when the mode is off."""
+        cw = self.camera_weights
+        if cw is None:
+            return None
+        if getattr(self, "feather_log2", 0) or self.blend_weights is not None:
+            raise ValueError("camera_weights cannot be combined with feather_log2 / blend_weights")
+        by_label = {str(k): v for k, v in dict(cw).items()}
+        labels = [str(l) for l in self.img_labels]
+        unknown = sorted(set(by_label) - set(labels))
+        if unknown:
+            raise ValueError("camera_weights names unknown cameras %r (cameras: %r)" % (unknown, labels))
+        out = []
+        for i, label in enumerate(labels):
+            m = by_label.get(label)
+            if m is not None:
+                m = np.asarray(m)
+                # calibrated frame size: imageB of the first stage for camera 0, imageA of stage i - 1 otherwise
+                st = self.stitchers[max(0, i - 1)]
+                size = st.BimgSize if i == 0 else st.AimgSize
+                if m.dtype != np.uint8 or m.ndim != 2 or (size is not None and m.shape != tuple(size[:2])):
+                    raise ValueError("camera_weights[%r] must be a uint8 array of the camera's calibrated (h, w) %r, "
+                                     "got %s %r" % (label, None if size is None else tuple(size[:2]), m.dtype, m.shape))
+            out.append(m)
+        return out
 
     # -- persistence -----------------------------------------------------------
     def save_stitcher(self, save_path):
@@ -497,8 +532,23 @@ def _segments(stages, frame_shapes, debugger=None):
     return segs
 
 
-def _composite(engine, stages, frames, batched, out=None, debugger=None, feather_log2=0, blend_weights=None):
-    """Run the fused kernel for this chain on these frames."""
+def edge_ramp(shape, width=64):
+    """A camera's edge ramp as a uint8 weight map for ``Stitcher.camera_weights``: ``min(255, (1 + distance to
+    the nearest frame edge) * 255 // width)`` over a frame of ``shape`` ((h, w) or an image shape).  With it on
+    every camera, overlaps blend like OpenCV's FeatherBlender."""
+    h, w = int(shape[0]), int(shape[1])
+    width = int(width)
+    if width < 1:
+        raise ValueError("ramp width must be at least 1, got %d" % width)
+    yy, xx = np.mgrid[0:h, 0:w]
+    d = np.minimum(np.minimum(xx, w - 1 - xx), np.minimum(yy, h - 1 - yy))
+    return np.minimum(255, (1 + d) * 255 // width).astype(np.uint8)
+
+
+def _composite(engine, stages, frames, batched, out=None, debugger=None, feather_log2=0, blend_weights=None,
+               camera_weights=None):
+    """Run the fused kernel for this chain on these frames.  ``camera_weights``: one entry per camera (None or
+    a uint8 map) for the camera-weighted blend, or None."""
     import torch  # local: keeps `import StitcherClass` cheap for calibration-only users
 
     on_device = _is_tensor(frames[0]) and frames[0].is_cuda
@@ -517,8 +567,12 @@ def _composite(engine, stages, frames, batched, out=None, debugger=None, feather
 
     def plan_for(sub_stages, sub_shapes):
         try:
+            if camera_weights is not None and len(segs) > 1:
+                raise PlanUnsupported("camera weights need the whole chain in one plan, but a composited canvas is "
+                                      "resized at stage %d" % segs[1]["a"])
             return engine.plan_for(sub_stages, sub_shapes, device, feather_log2=feather_log2,
-                                   blend_weights=[weight_of.get(id(st)) for st in sub_stages] if weight_of else None)
+                                   blend_weights=[weight_of.get(id(st)) for st in sub_stages] if weight_of else None,
+                                   camera_weights=camera_weights)
         except PlanUnsupported as e:
             if debugger is not None:
                 debugger.debugger(DEBUG_LEVEL_0, "[STITCHER] {}".format(e), log_type="err")

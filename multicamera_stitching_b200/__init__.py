@@ -5,9 +5,9 @@
 recalibration matcher / RANSAC run as hand-written sm_100a kernels behind the
 C ABI declared in ``include/mcs.h`` (``libmcs_b200.so``).
 """
-from .StitcherClass import Stitcher, StitcherBase  # noqa: F401
+from .StitcherClass import Stitcher, StitcherBase, edge_ramp  # noqa: F401
 from .Utils import (CalculateProjectionMatrix, get_projection_point_dst,  # noqa: F401
                     get_projection_point_src)
 
-__all__ = ["Stitcher", "StitcherBase", "CalculateProjectionMatrix",
+__all__ = ["Stitcher", "StitcherBase", "edge_ramp", "CalculateProjectionMatrix",
            "get_projection_point_dst", "get_projection_point_src"]

@@ -17,12 +17,12 @@ MCS_MAX_LAYERS = 16
 MCS_LAYER_COPY = 0
 MCS_LAYER_WARP = 1
 MCS_LAYER_REMAP = 2
-ABI_VERSION = 1
+ABI_VERSION = 2
 
 # every symbol include/mcs.h declares
 EXPORTS = (
     "mcs_abi_version", "mcs_last_error", "mcs_plan_create", "mcs_plan_create_maps", "mcs_plan_destroy",
-    "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_last_variant",
+    "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_set_camera_weights", "mcs_plan_last_variant",
     "mcs_plan_force_variant", "mcs_plan_rows_need_padding", "mcs_plan_promise_padded_rows",
     "mcs_plan_tiled_status", "mcs_plan_tiled_ctas_per_sm", "mcs_plan_tiled_stats", "mcs_launch_count",
     "mcs_match_hamming_top2", "mcs_match_l2_top2", "mcs_ransac_homography", "mcs_refit_homography", "mcs_resize_linear_u8",
@@ -100,6 +100,8 @@ def load(build_if_missing=False):
     lib.mcs_plan_set_feather.argtypes = [_vp, ctypes.c_int]
     lib.mcs_plan_set_blend.restype = ctypes.c_int
     lib.mcs_plan_set_blend.argtypes = [_vp, ctypes.c_int, _c_i32p, ctypes.POINTER(ctypes.c_void_p), _c_i64p]
+    lib.mcs_plan_set_camera_weights.restype = ctypes.c_int
+    lib.mcs_plan_set_camera_weights.argtypes = [_vp, ctypes.POINTER(ctypes.c_void_p), _c_i64p]
     lib.mcs_plan_tiled_ctas_per_sm.restype = ctypes.c_int
     lib.mcs_plan_tiled_ctas_per_sm.argtypes = [_vp]
     lib.mcs_plan_tiled_status.restype = ctypes.c_char_p
@@ -242,6 +244,7 @@ class Plan(object):
         self.out_h = int(out_h)
         self.src_hw = hw.copy()
         self._owned = None
+        self.camera_weighted = False   # set_camera_weights is in force
 
     def close(self):
         if getattr(self, "_h", None) is not None and _lib is not None:
@@ -328,6 +331,36 @@ class Plan(object):
             m_ptr, pitch_ptr = ptrs, pitches.ctypes.data_as(_c_i64p)
             keep.append(pitches)
         check(_lib.mcs_plan_set_blend(self._h, int(feather_log2), p_ptr, m_ptr, pitch_ptr), "mcs_plan_set_blend")
+
+    def set_camera_weights(self, weight_maps):
+        """``weight_maps``: None (the plain overwrite) or a list of n_layers entries, each None (255 everywhere)
+        or a uint8 array of that layer's source (height, width): the camera-weighted blend (include/mcs.h)."""
+        n = self.n_layers
+        if weight_maps is None:
+            check(_lib.mcs_plan_set_camera_weights(self._h, None, None), "mcs_plan_set_camera_weights")
+            self._owned = None
+            self.camera_weighted = False
+            return
+        if len(weight_maps) != n:
+            raise ValueError("weight_maps must list %d entries (one per layer)" % n)
+        ptrs = (ctypes.c_void_p * n)()
+        pitches = np.zeros(n, np.int64)
+        keep = []   # host arrays must outlive the call
+        for k, m in enumerate(weight_maps):
+            if m is None:
+                continue
+            m = np.ascontiguousarray(m, dtype=np.uint8)
+            if m.shape != tuple(int(v) for v in self.src_hw[k]):
+                raise ValueError("weight map %d has shape %r, its source is %r" % (k, m.shape, tuple(self.src_hw[k])))
+            keep.append(m)
+            ptrs[k] = m.ctypes.data
+            pitches[k] = m.strides[0]
+        self._owned = None
+        # on failure the library leaves the plan in the overwrite
+        self.camera_weighted = False
+        check(_lib.mcs_plan_set_camera_weights(self._h, ptrs, pitches.ctypes.data_as(_c_i64p)),
+              "mcs_plan_set_camera_weights")
+        self.camera_weighted = True
 
     def tiled_ctas_per_sm(self):
         return int(_lib.mcs_plan_tiled_ctas_per_sm(self._h))

@@ -8,7 +8,7 @@
 
 #include "mcs.h"
 
-#define MCS_ABI_VERSION 1
+#define MCS_ABI_VERSION 2
 
 // ---- error plumbing -------------------------------------------------------
 void mcs_set_error(const char* fmt, ...);
@@ -161,6 +161,10 @@ struct mcs_plan {
     uint8_t* d_wmap[MCS_MAX_LAYERS];   // per layer k >= 1: weight map of the paste of stage k (over the pasted
                              // rectangle of layer k - 1, values 0 .. 2^feather_log2), nullptr = the distance ramp
     unsigned* d_work;
+    // camera-weighted blend (mcs_plan_set_camera_weights, mcs_stitch_weighted.cu)
+    int cw_active;           // the plan blends every camera that sees a pixel, normalised by the summed weights
+    uint8_t* d_cwmap[MCS_MAX_LAYERS];   // per layer: device weight map, src_h x src_w bytes (nullptr = 255 everywhere)
+    long long cw_contrib[MCS_MAX_LAYERS];   // per layer: output pixels it contributes to
 };
 
 
@@ -176,6 +180,15 @@ void mcs_plan_free_tiles(mcs_plan* plan);
 // failure to build leaves the table empty; the on-the-fly band kernel then serves the mode.
 void mcs_feather_build_table(mcs_plan* plan);
 void mcs_feather_free_table(mcs_plan* plan);
+
+// Camera-weighted blend (mcs_stitch_weighted.cu): at most this many cameras blend into one pixel (their
+// weights stay in registers, and the multiply-high division is exact for sums up to 4 * 255)
+#define MCS_CW_MAX_CONTRIB 4
+// Per layer, the output pixels it contributes to, and the most contributors of any pixel (synchronous).
+int mcs_camera_weights_count(const mcs_plan* plan, long long* contrib, int* max_count);
+int mcs_launch_weighted(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,
+                        const int64_t* fstride, int n_frames, uint8_t* dst, int64_t dst_pitch,
+                        int64_t dst_frame_stride, cudaStream_t stream);
 
 // Tiled variant (mcs_stitch_tiled.cu): why it cannot serve a call (nullptr = it can), and its launch.
 const char* mcs_tiled_blocker(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,

@@ -212,8 +212,10 @@ extern "C" int mcs_plan_destroy(mcs_plan* plan) {
     mcs_feather_free_table(plan);
     if (plan->d_strips) cudaFree(plan->d_strips);
     if (plan->d_strip_prefix) cudaFree(plan->d_strip_prefix);
-    for (int k = 0; k < MCS_MAX_LAYERS; ++k)
+    for (int k = 0; k < MCS_MAX_LAYERS; ++k) {
         if (plan->d_wmap[k]) cudaFree(plan->d_wmap[k]);
+        if (plan->d_cwmap[k]) cudaFree(plan->d_cwmap[k]);
+    }
     mcs_plan_free_tiles(plan);
     free_maps(plan);
     delete plan;
@@ -233,7 +235,9 @@ extern "C" int mcs_plan_source_windows(const mcs_plan* plan, int32_t* xyxy) {
     MCS_CHECK_ARG(plan != nullptr && xyxy != nullptr, "mcs_plan_source_windows: NULL argument");
     // The feather band samples outer cameras inside the pasted rectangles, i.e. outside the
     // pixels they own: there every frame counts in full.
-    const bool known = plan->src_win_valid && ((plan->feather_log2 == 0 && !plan->blend_custom) || plan->band_fused);
+    // The camera-weighted blend samples every camera wherever its rectangle reaches: whole frames too.
+    const bool known = plan->src_win_valid && !plan->cw_active &&
+                       ((plan->feather_log2 == 0 && !plan->blend_custom) || plan->band_fused);
     for (int k = 0; k < plan->n_layers; ++k) {
         xyxy[4 * k + 0] = known ? plan->src_win[k][0] : 0;
         xyxy[4 * k + 1] = known ? plan->src_win[k][1] : 0;
@@ -250,7 +254,8 @@ extern "C" int mcs_plan_source_spans(const mcs_plan* plan, int layer, int band_r
     const McsLayer& L = plan->layers[layer];
     const int n_bands = (L.src_h + band_rows - 1) / band_rows;
     const int* span = plan->h_row_span[layer];
-    const bool known = plan->src_win_valid && ((plan->feather_log2 == 0 && !plan->blend_custom) || plan->band_fused) && span != nullptr;
+    const bool known = plan->src_win_valid && !plan->cw_active &&
+                       ((plan->feather_log2 == 0 && !plan->blend_custom) || plan->band_fused) && span != nullptr;
     for (int b = 0; b < n_bands; ++b) {
         int x0 = known ? INT_MAX : 0, x1 = known ? INT_MIN : L.src_w;
         for (int r = b * band_rows; known && r < (b + 1) * band_rows && r < L.src_h; ++r) {
@@ -367,6 +372,8 @@ extern "C" int mcs_plan_set_blend(mcs_plan* plan, int feather_log2, const int32_
     MCS_CHECK_ARG(!any_map || map_pitch != nullptr, "mcs_plan_set_blend: weight maps without their pitches");
     MCS_CHECK_ARG(!any_map || feather_log2 <= MCS_BAND_MAX_LOG2,
                   "mcs_plan_set_blend: weight maps take feather_log2 <= %d (got %d)", MCS_BAND_MAX_LOG2, feather_log2);
+    MCS_CHECK_ARG(!plan->cw_active || (feather_log2 == 0 && !any_map),
+                  "mcs_plan_set_blend: the plan blends with camera weights; clear them first");
     free_strips(plan);
     free_wmaps(plan);
     const bool had = plan->feather_log2 > 0 || plan->blend_custom;
@@ -485,5 +492,55 @@ extern "C" int mcs_plan_set_blend(mcs_plan* plan, int feather_log2, const int32_
     plan->feather_log2 = feather_log2;
     mcs_feather_build_table(plan);
     rebuild_tiles(plan);   // the tile table knows the seam bands (BAND tiles): the tiled kernel then blends them itself
+    return MCS_OK;
+}
+
+static void free_cwmaps(mcs_plan* plan) {
+    for (int k = 0; k < MCS_MAX_LAYERS; ++k) {
+        if (plan->d_cwmap[k]) cudaFree(plan->d_cwmap[k]);
+        plan->d_cwmap[k] = nullptr;
+    }
+    plan->cw_active = 0;
+}
+
+extern "C" int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_maps, const int64_t* map_pitch) {
+    MCS_CHECK_ARG(plan != nullptr, "mcs_plan_set_camera_weights: plan is NULL");
+    bool any_map = false;
+    for (int k = 0; weight_maps && k < plan->n_layers; ++k) any_map = any_map || weight_maps[k] != nullptr;
+    MCS_CHECK_ARG(!any_map || map_pitch != nullptr, "mcs_plan_set_camera_weights: weight maps without their pitches");
+    for (int k = 0; any_map && k < plan->n_layers; ++k)
+        MCS_CHECK_ARG(!weight_maps[k] || map_pitch[k] >= plan->layers[k].src_w,
+                      "mcs_plan_set_camera_weights: weight map %d: pitch %lld < %d columns", k, (long long)map_pitch[k],
+                      plan->layers[k].src_w);
+    MCS_CHECK_ARG(!weight_maps || (plan->feather_log2 == 0 && !plan->blend_custom),
+                  "mcs_plan_set_camera_weights: the plan feathers its pastes (mcs_plan_set_blend); switch that off first");
+    free_cwmaps(plan);
+    if (!weight_maps) return MCS_OK;
+    for (int k = 0; k < plan->n_layers; ++k) {
+        if (!weight_maps[k]) continue;
+        const McsLayer& L = plan->layers[k];
+        cudaError_t e = cudaMalloc(&plan->d_cwmap[k], (size_t)L.src_w * L.src_h);
+        if (e == cudaSuccess)
+            e = cudaMemcpy2D(plan->d_cwmap[k], (size_t)L.src_w, weight_maps[k], (size_t)map_pitch[k], (size_t)L.src_w,
+                             (size_t)L.src_h, cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) {
+            free_cwmaps(plan);
+            mcs_set_error("mcs_plan_set_camera_weights: weight map %d: %s", k, cudaGetErrorString(e));
+            return MCS_ERR_CUDA;
+        }
+    }
+    int most = 0;
+    const int rc = mcs_camera_weights_count(plan, plan->cw_contrib, &most);
+    if (rc != MCS_OK) {
+        free_cwmaps(plan);
+        return rc;
+    }
+    if (most > MCS_CW_MAX_CONTRIB) {
+        free_cwmaps(plan);
+        mcs_set_error("mcs_plan_set_camera_weights: %d cameras with non-zero weight meet at one output pixel (at most %d "
+                      "blend); lower the weights of some of them there", most, MCS_CW_MAX_CONTRIB);
+        return MCS_ERR_UNSUPPORTED;
+    }
+    plan->cw_active = 1;
     return MCS_OK;
 }

@@ -87,7 +87,7 @@ class PinnedResults(object):
 class CompiledPlan(object):
     """A flattened chain plus its ``mcs_plan`` on one device."""
 
-    def __init__(self, flat, device, feather_log2=0, blend_weights=None):
+    def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None):
         self.flat = flat
         self.device = torch.device(device)
         self.feather_log2 = int(feather_log2)
@@ -105,13 +105,20 @@ class CompiledPlan(object):
             if self.feather_log2 or maps is not None:
                 # the paste rectangles matter only when a super-mode crop cut a visible one
                 self.handle.set_blend(self.feather_log2, plan_paste(flat), maps)
+            if camera_weights is not None:   # one map per camera, in the layer order of the plan
+                self.handle.set_camera_weights([camera_weights[l.cam] if l.cam < len(camera_weights) else None
+                                                for l in flat.layers])
             # rows that are not a multiple of 4 bytes: run() always passes them through its
             # zero-padded scratch buffers, which is what the tiled kernel needs to serve them
-            self.pad_rows = self.handle.tiled_status() == "" and self.handle.rows_need_padding()
+            self.pad_rows = self._tiled() and self.handle.rows_need_padding()
             if self.pad_rows:
                 self.handle.promise_padded_rows(True)
         self.cams = [l.cam for l in flat.layers]
         self.out_w, self.out_h, self.channels = flat.out_w, flat.out_h, flat.channels
+
+    def _tiled(self):
+        """Whether the tiled kernel serves this plan (it does not serve the camera-weighted blend)."""
+        return self.handle.tiled_status() == "" and not self.handle.camera_weighted
 
     # ---- geometry helpers -------------------------------------------------
     def out_shape(self, n_frames=None):
@@ -222,7 +229,7 @@ class CompiledPlan(object):
         if tuple(out.shape) != self.out_shape(n_frames):
             raise ValueError("output shape %r != %r" % (tuple(out.shape), self.out_shape(n_frames)))
         ptrs, pitches, fstrides = [], [], []
-        tiled = self.handle.tiled_status() == ""
+        tiled = self._tiled()
         for l in self.flat.layers:
             t = frames_by_cam[l.cam]
             want = ((F,) if batched else ()) + tuple(l.src_hw) + ((self.channels,) if self.flat.ndim == 3 else ())
@@ -265,7 +272,7 @@ class CompositeEngine(object):
             self._device = torch.device("cuda", torch.cuda.current_device())
         return torch.device(self._device)
 
-    def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None):
+    def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None, camera_weights=None):
         """Compiled plan for this chain state and these frame shapes, or None
         when no stage is calibrated (decided on the host, no device needed)."""
         shapes = tuple(tuple(int(v) for v in s) for s in cam_shapes)
@@ -278,14 +285,19 @@ class CompositeEngine(object):
         if blend_weights is not None and any(w is not None for w in blend_weights):
             wkey = tuple(None if w is None else (np.asarray(w).shape, hash(np.ascontiguousarray(w, dtype=np.uint8).tobytes()))
                          for w in blend_weights)
-        key = (str(device), shapes, sig, feather_log2, wkey)
+        ckey = None
+        if camera_weights is not None:
+            ckey = tuple(None if w is None else (np.asarray(w).shape, hash(np.ascontiguousarray(w, dtype=np.uint8).tobytes()))
+                         for w in camera_weights)
+        key = (str(device), shapes, sig, feather_log2, wkey, ckey)
         if key in self._plans:
             self._plans[key] = self._plans.pop(key)      # most recently used last
         else:
             flat = flatten_chain(stages, shapes)
             while len(self._plans) >= self.max_plans:     # evict the least recently used, one at a time
                 self._plans.pop(next(iter(self._plans)))
-            self._plans[key] = CompiledPlan(flat, device, feather_log2, blend_weights) if flat is not None else None
+            self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights)
+                                if flat is not None else None)
         return self._plans[key]
 
     def upload(self, cam, arr, device, bands=None):
