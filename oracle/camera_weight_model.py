@@ -114,6 +114,13 @@ def blend(layers, out_w, out_h, frames, maps):
 def chain(states, img_labels, images_dic, maps_by_label):
     """The chain restatement with cv2, stage by stage (oracle dict states, ``stitcher_ref``'s field
     names).  ``maps_by_label[label]``: uint8 map of the camera's frame or None.  Returns the panorama."""
+    planes = chain_planes(states, img_labels, images_dic, maps_by_label)
+    out, _, _ = combine(*zip(*planes))
+    return out[:, :, 0] if np.asarray(images_dic[img_labels[0]]).ndim == 2 else out
+
+
+def chain_planes(states, img_labels, images_dic, maps_by_label):
+    """The per-camera ``(value, weight, reach)`` planes of ``chain``, each the size of the panorama."""
     def wmap(label):
         m = maps_by_label.get(label)
         return np.full(np.asarray(images_dic[label]).shape[:2], 255, np.uint8) if m is None else np.asarray(m, np.uint8)
@@ -141,8 +148,7 @@ def chain(states, img_labels, images_dic, maps_by_label):
             ys, xs = slice(st["y_limits"][0], st["y_limits"][1]), slice(st["x_limits"][0], st["x_limits"][1])
             moved = [(v[ys, xs], w[ys, xs], r[ys, xs]) for v, w, r in moved]
         planes = moved
-    out, _, _ = combine(*zip(*planes))
-    return out[:, :, 0] if f0.ndim == 2 else out
+    return planes
 
 
 def mulhi_div(n, S):

@@ -7,7 +7,8 @@ from multicamera_stitching_b200 import edge_ramp
 from multicamera_stitching_b200.plan import flatten_chain
 from oracle import camera_weight_model, stitcher_ref
 
-MAP_KINDS = ("random", "binary", "ramp", "absent", "mixed")
+SUPER_TRIM = (9, 5)   # super-mode crops this many pixels inside every stage canvas: several cameras stay
+MAP_KINDS = ("random", "binary", "ramp", "absent", "mixed", "tiny", "rim")   # "mixed" cycles the first four
 
 
 def make_maps(images, labels, kind, seed=0):
@@ -26,13 +27,19 @@ def make_maps(images, labels, kind, seed=0):
             m[:h // 5, :w // 6] = 0                     # a lens-hood corner
         elif k == "ramp":
             m = edge_ramp((h, w), 1 + (i * 7) % 24)
+        elif k == "tiny":                               # weights 0..3: sampled weights of 0 and 1, small sums
+            m = rng.integers(0, 4, size=(h, w), dtype=np.uint8)
+        elif k == "rim":                                # 255 inside a ring of 1 and a one-pixel border of 0
+            m = np.zeros((h, w), np.uint8)
+            m[1:h - 1, 1:w - 1] = 1
+            m[2:h - 2, 2:w - 2] = 255
         else:
             m = None
         out[l] = m
     return out
 
 
-def trimmed_super_chain(n, h, w, c, trim=(9, 5), kind="noise", frame_index=0):
+def trimmed_super_chain(n, h, w, c, trim=SUPER_TRIM, kind="noise", frame_index=0):
     """A super-mode chain whose crops trim a few pixels off every stage canvas (the synthetic default
     limits keep only the newest camera): ``(stitcher, oracle states, labels, images)``."""
     from multicamera_stitching_b200 import Stitcher, synthetic

@@ -3,54 +3,17 @@ camera counts, frame sizes, channel counts, canvas offsets, super mode and homog
 the benchmark's near-identity ones (rotation, anisotropic scale, perspective, mirrored axes), each
 through the automatic variant and, where the plan allows it, with the tiled and the gather kernels
 forced.  Everything must be bit-exact."""
-import math
-
 import numpy as np
 import pytest
 
 from helpers import compare_u8
-from multicamera_stitching_b200 import Stitcher, _cabi
+from multicamera_stitching_b200 import _cabi
 from oracle import stitcher_ref
+from random_rigs import random_chain
 
 pytestmark = pytest.mark.gpu
 
 TILED_SEEDS = []   # seeds whose chain also ran through the forced tiled variant
-
-
-def random_chain(seed):
-    rng = np.random.default_rng(1000 + seed)
-    n = int(rng.integers(2, 6))
-    c = int(rng.choice([1, 3, 3, 4]))
-    h = int(rng.integers(24, 260))
-    w = int(rng.integers(2, 22)) * 16                     # 16-byte rows at every channel count: the tiled variant applies
-    if seed % 5 == 4:
-        w += int(rng.integers(1, 4))                      # odd rows: the gather variant serves them
-    super_mode = bool(seed % 4 == 3)
-    xo, yo = int(rng.integers(0, 30)), int(rng.integers(0, 30))
-    shape = (h, w) if c == 1 else (h, w, c)
-    images = {"CAM%d" % (k + 1): rng.integers(0, 256, size=shape, dtype=np.uint8) for k in range(n)}
-    st = Stitcher(images, super_mode=super_mode)
-    labels = list(st.img_labels)
-    states = []
-    shapeB = shape
-    for k in range(n - 1):
-        ang = math.radians(rng.uniform(-12, 12))
-        sx, sy = rng.uniform(0.7, 1.3, size=2)
-        if seed % 7 == 6 and k == 0:
-            sx = -sx                                      # a mirrored camera
-        A = np.array([[sx * math.cos(ang), -sy * math.sin(ang) + rng.uniform(-0.1, 0.1), 0.0],
-                      [sx * math.sin(ang), sy * math.cos(ang), 0.0], [0.0, 0.0, 1.0]])
-        A[0, 2] = shapeB[1] * rng.uniform(0.3, 0.9) + (w if sx < 0 else 0)
-        A[1, 2] = rng.uniform(-0.2, 0.2) * h
-        A[2, 0], A[2, 1] = rng.uniform(-2e-4, 2e-4, size=2)
-        st.stitchers[k].set_homography(A, shapeA=shape, shapeB=shapeB, xoffset=xo, yoffset=yo)
-        ost = stitcher_ref.new_state(sid=str(k), super_mode=super_mode)
-        stitcher_ref.geometry_from_homography(ost, A, shape, shapeB, xo, yo)
-        states.append(ost)
-        shapeB = st.stitchers[k].result_shape()
-        if shapeB[0] <= 0 or shapeB[1] <= 0 or shapeB[0] * shapeB[1] > 40e6:
-            return None
-    return st, states, labels, images
 
 
 @pytest.mark.parametrize("seed", range(28))

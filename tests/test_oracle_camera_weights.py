@@ -8,10 +8,11 @@ import cv2
 import numpy as np
 import pytest
 
-from camera_weight_cases import chain_case, layer_model, make_maps
+from camera_weight_cases import MAP_KINDS, SUPER_TRIM, chain_case, layer_model, make_maps
 from multicamera_stitching_b200 import Stitcher, _cabi, edge_ramp
 from multicamera_stitching_b200.plan import flatten_chain
 from oracle import camera_weight_model, stitcher_ref
+from random_rigs import random_chain
 
 CASES = [  # cameras, height, width, channels, super mode, map kind
     (2, 64, 96, 3, False, "random"), (3, 90, 160, 1, False, "binary"), (4, 72, 120, 4, False, "ramp"),
@@ -29,6 +30,26 @@ def test_layer_model_equals_the_cv2_chain(n, h, w, c, super_mode, kind):
     assert got.shape == ref.shape == stitcher_ref.stitch_chain(states, labels, images).shape
     assert np.array_equal(got, ref)
     assert sum(contrib) > 0 and most >= 1
+
+
+@pytest.mark.parametrize("seed", range(28))
+def test_layer_model_equals_the_cv2_chain_on_random_rigs(seed):
+    """The seeded random rigs of the overwrite fuzz (rotations, anisotropic scales, perspective, mirrored cameras,
+    odd widths, 1/3/4 channels), super-mode crops trimmed so that they keep several cameras, under every map kind.
+    ``most`` is held against a per-pixel count of the cv2 chain's planes."""
+    made = random_chain(seed, trim=SUPER_TRIM)
+    if made is None:
+        pytest.skip("degenerate canvas for this seed")
+    st, states, labels, images = made
+    for kind in MAP_KINDS:
+        maps = make_maps(images, labels, kind, seed=seed)
+        got, contrib, most = layer_model(st, labels, images, maps)
+        planes = camera_weight_model.chain_planes(states, labels, images, maps)
+        ref = camera_weight_model.chain(states, labels, images, maps)
+        assert got.shape == ref.shape and np.array_equal(got, ref), kind
+        count = sum((r & (w > 0)).astype(np.int64) for _, w, r in planes)
+        assert most == int(count.max()) and sum(contrib) == int(count.sum()), kind
+        assert 1 <= most <= camera_weight_model.MAX_CONTRIBUTORS, kind
 
 
 @pytest.mark.parametrize("j", [0, 1, 2])
