@@ -108,6 +108,29 @@ def test_feather_super_mode_crops_after_the_blended_paste():
     assert np.array_equal(soft[:, :20], hard[:, :20])
 
 
+@pytest.mark.parametrize("seed", range(28))
+def test_specification_reduces_to_the_overwrite_on_random_rigs(seed):
+    """On the seeded random rigs (super-mode crops cutting the pasted rectangles): a one-pixel feather and maps
+    of F everywhere are the reference's overwrite, and map values above F count as F."""
+    from feather_cases import make_maps, rig, stage_shapes
+    made = rig(seed)
+    if made is None:
+        pytest.skip("degenerate canvas for this seed")
+    st, states, labels, images = made
+    hard = stitcher_ref.stitch_chain(states, labels, images)
+    assert np.array_equal(feather_model.feather_chain(states, labels, images, 0), hard)
+    log2 = 1 + seed % 5
+    shapes = stage_shapes(st, images, labels)
+    full = make_maps(shapes, log2, "full")
+    assert np.array_equal(feather_model.feather_chain(states, labels, images, log2, full), hard)
+    over = make_maps(shapes, log2, "over", seed=seed)
+    assert all(m.max() > (1 << log2) for m in over)
+    clipped = [np.minimum(m, 1 << log2).astype(np.uint8) for m in over]
+    soft = feather_model.feather_chain(states, labels, images, log2, over)
+    assert np.array_equal(soft, feather_model.feather_chain(states, labels, images, log2, clipped))
+    assert (soft != hard).any()
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("n,h,w,c,log2", [
     (2, 64, 96, 3, 2), (3, 120, 200, 3, 3), (4, 90, 160, 1, 4), (4, 90, 160, 4, 1), (6, 270, 480, 3, 5),
