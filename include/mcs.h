@@ -140,7 +140,7 @@ int mcs_plan_owned_pixels(const mcs_plan* plan, int64_t* owned_host, void* cuda_
  * the window cannot influence the panorama - they belong to the part of the camera that the
  * reference's paste (StitcherClass.py:240-241) overwrites - so a host-facing caller needs to
  * bring only the window onto the device.  Whole frames when the windows are not known (no tile
- * table, feather mode, camera weights).
+ * table, feather mode, camera weights, multi-band blend).
  */
 int mcs_plan_source_windows(const mcs_plan* plan, int32_t* xyxy);
 
@@ -269,10 +269,39 @@ int mcs_plan_set_blend(mcs_plan* plan, int feather_log2, const int32_t* paste_xy
  */
 int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_maps, const int64_t* map_pitch);
 
+/*
+ * mcs_plan_set_multiband - the multi-band blend of the camera-weighted panorama: OpenCV's
+ * cv::detail::MultiBandBlender(try_gpu = 0, num_bands, CV_16S), bit for bit.  Every layer k with a
+ * non-empty visible rectangle feeds v_k (as int16) with the mask w_k (both as defined for
+ * mcs_plan_set_camera_weights) at the rectangle's corner, innermost first, into a blender prepared
+ * for (0, 0, out_w, out_h); the output is the blended int16 image saturated to u8, 0 where the mask
+ * of blend() is 0.  Low frequencies mix over a wide region and fine detail over a narrow one, which
+ * hides seams between cameras of different exposure.  Specification in oracle/multiband_model.py.
+ *
+ * The plan must hold camera weights (mcs_plan_set_camera_weights; a rig that call refused only
+ * because more than 4 cameras meet at a pixel counts: this mode has no contributor limit), else
+ * MCS_ERR_INVALID.  num_bands = 0 goes back to the camera-weighted blend (the overwrite for such a
+ * refused rig); 1..8 switch the mode on; anything else fails with MCS_ERR_INVALID.  The effective
+ * count is clamped as MultiBandBlender::prepare does, to ceil(log2(max(out_w, out_h))), and
+ * mcs_plan_multiband_bands reads it back (0 while the mode is off).  mcs_plan_set_camera_weights, and
+ * clearing the weights, switch the mode off; the stage-wise blend of mcs_plan_set_blend excludes it.
+ *
+ * The weight pyramids are built here, once, on the device.  The plan also keeps a workspace for the
+ * per-frame camera and panorama pyramids of MCS_MB_FRAMES frame-sets - 2 bytes * C * (sum over
+ * cameras and levels of the feed regions' pixels + sum over levels >= 1 of the padded panorama's
+ * pixels) per frame-set - and mcs_stitch_u8 runs the frames in sub-batches of that size, 2n + 2
+ * launches each for n effective bands.  mcs_stitch_u8 reports variant 6; forcing the gather or tiled
+ * variant fails with MCS_ERR_UNSUPPORTED; mcs_plan_source_windows / _spans report whole frames.
+ * Synchronous.
+ */
+#define MCS_MB_FRAMES 16
+int mcs_plan_set_multiband(mcs_plan* plan, int num_bands);
+int mcs_plan_multiband_bands(const mcs_plan* plan);
+
 /* Which kernel variant the last mcs_stitch_u8 on this plan launched
  * (diagnostics for tests / bench): 0 = none yet, 1 = gather, 2 = tiled, 3 = overwrite pass +
  * feather band pass, 4 = tiled with the seam bands blended in the same launch, 5 = camera-weighted
- * blend (mcs_plan_set_camera_weights). */
+ * blend (mcs_plan_set_camera_weights), 6 = multi-band blend (mcs_plan_set_multiband). */
 int mcs_plan_last_variant(const mcs_plan* plan);
 
 /* Pin the kernel variant of a plan: 0 = automatic (tiled when the plan and the buffers allow

@@ -69,6 +69,11 @@ class Stitcher(Debugger):
     # missing label likewise.  None (the default) keeps the reference's overwrite.  ``edge_ramp`` gives the
     # FeatherBlender-style map.
     camera_weights = None
+    # Optional multi-band blend of the camera weights (extension, include/mcs.h mcs_plan_set_multiband): 0 (the
+    # default) = off, 1..8 = the Laplacian-pyramid blend of OpenCV's MultiBandBlender with that many bands (clamped
+    # to ceil(log2) of the panorama's longer side).  ``camera_weights`` supplies the masks; without them every camera
+    # weighs 255 everywhere.
+    blend_bands = 0
 
     def __init__(self, images_dic, super_mode=False):
         # labels sorted like np.sort(images_dic.keys()) (reference :61)
@@ -148,7 +153,7 @@ class Stitcher(Debugger):
         frames = [images_dic[label] for label in self.img_labels]
         out = _composite(self._engine_(), self.stitchers, frames, batched=False, debugger=self,
                          feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
-                         camera_weights=self._camera_weight_list())
+                         camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands())
         if draw_descriptors and not _is_tensor(out):
             out = self._draw_overlays(out, frames)
         return out
@@ -192,21 +197,31 @@ class Stitcher(Debugger):
         frames = [frames_dic[label] for label in self.img_labels]
         return _composite(self._engine_(), self.stitchers, frames, batched=True, out=out, debugger=self,
                           feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
-                          camera_weights=self._camera_weight_list())
+                          camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands())
 
     def plan(self, img_shapes, device=None):
         """Compiled plan (``engine.CompiledPlan``) for frames of these shapes."""
         return self._engine_().plan_for(self.stitchers, [tuple(s) for s in img_shapes], device,
                                         feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
-                                        camera_weights=self._camera_weight_list())
+                                        camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands())
+
+    def _blend_bands(self):
+        """``blend_bands`` checked: an int in 0..8."""
+        n = self.blend_bands
+        if isinstance(n, bool) or not isinstance(n, (int, np.integer)) or not 0 <= int(n) <= 8:
+            raise ValueError("blend_bands must be an integer in 0..8, got %r" % (n,))
+        return int(n)
 
     def _camera_weight_list(self):
-        """``camera_weights`` checked and as a list in camera order, or None when the mode is off."""
+        """``camera_weights`` checked and as a list in camera order, or None when the mode is off (with
+        ``blend_bands`` > 0 and no ``camera_weights``: 255 everywhere for every camera)."""
         cw = self.camera_weights
+        if cw is None and self._blend_bands():
+            cw = {}
         if cw is None:
             return None
         if getattr(self, "feather_log2", 0) or self.blend_weights is not None:
-            raise ValueError("camera_weights cannot be combined with feather_log2 / blend_weights")
+            raise ValueError("camera_weights / blend_bands cannot be combined with feather_log2 / blend_weights")
         by_label = {str(k): v for k, v in dict(cw).items()}
         labels = [str(l) for l in self.img_labels]
         unknown = sorted(set(by_label) - set(labels))
@@ -546,9 +561,9 @@ def edge_ramp(shape, width=64):
 
 
 def _composite(engine, stages, frames, batched, out=None, debugger=None, feather_log2=0, blend_weights=None,
-               camera_weights=None):
+               camera_weights=None, blend_bands=0):
     """Run the fused kernel for this chain on these frames.  ``camera_weights``: one entry per camera (None or
-    a uint8 map) for the camera-weighted blend, or None."""
+    a uint8 map) for the camera-weighted blend, or None; ``blend_bands`` > 0 blends them in that many bands."""
     import torch  # local: keeps `import StitcherClass` cheap for calibration-only users
 
     on_device = _is_tensor(frames[0]) and frames[0].is_cuda
@@ -572,7 +587,7 @@ def _composite(engine, stages, frames, batched, out=None, debugger=None, feather
                                       "resized at stage %d" % segs[1]["a"])
             return engine.plan_for(sub_stages, sub_shapes, device, feather_log2=feather_log2,
                                    blend_weights=[weight_of.get(id(st)) for st in sub_stages] if weight_of else None,
-                                   camera_weights=camera_weights)
+                                   camera_weights=camera_weights, blend_bands=blend_bands)
         except PlanUnsupported as e:
             if debugger is not None:
                 debugger.debugger(DEBUG_LEVEL_0, "[STITCHER] {}".format(e), log_type="err")

@@ -17,20 +17,26 @@ MCS_MAX_LAYERS = 16
 MCS_LAYER_COPY = 0
 MCS_LAYER_WARP = 1
 MCS_LAYER_REMAP = 2
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 # every symbol include/mcs.h declares
 EXPORTS = (
     "mcs_abi_version", "mcs_last_error", "mcs_plan_create", "mcs_plan_create_maps", "mcs_plan_destroy",
-    "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_set_camera_weights", "mcs_plan_last_variant",
+    "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_set_camera_weights",
+    "mcs_plan_set_multiband", "mcs_plan_multiband_bands", "mcs_plan_last_variant",
     "mcs_plan_force_variant", "mcs_plan_rows_need_padding", "mcs_plan_promise_padded_rows",
     "mcs_plan_tiled_status", "mcs_plan_tiled_ctas_per_sm", "mcs_plan_tiled_stats", "mcs_launch_count",
     "mcs_match_hamming_top2", "mcs_match_l2_top2", "mcs_ransac_homography", "mcs_refit_homography", "mcs_resize_linear_u8",
 )
 
 
+MCS_ERR_UNSUPPORTED = -3
+
+
 class McsError(RuntimeError):
-    pass
+    def __init__(self, msg, code=None):
+        RuntimeError.__init__(self, msg)
+        self.code = code
 
 
 _lib = None
@@ -102,6 +108,10 @@ def load(build_if_missing=False):
     lib.mcs_plan_set_blend.argtypes = [_vp, ctypes.c_int, _c_i32p, ctypes.POINTER(ctypes.c_void_p), _c_i64p]
     lib.mcs_plan_set_camera_weights.restype = ctypes.c_int
     lib.mcs_plan_set_camera_weights.argtypes = [_vp, ctypes.POINTER(ctypes.c_void_p), _c_i64p]
+    lib.mcs_plan_set_multiband.restype = ctypes.c_int
+    lib.mcs_plan_set_multiband.argtypes = [_vp, ctypes.c_int]
+    lib.mcs_plan_multiband_bands.restype = ctypes.c_int
+    lib.mcs_plan_multiband_bands.argtypes = [_vp]
     lib.mcs_plan_tiled_ctas_per_sm.restype = ctypes.c_int
     lib.mcs_plan_tiled_ctas_per_sm.argtypes = [_vp]
     lib.mcs_plan_tiled_status.restype = ctypes.c_char_p
@@ -130,7 +140,7 @@ def load(build_if_missing=False):
 def check(rc, what):
     if rc != MCS_OK:
         msg = load().mcs_last_error().decode(errors="replace")
-        raise McsError("%s failed (code %d): %s" % (what, rc, msg))
+        raise McsError("%s failed (code %d): %s" % (what, rc, msg), rc)
 
 
 def launch_count():
@@ -245,6 +255,8 @@ class Plan(object):
         self.src_hw = hw.copy()
         self._owned = None
         self.camera_weighted = False   # set_camera_weights is in force
+        self.multiband = False         # set_multiband is in force
+        self.blend_bands = 0           # its effective band count
 
     def close(self):
         if getattr(self, "_h", None) is not None and _lib is not None:
@@ -336,6 +348,7 @@ class Plan(object):
         """``weight_maps``: None (the plain overwrite) or a list of n_layers entries, each None (255 everywhere)
         or a uint8 array of that layer's source (height, width): the camera-weighted blend (include/mcs.h)."""
         n = self.n_layers
+        self.multiband, self.blend_bands = False, 0   # every call switches the multi-band blend off
         if weight_maps is None:
             check(_lib.mcs_plan_set_camera_weights(self._h, None, None), "mcs_plan_set_camera_weights")
             self._owned = None
@@ -361,6 +374,15 @@ class Plan(object):
         check(_lib.mcs_plan_set_camera_weights(self._h, ptrs, pitches.ctypes.data_as(_c_i64p)),
               "mcs_plan_set_camera_weights")
         self.camera_weighted = True
+
+    def set_multiband(self, num_bands):
+        """The multi-band blend of the camera weights (include/mcs.h mcs_plan_set_multiband); 0 switches it
+        off.  Returns the effective band count."""
+        self.multiband, self.blend_bands = False, 0
+        check(_lib.mcs_plan_set_multiband(self._h, int(num_bands)), "mcs_plan_set_multiband")
+        self.multiband = int(num_bands) > 0
+        self.blend_bands = int(_lib.mcs_plan_multiband_bands(self._h))
+        return self.blend_bands
 
     def tiled_ctas_per_sm(self):
         return int(_lib.mcs_plan_tiled_ctas_per_sm(self._h))

@@ -14,7 +14,7 @@ REPO_DIR = os.path.dirname(PKG_DIR)
 CSRC_DIR = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libmcs_b200.so")
 
-SOURCES = ["mcs_plan.cu", "mcs_tiles.cu", "mcs_stitch.cu", "mcs_stitch_tiled.cu", "mcs_stitch_weighted.cu", "mcs_match.cu", "mcs_ransac.cu", "mcs_resize.cu", "mcs_hostio.cu", "mcs_refit.cu"]
+SOURCES = ["mcs_plan.cu", "mcs_tiles.cu", "mcs_stitch.cu", "mcs_stitch_tiled.cu", "mcs_stitch_weighted.cu", "mcs_stitch_multiband.cu", "mcs_match.cu", "mcs_ransac.cu", "mcs_resize.cu", "mcs_hostio.cu", "mcs_refit.cu"]
 HEADERS = [os.path.join(CSRC_DIR, "mcs_common.h"), os.path.join(CSRC_DIR, "mcs_device.cuh"),
            os.path.join(REPO_DIR, "include", "mcs.h")]
 

@@ -8,7 +8,7 @@
 
 #include "mcs.h"
 
-#define MCS_ABI_VERSION 2
+#define MCS_ABI_VERSION 3
 
 // ---- error plumbing -------------------------------------------------------
 void mcs_set_error(const char* fmt, ...);
@@ -165,6 +165,13 @@ struct mcs_plan {
     int cw_active;           // the plan blends every camera that sees a pixel, normalised by the summed weights
     uint8_t* d_cwmap[MCS_MAX_LAYERS];   // per layer: device weight map, src_h x src_w bytes (nullptr = 255 everywhere)
     long long cw_contrib[MCS_MAX_LAYERS];   // per layer: output pixels it contributes to
+    int cw_maps;             // the maps of the last mcs_plan_set_camera_weights are held: also when the rig was refused
+                             // for the camera-weighted kernel (more than MCS_CW_MAX_CONTRIB contributors), since the
+                             // multi-band blend takes such rigs
+    // multi-band blend (mcs_plan_set_multiband, mcs_stitch_multiband.cu)
+    int mb_on;               // the multi-band blend serves the plan
+    int mb_bands;            // its effective band count (clamped like MultiBandBlender::prepare)
+    struct McsMultiband* mb; // geometry, weight pyramids and workspace
 };
 
 
@@ -189,6 +196,15 @@ int mcs_camera_weights_count(const mcs_plan* plan, long long* contrib, int* max_
 int mcs_launch_weighted(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,
                         const int64_t* fstride, int n_frames, uint8_t* dst, int64_t dst_pitch,
                         int64_t dst_frame_stride, cudaStream_t stream);
+
+// Multi-band blend (mcs_stitch_multiband.cu): at most this many pyramid levels (8 bands + the top)
+#define MCS_MB_MAX_LEVELS 9
+// Builds the geometry, the weight pyramids and sums of the plan's held camera maps and the workspace for
+// `bands` requested bands (synchronous); frees them.
+int mcs_multiband_build(mcs_plan* plan, int bands);
+void mcs_multiband_free(mcs_plan* plan);
+int mcs_launch_multiband(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch, const int64_t* fstride,
+                         int n_frames, uint8_t* dst, int64_t dst_pitch, int64_t dst_frame_stride, cudaStream_t stream);
 
 // Tiled variant (mcs_stitch_tiled.cu): why it cannot serve a call (nullptr = it can), and its launch.
 const char* mcs_tiled_blocker(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,

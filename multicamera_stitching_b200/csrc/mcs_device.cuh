@@ -40,6 +40,22 @@ __device__ __forceinline__ void fixed_coords(double m0, double m3, double m6, co
 // saturate_cast<short> of the integer part of a 1/32-px coordinate
 __device__ __forceinline__ int sat16(int v) { return max(-32768, min(32767, v)); }
 
+// Fixed-point bilinear sample of one uint8 weight map (w x h, no pitch) at (X, Y), 1/32 px; taps outside the map read 0,
+// a missing map reads 255 inside.
+__device__ __forceinline__ int weight_sample(const uint8_t* __restrict__ m, int w, int h, int X, int Y) {
+    const int sx = sat16(X >> 5), sy = sat16(Y >> 5), ax = X & 31, ay = Y & 31;
+    const bool x0in = (unsigned)sx < (unsigned)w, x1in = (unsigned)(sx + 1) < (unsigned)w;
+    const bool y0in = (unsigned)sy < (unsigned)h, y1in = (unsigned)(sy + 1) < (unsigned)h;
+    const uint8_t* r0 = m + (long long)sy * w + sx;
+    int p00 = 0, p01 = 0, p10 = 0, p11 = 0;
+    if (y0in && x0in) p00 = m ? __ldg(r0) : 255;
+    if (y0in && x1in) p01 = m ? __ldg(r0 + 1) : 255;
+    if (y1in && x0in) p10 = m ? __ldg(r0 + w) : 255;
+    if (y1in && x1in) p11 = m ? __ldg(r0 + w + 1) : 255;
+    return ((32 - ay) * (32 - ax) * 32 * p00 + (32 - ay) * ax * 32 * p01 + ay * (32 - ax) * 32 * p10 +
+            ay * ax * 32 * p11 + 16384) >> 15;
+}
+
 // Some of the four bilinear taps at 1/32-px (X, Y) lies inside the layer's source (otherwise the
 // sample is BORDER_CONSTANT 0 and the layer does not touch the pixel).
 __device__ __forceinline__ bool some_tap_inside(const McsLayer& g, int X, int Y) {

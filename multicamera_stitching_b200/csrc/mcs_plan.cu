@@ -216,6 +216,7 @@ extern "C" int mcs_plan_destroy(mcs_plan* plan) {
         if (plan->d_wmap[k]) cudaFree(plan->d_wmap[k]);
         if (plan->d_cwmap[k]) cudaFree(plan->d_cwmap[k]);
     }
+    mcs_multiband_free(plan);
     mcs_plan_free_tiles(plan);
     free_maps(plan);
     delete plan;
@@ -235,8 +236,9 @@ extern "C" int mcs_plan_source_windows(const mcs_plan* plan, int32_t* xyxy) {
     MCS_CHECK_ARG(plan != nullptr && xyxy != nullptr, "mcs_plan_source_windows: NULL argument");
     // The feather band samples outer cameras inside the pasted rectangles, i.e. outside the
     // pixels they own: there every frame counts in full.
-    // The camera-weighted blend samples every camera wherever its rectangle reaches: whole frames too.
-    const bool known = plan->src_win_valid && !plan->cw_active &&
+    // The camera-weighted and multi-band blends sample every camera wherever its rectangle reaches:
+    // whole frames too.
+    const bool known = plan->src_win_valid && !plan->cw_active && !plan->mb_on &&
                        ((plan->feather_log2 == 0 && !plan->blend_custom) || plan->band_fused);
     for (int k = 0; k < plan->n_layers; ++k) {
         xyxy[4 * k + 0] = known ? plan->src_win[k][0] : 0;
@@ -254,7 +256,7 @@ extern "C" int mcs_plan_source_spans(const mcs_plan* plan, int layer, int band_r
     const McsLayer& L = plan->layers[layer];
     const int n_bands = (L.src_h + band_rows - 1) / band_rows;
     const int* span = plan->h_row_span[layer];
-    const bool known = plan->src_win_valid && !plan->cw_active &&
+    const bool known = plan->src_win_valid && !plan->cw_active && !plan->mb_on &&
                        ((plan->feather_log2 == 0 && !plan->blend_custom) || plan->band_fused) && span != nullptr;
     for (int b = 0; b < n_bands; ++b) {
         int x0 = known ? INT_MAX : 0, x1 = known ? INT_MIN : L.src_w;
@@ -372,7 +374,7 @@ extern "C" int mcs_plan_set_blend(mcs_plan* plan, int feather_log2, const int32_
     MCS_CHECK_ARG(!any_map || map_pitch != nullptr, "mcs_plan_set_blend: weight maps without their pitches");
     MCS_CHECK_ARG(!any_map || feather_log2 <= MCS_BAND_MAX_LOG2,
                   "mcs_plan_set_blend: weight maps take feather_log2 <= %d (got %d)", MCS_BAND_MAX_LOG2, feather_log2);
-    MCS_CHECK_ARG(!plan->cw_active || (feather_log2 == 0 && !any_map),
+    MCS_CHECK_ARG(!(plan->cw_active || plan->mb_on) || (feather_log2 == 0 && !any_map),
                   "mcs_plan_set_blend: the plan blends with camera weights; clear them first");
     free_strips(plan);
     free_wmaps(plan);
@@ -501,6 +503,9 @@ static void free_cwmaps(mcs_plan* plan) {
         plan->d_cwmap[k] = nullptr;
     }
     plan->cw_active = 0;
+    plan->cw_maps = 0;
+    plan->mb_on = 0;
+    mcs_multiband_free(plan);
 }
 
 extern "C" int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_maps, const int64_t* map_pitch) {
@@ -535,8 +540,8 @@ extern "C" int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const*
         free_cwmaps(plan);
         return rc;
     }
-    if (most > MCS_CW_MAX_CONTRIB) {
-        free_cwmaps(plan);
+    plan->cw_maps = 1;
+    if (most > MCS_CW_MAX_CONTRIB) {   // the maps stay held for mcs_plan_set_multiband
         mcs_set_error("mcs_plan_set_camera_weights: %d cameras with non-zero weight meet at one output pixel (at most %d "
                       "blend); lower the weights of some of them there", most, MCS_CW_MAX_CONTRIB);
         return MCS_ERR_UNSUPPORTED;
@@ -544,3 +549,21 @@ extern "C" int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const*
     plan->cw_active = 1;
     return MCS_OK;
 }
+
+extern "C" int mcs_plan_set_multiband(mcs_plan* plan, int num_bands) {
+    MCS_CHECK_ARG(plan != nullptr, "mcs_plan_set_multiband: plan is NULL");
+    MCS_CHECK_ARG(num_bands >= 0 && num_bands <= MCS_MB_MAX_LEVELS - 1, "mcs_plan_set_multiband: num_bands=%d outside 0..%d",
+                  num_bands, MCS_MB_MAX_LEVELS - 1);
+    MCS_CHECK_ARG(plan->cw_maps, "mcs_plan_set_multiband: the plan has no camera weights (mcs_plan_set_camera_weights)");
+    MCS_CHECK_ARG(plan->feather_log2 == 0 && !plan->blend_custom,
+                  "mcs_plan_set_multiband: the plan feathers its pastes (mcs_plan_set_blend); switch that off first");
+    plan->mb_on = 0;
+    mcs_multiband_free(plan);
+    if (num_bands == 0) return MCS_OK;
+    const int rc = mcs_multiband_build(plan, num_bands);
+    if (rc != MCS_OK) return rc;
+    plan->mb_on = 1;
+    return MCS_OK;
+}
+
+extern "C" int mcs_plan_multiband_bands(const mcs_plan* plan) { return plan && plan->mb_on ? plan->mb_bands : 0; }

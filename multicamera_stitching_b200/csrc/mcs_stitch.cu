@@ -439,6 +439,17 @@ extern "C" int mcs_stitch_u8(const mcs_plan* plan_c, const uint8_t* const* src,
     }
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     const int force = plan->force_variant;
+    if (plan->mb_on) {
+        if (force != 0) {
+            mcs_set_error("mcs_stitch_u8: %s variant forced but unavailable: the plan blends in bands",
+                          force == 1 ? "gather" : "tiled");
+            return MCS_ERR_UNSUPPORTED;
+        }
+        const int rc = mcs_launch_multiband(plan, src, src_pitch_bytes, src_frame_stride, n_frames, dst, dst_pitch_bytes,
+                                            dst_frame_stride, stream);
+        if (rc == MCS_OK) plan->last_variant = 6;
+        return rc;
+    }
     if (plan->cw_active) {
         if (force == 2) {
             mcs_set_error("mcs_stitch_u8: tiled variant forced but unavailable: the plan blends with camera weights");
@@ -507,7 +518,7 @@ extern "C" int mcs_stitch_u8(const mcs_plan* plan_c, const uint8_t* const* src,
 
 extern "C" int mcs_plan_owned_pixels(const mcs_plan* plan, int64_t* owned_host, void* cuda_stream) {
     MCS_CHECK_ARG(plan != nullptr && owned_host != nullptr, "mcs_plan_owned_pixels: NULL argument");
-    if (plan->cw_active) {   // counted when the weights were set
+    if (plan->cw_active || plan->mb_on) {   // counted when the weights were set
         for (int k = 0; k < plan->n_layers; ++k) owned_host[k] = (int64_t)plan->cw_contrib[k];
         return MCS_OK;
     }

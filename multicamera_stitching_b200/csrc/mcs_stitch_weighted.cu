@@ -36,22 +36,6 @@ struct CwArgs {
 #define CW_BY 4
 #define CW_FRAMES 16   // frames per thread (grid.z covers the rest)
 
-// Fixed-point bilinear sample of one weight map at (X, Y), 1/32 px; taps outside the map read 0,
-// a missing map reads 255 inside.
-__device__ __forceinline__ int weight_sample(const uint8_t* __restrict__ m, int w, int h, int X, int Y) {
-    const int sx = sat16(X >> 5), sy = sat16(Y >> 5), ax = X & 31, ay = Y & 31;
-    const bool x0in = (unsigned)sx < (unsigned)w, x1in = (unsigned)(sx + 1) < (unsigned)w;
-    const bool y0in = (unsigned)sy < (unsigned)h, y1in = (unsigned)(sy + 1) < (unsigned)h;
-    const uint8_t* r0 = m + (long long)sy * w + sx;
-    int p00 = 0, p01 = 0, p10 = 0, p11 = 0;
-    if (y0in && x0in) p00 = m ? __ldg(r0) : 255;
-    if (y0in && x1in) p01 = m ? __ldg(r0 + 1) : 255;
-    if (y1in && x0in) p10 = m ? __ldg(r0 + w) : 255;
-    if (y1in && x1in) p11 = m ? __ldg(r0 + w + 1) : 255;
-    return ((32 - ay) * (32 - ax) * 32 * p00 + (32 - ay) * ax * 32 * p01 + ay * (32 - ax) * 32 * p10 +
-            ay * ax * 32 * p11 + 16384) >> 15;
-}
-
 // One contributor: tap address of the launch's first frame, packed 16-bit tap weights for IDP.2A,
 // and meta = tap-inside flags (bits 0..3: 00, 01, 10, 11) | word path (bit 4) | layer << 8 | w_k << 16.
 struct Contrib {

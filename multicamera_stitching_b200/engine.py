@@ -87,7 +87,7 @@ class PinnedResults(object):
 class CompiledPlan(object):
     """A flattened chain plus its ``mcs_plan`` on one device."""
 
-    def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None):
+    def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None, blend_bands=0):
         self.flat = flat
         self.device = torch.device(device)
         self.feather_log2 = int(feather_log2)
@@ -106,8 +106,16 @@ class CompiledPlan(object):
                 # the paste rectangles matter only when a super-mode crop cut a visible one
                 self.handle.set_blend(self.feather_log2, plan_paste(flat), maps)
             if camera_weights is not None:   # one map per camera, in the layer order of the plan
-                self.handle.set_camera_weights([camera_weights[l.cam] if l.cam < len(camera_weights) else None
-                                                for l in flat.layers])
+                try:
+                    self.handle.set_camera_weights([camera_weights[l.cam] if l.cam < len(camera_weights) else None
+                                                    for l in flat.layers])
+                except _cabi.McsError as e:
+                    # more than 4 cameras meet at a pixel: the single-band kernel refuses the rig, the
+                    # multi-band blend takes it (the library keeps the maps for it)
+                    if not blend_bands or e.code != _cabi.MCS_ERR_UNSUPPORTED:
+                        raise
+                if blend_bands:
+                    self.handle.set_multiband(blend_bands)
             # rows that are not a multiple of 4 bytes: run() always passes them through its
             # zero-padded scratch buffers, which is what the tiled kernel needs to serve them
             self.pad_rows = self._tiled() and self.handle.rows_need_padding()
@@ -117,8 +125,8 @@ class CompiledPlan(object):
         self.out_w, self.out_h, self.channels = flat.out_w, flat.out_h, flat.channels
 
     def _tiled(self):
-        """Whether the tiled kernel serves this plan (it does not serve the camera-weighted blend)."""
-        return self.handle.tiled_status() == "" and not self.handle.camera_weighted
+        """Whether the tiled kernel serves this plan (it does not serve the camera-weighted blends)."""
+        return self.handle.tiled_status() == "" and not (self.handle.camera_weighted or self.handle.multiband)
 
     # ---- geometry helpers -------------------------------------------------
     def out_shape(self, n_frames=None):
@@ -272,7 +280,8 @@ class CompositeEngine(object):
             self._device = torch.device("cuda", torch.cuda.current_device())
         return torch.device(self._device)
 
-    def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None, camera_weights=None):
+    def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None, camera_weights=None,
+                 blend_bands=0):
         """Compiled plan for this chain state and these frame shapes, or None
         when no stage is calibrated (decided on the host, no device needed)."""
         shapes = tuple(tuple(int(v) for v in s) for s in cam_shapes)
@@ -289,14 +298,15 @@ class CompositeEngine(object):
         if camera_weights is not None:
             ckey = tuple(None if w is None else (np.asarray(w).shape, hash(np.ascontiguousarray(w, dtype=np.uint8).tobytes()))
                          for w in camera_weights)
-        key = (str(device), shapes, sig, feather_log2, wkey, ckey)
+        blend_bands = int(blend_bands or 0)
+        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands)
         if key in self._plans:
             self._plans[key] = self._plans.pop(key)      # most recently used last
         else:
             flat = flatten_chain(stages, shapes)
             while len(self._plans) >= self.max_plans:     # evict the least recently used, one at a time
                 self._plans.pop(next(iter(self._plans)))
-            self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights)
+            self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights, blend_bands)
                                 if flat is not None else None)
         return self._plans[key]
 
