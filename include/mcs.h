@@ -298,6 +298,30 @@ int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_map
 int mcs_plan_set_multiband(mcs_plan* plan, int num_bands);
 int mcs_plan_multiband_bands(const mcs_plan* plan);
 
+/*
+ * mcs_plan_set_voronoi_seams - cut the masks of the multi-band blend at Voronoi seams first, as OpenCV's
+ * stitching pipeline does with cv::detail::VoronoiSeamFinder, bit for bit.  The finder runs on the layers that
+ * feed the blend (non-empty visible rectangle, innermost first) with their rectangles and the masks w_k: for
+ * every pair i < j whose rectangles overlap, in that order and on the masks earlier pairs cut, each pixel of the
+ * overlap goes to the camera whose own (non-overlapping) mask pixels lie nearer in the L1 metric, ties to the
+ * later camera, and is zeroed in the other.  Each overlap pixel then belongs to one camera: fine detail comes from
+ * that camera alone and only the low bands mix across the seam, so cameras that disagree (parallax, calibration
+ * residue) no longer leave a double image.  Specification in oracle/seam_model.py.
+ *
+ * The seams depend on the calibration only: they are found here, once, on the device (one launch to sample the
+ * weights, two per overlapping pair), and the weight pyramids and sums are rebuilt from the cut masks; the
+ * per-frame work of mcs_stitch_u8 (variant 6) does not change.  enable = 0 goes back to the full masks.  Requires
+ * the multi-band blend (mcs_plan_set_multiband), else MCS_ERR_INVALID.  The finder works in submasks of the
+ * overlap grown by 10 pixels on every side; one of W + H >= 32768 fails with MCS_ERR_UNSUPPORTED and leaves the
+ * plan as it was.  mcs_plan_set_multiband and mcs_plan_set_camera_weights switch the seams off.  Synchronous.
+ *
+ * mcs_plan_seam_weights - reads back the seam-cut mask of layer `layer` over its visible rectangle clipped to the
+ * panorama (host uint8, rows dst_pitch bytes apart); MCS_ERR_INVALID while the seams are off or for a layer that
+ * feeds nothing.
+ */
+int mcs_plan_set_voronoi_seams(mcs_plan* plan, int enable);
+int mcs_plan_seam_weights(const mcs_plan* plan, int layer, uint8_t* host_dst, int64_t dst_pitch);
+
 /* Which kernel variant the last mcs_stitch_u8 on this plan launched
  * (diagnostics for tests / bench): 0 = none yet, 1 = gather, 2 = tiled, 3 = overwrite pass +
  * feather band pass, 4 = tiled with the seam bands blended in the same launch, 5 = camera-weighted

@@ -74,6 +74,10 @@ class Stitcher(Debugger):
     # to ceil(log2) of the panorama's longer side).  ``camera_weights`` supplies the masks; without them every camera
     # weighs 255 everywhere.
     blend_bands = 0
+    # Optional Voronoi seams for the multi-band blend (extension, include/mcs.h mcs_plan_set_voronoi_seams): True cuts
+    # every overlap at OpenCV's VoronoiSeamFinder seam before the blend, so that each overlap pixel takes its fine
+    # detail from one camera and only the low bands mix across the seam.  Needs ``blend_bands`` > 0.
+    voronoi_seams = False
 
     def __init__(self, images_dic, super_mode=False):
         # labels sorted like np.sort(images_dic.keys()) (reference :61)
@@ -153,7 +157,8 @@ class Stitcher(Debugger):
         frames = [images_dic[label] for label in self.img_labels]
         out = _composite(self._engine_(), self.stitchers, frames, batched=False, debugger=self,
                          feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
-                         camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands())
+                         camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
+                         voronoi_seams=self._voronoi_seams())
         if draw_descriptors and not _is_tensor(out):
             out = self._draw_overlays(out, frames)
         return out
@@ -197,13 +202,15 @@ class Stitcher(Debugger):
         frames = [frames_dic[label] for label in self.img_labels]
         return _composite(self._engine_(), self.stitchers, frames, batched=True, out=out, debugger=self,
                           feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
-                          camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands())
+                          camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
+                          voronoi_seams=self._voronoi_seams())
 
     def plan(self, img_shapes, device=None):
         """Compiled plan (``engine.CompiledPlan``) for frames of these shapes."""
         return self._engine_().plan_for(self.stitchers, [tuple(s) for s in img_shapes], device,
                                         feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
-                                        camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands())
+                                        camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
+                          voronoi_seams=self._voronoi_seams())
 
     def _blend_bands(self):
         """``blend_bands`` checked: an int in 0..8."""
@@ -211,6 +218,15 @@ class Stitcher(Debugger):
         if isinstance(n, bool) or not isinstance(n, (int, np.integer)) or not 0 <= int(n) <= 8:
             raise ValueError("blend_bands must be an integer in 0..8, got %r" % (n,))
         return int(n)
+
+    def _voronoi_seams(self):
+        """``voronoi_seams`` checked: a bool, True only with ``blend_bands`` > 0."""
+        v = self.voronoi_seams
+        if not isinstance(v, (bool, np.bool_)):
+            raise ValueError("voronoi_seams must be True or False, got %r" % (v,))
+        if v and not self._blend_bands():
+            raise ValueError("voronoi_seams cuts the masks of the multi-band blend: set blend_bands > 0 too")
+        return bool(v)
 
     def _camera_weight_list(self):
         """``camera_weights`` checked and as a list in camera order, or None when the mode is off (with
@@ -561,9 +577,10 @@ def edge_ramp(shape, width=64):
 
 
 def _composite(engine, stages, frames, batched, out=None, debugger=None, feather_log2=0, blend_weights=None,
-               camera_weights=None, blend_bands=0):
+               camera_weights=None, blend_bands=0, voronoi_seams=False):
     """Run the fused kernel for this chain on these frames.  ``camera_weights``: one entry per camera (None or
-    a uint8 map) for the camera-weighted blend, or None; ``blend_bands`` > 0 blends them in that many bands."""
+    a uint8 map) for the camera-weighted blend, or None; ``blend_bands`` > 0 blends them in that many bands, with
+    their masks cut at Voronoi seams when ``voronoi_seams``."""
     import torch  # local: keeps `import StitcherClass` cheap for calibration-only users
 
     on_device = _is_tensor(frames[0]) and frames[0].is_cuda
@@ -587,7 +604,7 @@ def _composite(engine, stages, frames, batched, out=None, debugger=None, feather
                                       "resized at stage %d" % segs[1]["a"])
             return engine.plan_for(sub_stages, sub_shapes, device, feather_log2=feather_log2,
                                    blend_weights=[weight_of.get(id(st)) for st in sub_stages] if weight_of else None,
-                                   camera_weights=camera_weights, blend_bands=blend_bands)
+                                   camera_weights=camera_weights, blend_bands=blend_bands, voronoi_seams=voronoi_seams)
         except PlanUnsupported as e:
             if debugger is not None:
                 debugger.debugger(DEBUG_LEVEL_0, "[STITCHER] {}".format(e), log_type="err")

@@ -17,13 +17,14 @@ MCS_MAX_LAYERS = 16
 MCS_LAYER_COPY = 0
 MCS_LAYER_WARP = 1
 MCS_LAYER_REMAP = 2
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # every symbol include/mcs.h declares
 EXPORTS = (
     "mcs_abi_version", "mcs_last_error", "mcs_plan_create", "mcs_plan_create_maps", "mcs_plan_destroy",
     "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_set_camera_weights",
-    "mcs_plan_set_multiband", "mcs_plan_multiband_bands", "mcs_plan_last_variant",
+    "mcs_plan_set_multiband", "mcs_plan_multiband_bands", "mcs_plan_set_voronoi_seams", "mcs_plan_seam_weights",
+    "mcs_plan_last_variant",
     "mcs_plan_force_variant", "mcs_plan_rows_need_padding", "mcs_plan_promise_padded_rows",
     "mcs_plan_tiled_status", "mcs_plan_tiled_ctas_per_sm", "mcs_plan_tiled_stats", "mcs_launch_count",
     "mcs_match_hamming_top2", "mcs_match_l2_top2", "mcs_ransac_homography", "mcs_refit_homography", "mcs_resize_linear_u8",
@@ -112,6 +113,10 @@ def load(build_if_missing=False):
     lib.mcs_plan_set_multiband.argtypes = [_vp, ctypes.c_int]
     lib.mcs_plan_multiband_bands.restype = ctypes.c_int
     lib.mcs_plan_multiband_bands.argtypes = [_vp]
+    lib.mcs_plan_set_voronoi_seams.restype = ctypes.c_int
+    lib.mcs_plan_set_voronoi_seams.argtypes = [_vp, ctypes.c_int]
+    lib.mcs_plan_seam_weights.restype = ctypes.c_int
+    lib.mcs_plan_seam_weights.argtypes = [_vp, ctypes.c_int, _vp, ctypes.c_int64]
     lib.mcs_plan_tiled_ctas_per_sm.restype = ctypes.c_int
     lib.mcs_plan_tiled_ctas_per_sm.argtypes = [_vp]
     lib.mcs_plan_tiled_status.restype = ctypes.c_char_p
@@ -253,10 +258,16 @@ class Plan(object):
         self.out_w = int(out_w)
         self.out_h = int(out_h)
         self.src_hw = hw.copy()
+        # visible rectangles clipped to the panorama, as the library keeps them
+        r = rect.astype(np.int64)
+        x0, y0 = np.maximum(r[:, 0], 0), np.maximum(r[:, 1], 0)
+        self.rects = np.stack([x0, y0, np.maximum(x0, np.minimum(r[:, 2], out_w)),
+                               np.maximum(y0, np.minimum(r[:, 3], out_h))], axis=1)
         self._owned = None
         self.camera_weighted = False   # set_camera_weights is in force
         self.multiband = False         # set_multiband is in force
         self.blend_bands = 0           # its effective band count
+        self.voronoi_seams = False     # set_voronoi_seams is in force
 
     def close(self):
         if getattr(self, "_h", None) is not None and _lib is not None:
@@ -349,6 +360,7 @@ class Plan(object):
         or a uint8 array of that layer's source (height, width): the camera-weighted blend (include/mcs.h)."""
         n = self.n_layers
         self.multiband, self.blend_bands = False, 0   # every call switches the multi-band blend off
+        self.voronoi_seams = False
         if weight_maps is None:
             check(_lib.mcs_plan_set_camera_weights(self._h, None, None), "mcs_plan_set_camera_weights")
             self._owned = None
@@ -378,11 +390,29 @@ class Plan(object):
     def set_multiband(self, num_bands):
         """The multi-band blend of the camera weights (include/mcs.h mcs_plan_set_multiband); 0 switches it
         off.  Returns the effective band count."""
-        self.multiband, self.blend_bands = False, 0
+        self.multiband, self.blend_bands, self.voronoi_seams = False, 0, False
         check(_lib.mcs_plan_set_multiband(self._h, int(num_bands)), "mcs_plan_set_multiband")
         self.multiband = int(num_bands) > 0
         self.blend_bands = int(_lib.mcs_plan_multiband_bands(self._h))
         return self.blend_bands
+
+    def set_voronoi_seams(self, enable):
+        """Cut the multi-band blend's masks at Voronoi seams (include/mcs.h mcs_plan_set_voronoi_seams); False goes
+        back to the full masks."""
+        rc = _lib.mcs_plan_set_voronoi_seams(self._h, int(bool(enable)))
+        if rc != MCS_ERR_UNSUPPORTED:   # beyond the bound the plan stays as it was
+            self.voronoi_seams = bool(enable) and rc == MCS_OK
+            self.blend_bands = int(_lib.mcs_plan_multiband_bands(self._h))
+            self.multiband = self.blend_bands > 0
+        check(rc, "mcs_plan_set_voronoi_seams")
+
+    def seam_weights(self, layer):
+        """The seam-cut mask of ``layer`` over its visible rectangle clipped to the panorama (uint8 h x w)."""
+        x0, y0, x1, y1 = (int(v) for v in self.rects[int(layer)]) if 0 <= int(layer) < self.n_layers else (0, 0, 0, 0)
+        out = np.zeros((max(1, y1 - y0), max(1, x1 - x0)), np.uint8)
+        check(_lib.mcs_plan_seam_weights(self._h, int(layer), _vp(out.ctypes.data), out.strides[0]),
+              "mcs_plan_seam_weights")
+        return out
 
     def tiled_ctas_per_sm(self):
         return int(_lib.mcs_plan_tiled_ctas_per_sm(self._h))

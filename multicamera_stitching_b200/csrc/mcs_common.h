@@ -8,7 +8,7 @@
 
 #include "mcs.h"
 
-#define MCS_ABI_VERSION 3
+#define MCS_ABI_VERSION 4
 
 // ---- error plumbing -------------------------------------------------------
 void mcs_set_error(const char* fmt, ...);
@@ -172,6 +172,10 @@ struct mcs_plan {
     int mb_on;               // the multi-band blend serves the plan
     int mb_bands;            // its effective band count (clamped like MultiBandBlender::prepare)
     struct McsMultiband* mb; // geometry, weight pyramids and workspace
+    // Voronoi seams of the multi-band blend (mcs_plan_set_voronoi_seams, mcs_seams.cu)
+    int seams_on;            // the weight pyramids were built from the seam-cut weights
+    uint8_t* d_seam[MCS_MAX_LAYERS];   // per fed layer: the seam-cut weights over its clipped rectangle (row pitch =
+                             // its width), nullptr for a layer that feeds nothing or while the seams are off
 };
 
 
@@ -205,6 +209,12 @@ int mcs_multiband_build(mcs_plan* plan, int bands);
 void mcs_multiband_free(mcs_plan* plan);
 int mcs_launch_multiband(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch, const int64_t* fstride,
                          int n_frames, uint8_t* dst, int64_t dst_pitch, int64_t dst_frame_stride, cudaStream_t stream);
+
+// Voronoi seams (mcs_seams.cu): finds the seams of the plan's fed layers from their weight samples into
+// plan->d_seam (synchronous).  Fails with MCS_ERR_UNSUPPORTED, the plan unchanged, where a submask exceeds the
+// bound of the uint16 distances; frees the planes.
+int mcs_seams_build(mcs_plan* plan);
+void mcs_seams_free(mcs_plan* plan);
 
 // Tiled variant (mcs_stitch_tiled.cu): why it cannot serve a call (nullptr = it can), and its launch.
 const char* mcs_tiled_blocker(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,

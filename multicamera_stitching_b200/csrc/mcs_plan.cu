@@ -217,6 +217,7 @@ extern "C" int mcs_plan_destroy(mcs_plan* plan) {
         if (plan->d_cwmap[k]) cudaFree(plan->d_cwmap[k]);
     }
     mcs_multiband_free(plan);
+    mcs_seams_free(plan);
     mcs_plan_free_tiles(plan);
     free_maps(plan);
     delete plan;
@@ -506,6 +507,7 @@ static void free_cwmaps(mcs_plan* plan) {
     plan->cw_maps = 0;
     plan->mb_on = 0;
     mcs_multiband_free(plan);
+    mcs_seams_free(plan);
 }
 
 extern "C" int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_maps, const int64_t* map_pitch) {
@@ -559,6 +561,7 @@ extern "C" int mcs_plan_set_multiband(mcs_plan* plan, int num_bands) {
                   "mcs_plan_set_multiband: the plan feathers its pastes (mcs_plan_set_blend); switch that off first");
     plan->mb_on = 0;
     mcs_multiband_free(plan);
+    mcs_seams_free(plan);
     if (num_bands == 0) return MCS_OK;
     const int rc = mcs_multiband_build(plan, num_bands);
     if (rc != MCS_OK) return rc;
@@ -567,3 +570,39 @@ extern "C" int mcs_plan_set_multiband(mcs_plan* plan, int num_bands) {
 }
 
 extern "C" int mcs_plan_multiband_bands(const mcs_plan* plan) { return plan && plan->mb_on ? plan->mb_bands : 0; }
+
+extern "C" int mcs_plan_set_voronoi_seams(mcs_plan* plan, int enable) {
+    MCS_CHECK_ARG(plan != nullptr, "mcs_plan_set_voronoi_seams: plan is NULL");
+    MCS_CHECK_ARG(plan->mb_on, "mcs_plan_set_voronoi_seams: the plan does not blend in bands (mcs_plan_set_multiband)");
+    const int bands = plan->mb_bands;
+    int rc = MCS_OK;
+    if (enable) {
+        rc = mcs_seams_build(plan);
+        if (rc == MCS_ERR_UNSUPPORTED) return rc;   // beyond the bound the plan stays as it was
+    } else {
+        if (!plan->seams_on) return MCS_OK;
+        mcs_seams_free(plan);
+    }
+    // the weight pyramids and sums of the seam-cut weights, or of the full ones again (also after a failed search)
+    const int built = mcs_multiband_build(plan, bands);
+    if (built != MCS_OK) {
+        plan->mb_on = 0;
+        mcs_seams_free(plan);
+        return built;
+    }
+    return rc;
+}
+
+extern "C" int mcs_plan_seam_weights(const mcs_plan* plan, int layer, uint8_t* host_dst, int64_t dst_pitch) {
+    MCS_CHECK_ARG(plan != nullptr && host_dst != nullptr, "mcs_plan_seam_weights: NULL argument");
+    MCS_CHECK_ARG(plan->seams_on, "mcs_plan_seam_weights: the plan has no Voronoi seams (mcs_plan_set_voronoi_seams)");
+    MCS_CHECK_ARG(layer >= 0 && layer < plan->n_layers && plan->d_seam[layer] != nullptr,
+                  "mcs_plan_seam_weights: layer %d feeds nothing (layers 0..%d)", layer, plan->n_layers - 1);
+    const McsLayer& L = plan->layers[layer];
+    const int w = (L.rx1 < plan->out_w ? L.rx1 : plan->out_w) - (L.rx0 > 0 ? L.rx0 : 0);
+    const int h = (L.ry1 < plan->out_h ? L.ry1 : plan->out_h) - (L.ry0 > 0 ? L.ry0 : 0);
+    MCS_CHECK_ARG(dst_pitch >= w, "mcs_plan_seam_weights: pitch %lld < %d columns", (long long)dst_pitch, w);
+    MCS_CHECK_CUDA(cudaMemcpy2D(host_dst, (size_t)dst_pitch, plan->d_seam[layer], (size_t)w, (size_t)w, (size_t)h,
+                                cudaMemcpyDeviceToHost));
+    return MCS_OK;
+}

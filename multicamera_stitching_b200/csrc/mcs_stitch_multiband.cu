@@ -55,6 +55,8 @@ struct MbArgs {
     long long frame_stride[MCS_MAX_LAYERS];
     uint8_t* dst;
     long long dst_pitch, dst_frame_stride;
+    // plan time: per layer the seam-cut weights over its rectangle (mcs_seams.cu), nullptr = sample the map
+    const uint8_t* seam[MCS_MAX_LAYERS];
 };
 
 struct McsMultiband {
@@ -146,7 +148,8 @@ __global__ void __launch_bounds__(MB_BX * MB_BY) mb_level0_kernel(const __grid_c
     }
 }
 
-// Plan time: level 0 of every camera's weight pyramid, w + (w != 0) inside the rectangle, 0 in the border.
+// Plan time: level 0 of every camera's weight pyramid, w + (w != 0) inside the rectangle, 0 in the border; w is the
+// weight sample, or with Voronoi seams the seam-cut weight the plan holds.
 __global__ void __launch_bounds__(MB_BX * MB_BY) mb_weight0_kernel(const __grid_constant__ MbArgs a) {
     const int j = blockIdx.z;
     const MbCam& c = a.cam[j];
@@ -155,10 +158,14 @@ __global__ void __launch_bounds__(MB_BX * MB_BY) mb_weight0_kernel(const __grid_
     const int px = c.tlx + x, py = c.tly + y;
     int w = 0;
     if (px >= c.x0 && px < c.x1 && py >= c.y0 && py < c.y1) {
-        const McsLayer& g = a.g[c.k];
-        int X, Y;
-        mb_coords(g, px, py, X, Y);
-        w = weight_sample(a.wmap[c.k], g.src_w, g.src_h, X, Y);
+        if (a.seam[c.k]) {
+            w = a.seam[c.k][(long long)(py - c.y0) * (c.x1 - c.x0) + px - c.x0];
+        } else {
+            const McsLayer& g = a.g[c.k];
+            int X, Y;
+            mb_coords(g, px, py, X, Y);
+            w = weight_sample(a.wmap[c.k], g.src_w, g.src_h, X, Y);
+        }
         w += w != 0 ? 1 : 0;
     }
     a.wpyr[a.woff[j][0] + (long long)y * c.bw + x] = (int16_t)w;
@@ -304,6 +311,7 @@ int mcs_multiband_build(mcs_plan* plan, int bands) {
         const McsLayer& L = plan->layers[k];
         a.g[k] = L;
         a.wmap[k] = plan->d_cwmap[k];
+        a.seam[k] = plan->seams_on ? plan->d_seam[k] : nullptr;
         MbCam c;
         c.k = k;
         c.x0 = L.rx0 > 0 ? L.rx0 : 0;

@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .plan import flatten_chain, plan_maps, plan_paste, plan_tables, stage_signature
+from .plan import PlanUnsupported, flatten_chain, plan_maps, plan_paste, plan_tables, stage_signature
 
 
 def _stage_field(st, name):
@@ -87,7 +87,8 @@ class PinnedResults(object):
 class CompiledPlan(object):
     """A flattened chain plus its ``mcs_plan`` on one device."""
 
-    def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None, blend_bands=0):
+    def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None, blend_bands=0,
+                 voronoi_seams=False):
         self.flat = flat
         self.device = torch.device(device)
         self.feather_log2 = int(feather_log2)
@@ -116,6 +117,13 @@ class CompiledPlan(object):
                         raise
                 if blend_bands:
                     self.handle.set_multiband(blend_bands)
+                if voronoi_seams:
+                    try:
+                        self.handle.set_voronoi_seams(True)
+                    except _cabi.McsError as e:
+                        if e.code == _cabi.MCS_ERR_UNSUPPORTED:
+                            raise PlanUnsupported(str(e))
+                        raise
             # rows that are not a multiple of 4 bytes: run() always passes them through its
             # zero-padded scratch buffers, which is what the tiled kernel needs to serve them
             self.pad_rows = self._tiled() and self.handle.rows_need_padding()
@@ -281,7 +289,7 @@ class CompositeEngine(object):
         return torch.device(self._device)
 
     def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None, camera_weights=None,
-                 blend_bands=0):
+                 blend_bands=0, voronoi_seams=False):
         """Compiled plan for this chain state and these frame shapes, or None
         when no stage is calibrated (decided on the host, no device needed)."""
         shapes = tuple(tuple(int(v) for v in s) for s in cam_shapes)
@@ -299,14 +307,16 @@ class CompositeEngine(object):
             ckey = tuple(None if w is None else (np.asarray(w).shape, hash(np.ascontiguousarray(w, dtype=np.uint8).tobytes()))
                          for w in camera_weights)
         blend_bands = int(blend_bands or 0)
-        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands)
+        voronoi_seams = bool(voronoi_seams)
+        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands, voronoi_seams)
         if key in self._plans:
             self._plans[key] = self._plans.pop(key)      # most recently used last
         else:
             flat = flatten_chain(stages, shapes)
             while len(self._plans) >= self.max_plans:     # evict the least recently used, one at a time
                 self._plans.pop(next(iter(self._plans)))
-            self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights, blend_bands)
+            self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights, blend_bands,
+                                             voronoi_seams)
                                 if flat is not None else None)
         return self._plans[key]
 
