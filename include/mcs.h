@@ -322,6 +322,33 @@ int mcs_plan_multiband_bands(const mcs_plan* plan);
 int mcs_plan_set_voronoi_seams(mcs_plan* plan, int enable);
 int mcs_plan_seam_weights(const mcs_plan* plan, int layer, uint8_t* host_dst, int64_t dst_pitch);
 
+/*
+ * mcs_plan_set_graphcut_seams - cut the masks of the multi-band blend where the cameras agree on colour, as
+ * OpenCV's default stitching pipeline does with cv::detail::GraphCutSeamFinder("COST_COLOR").  Voronoi seams cut
+ * each overlap halfway between the cameras whatever the content, so a seam can run through an object the cameras
+ * see at different parallax; a graph-cut seam goes around it.  The finder runs on the same layers, pairs, order and
+ * 10-pixel-grown submasks as mcs_plan_set_voronoi_seams, with the overwrite samples v_k of one frame-set: per pair
+ * the minimum cut of the grid graph whose 4-neighbour edges cost D(p) + D(q) + 1 (D = the squared RGB difference
+ * of the two cameras' samples, + 1000 where either mask is 0 at p or q), with terminal edges of 10000 to camera i
+ * where its mask is non-zero and to camera j where its mask is; inside the overlap each pixel goes to its side of
+ * the cut and is zeroed in the other camera's mask.  The cut is computed exactly (integer capacities, push-relabel
+ * maximum flow on the device).  Among several minimum cuts - flat or identical content, for example sky that both
+ * cameras saturate - it takes the minimal side of camera i (the pixels reachable from camera i's terminal in the
+ * residual graph of a maximum flow), which is unique; cv2 takes whichever cut its search order finds, so there,
+ * and only there, the masks can differ from cv2's.  Specification in oracle/graphcut_seam_model.py.
+ *
+ * src / src_pitch: one device frame-set laid out as for mcs_stitch_u8 with one frame (per layer the frame of its
+ * camera, H x W x 3 uint8).  It is read only during the call: the seams are found once (one launch to sample the
+ * weights, one for the images, then per overlapping pair rounds of launches until the flow is maximal), the
+ * weight pyramids and sums are rebuilt from the cut masks, and the per-frame work of mcs_stitch_u8 (variant 6) does
+ * not change.  Replaces Voronoi seams (and mcs_plan_set_voronoi_seams replaces these); src = NULL goes back to the
+ * full masks.  Requires the multi-band blend, else MCS_ERR_INVALID; a plan of 1 or 4 channels fails with
+ * MCS_ERR_UNSUPPORTED and is unchanged.  A flow that does not end within 2^22 push-relabel rounds (a guard against
+ * bugs, not an input case) fails with MCS_ERR_CUDA and leaves the plan as it was.  mcs_plan_set_multiband and
+ * mcs_plan_set_camera_weights switch the seams off; mcs_plan_seam_weights reads the cut masks back.  Synchronous.
+ */
+int mcs_plan_set_graphcut_seams(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch);
+
 /* Which kernel variant the last mcs_stitch_u8 on this plan launched
  * (diagnostics for tests / bench): 0 = none yet, 1 = gather, 2 = tiled, 3 = overwrite pass +
  * feather band pass, 4 = tiled with the seam bands blended in the same launch, 5 = camera-weighted

@@ -18,6 +18,7 @@ reference) or uint8 CUDA tensors (result: a CUDA tensor, nothing leaves the
 device).  There is no CPU fallback: without the CUDA library these methods
 raise.
 """
+import hashlib
 import os
 import pickle
 
@@ -78,6 +79,11 @@ class Stitcher(Debugger):
     # every overlap at OpenCV's VoronoiSeamFinder seam before the blend, so that each overlap pixel takes its fine
     # detail from one camera and only the low bands mix across the seam.  Needs ``blend_bands`` > 0.
     voronoi_seams = False
+    # Optional graph-cut seams for the multi-band blend (extension, include/mcs.h mcs_plan_set_graphcut_seams), set by
+    # ``find_graphcut_seams``: None, or ``(digest, frames)`` - the read-only frame-set the seams are found on, in
+    # camera order, and its digest, which keys the compiled plans.  Needs ``blend_bands`` > 0, not with
+    # ``voronoi_seams``.
+    graphcut_seams = None
 
     def __init__(self, images_dic, super_mode=False):
         # labels sorted like np.sort(images_dic.keys()) (reference :61)
@@ -158,7 +164,7 @@ class Stitcher(Debugger):
         out = _composite(self._engine_(), self.stitchers, frames, batched=False, debugger=self,
                          feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
                          camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
-                         voronoi_seams=self._voronoi_seams())
+                         voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams())
         if draw_descriptors and not _is_tensor(out):
             out = self._draw_overlays(out, frames)
         return out
@@ -203,14 +209,14 @@ class Stitcher(Debugger):
         return _composite(self._engine_(), self.stitchers, frames, batched=True, out=out, debugger=self,
                           feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
                           camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
-                          voronoi_seams=self._voronoi_seams())
+                          voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams())
 
     def plan(self, img_shapes, device=None):
         """Compiled plan (``engine.CompiledPlan``) for frames of these shapes."""
         return self._engine_().plan_for(self.stitchers, [tuple(s) for s in img_shapes], device,
                                         feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
                                         camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
-                          voronoi_seams=self._voronoi_seams())
+                                        voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams())
 
     def _blend_bands(self):
         """``blend_bands`` checked: an int in 0..8."""
@@ -227,6 +233,55 @@ class Stitcher(Debugger):
         if v and not self._blend_bands():
             raise ValueError("voronoi_seams cuts the masks of the multi-band blend: set blend_bands > 0 too")
         return bool(v)
+
+    def find_graphcut_seams(self, images_dic):
+        """Cut the multi-band blend's masks at graph-cut seams (OpenCV's ``GraphCutSeamFinder("COST_COLOR")``) found
+        on this frame-set, ``{label: H x W x 3 uint8 frame}`` of every camera's calibrated size: each overlap is cut
+        where the two cameras agree on colour, around objects they see at different parallax.  Keeps a read-only
+        copy of the frames; the seams are found on the device when a plan is compiled and stay until this is called
+        again (new frames find new seams) or with None (back to the full masks)."""
+        if images_dic is None:
+            self.graphcut_seams = None
+            return
+        labels = [str(l) for l in self.img_labels]
+        by_label = {str(k): v for k, v in dict(images_dic).items()}
+        missing = sorted(set(labels) - set(by_label))
+        if missing:
+            raise ValueError("find_graphcut_seams needs a frame of every camera, missing %r" % (missing,))
+        frames = []
+        digest = hashlib.sha256()
+        for i, label in enumerate(labels):
+            f = by_label[label]
+            if _is_tensor(f):
+                f = f.detach().cpu().numpy()
+            f = np.asarray(f)
+            st = self.stitchers[max(0, i - 1)]
+            size = st.BimgSize if i == 0 else st.AimgSize
+            want = None if size is None else tuple(size[:2]) + (3,)
+            if f.dtype != np.uint8 or f.ndim != 3 or f.shape[2] != 3 or (want is not None and f.shape != want):
+                raise ValueError("find_graphcut_seams: camera %r needs a uint8 frame of its calibrated (h, w, 3) %r, "
+                                 "got %s %r" % (label, want, f.dtype, f.shape))
+            f = np.array(f, np.uint8, order="C", copy=True)
+            f.setflags(write=False)
+            digest.update(repr(f.shape).encode())
+            digest.update(f.data)
+            frames.append(f)
+        self.graphcut_seams = (digest.hexdigest(), tuple(frames))
+
+    def _graphcut_seams(self):
+        """``graphcut_seams`` checked: None, or ``(digest, frames)`` only with ``blend_bands`` > 0 and without
+        ``voronoi_seams``."""
+        g = self.graphcut_seams
+        if g is None:
+            return None
+        if not self._blend_bands():
+            raise ValueError("graph-cut seams cut the masks of the multi-band blend: set blend_bands > 0 too")
+        if self._voronoi_seams():
+            raise ValueError("graph-cut seams and voronoi_seams exclude each other: set voronoi_seams = False or "
+                             "call find_graphcut_seams(None)")
+        if not (isinstance(g, tuple) and len(g) == 2 and isinstance(g[0], str) and len(g[1]) == len(self.img_labels)):
+            raise ValueError("graphcut_seams is set by find_graphcut_seams, got %r" % (type(g),))
+        return g
 
     def _camera_weight_list(self):
         """``camera_weights`` checked and as a list in camera order, or None when the mode is off (with
@@ -577,10 +632,11 @@ def edge_ramp(shape, width=64):
 
 
 def _composite(engine, stages, frames, batched, out=None, debugger=None, feather_log2=0, blend_weights=None,
-               camera_weights=None, blend_bands=0, voronoi_seams=False):
+               camera_weights=None, blend_bands=0, voronoi_seams=False, graphcut_seams=None):
     """Run the fused kernel for this chain on these frames.  ``camera_weights``: one entry per camera (None or
     a uint8 map) for the camera-weighted blend, or None; ``blend_bands`` > 0 blends them in that many bands, with
-    their masks cut at Voronoi seams when ``voronoi_seams``."""
+    their masks cut at Voronoi seams when ``voronoi_seams`` or at the graph-cut seams of the frame-set
+    ``graphcut_seams = (digest, frames)``."""
     import torch  # local: keeps `import StitcherClass` cheap for calibration-only users
 
     on_device = _is_tensor(frames[0]) and frames[0].is_cuda
@@ -604,7 +660,8 @@ def _composite(engine, stages, frames, batched, out=None, debugger=None, feather
                                       "resized at stage %d" % segs[1]["a"])
             return engine.plan_for(sub_stages, sub_shapes, device, feather_log2=feather_log2,
                                    blend_weights=[weight_of.get(id(st)) for st in sub_stages] if weight_of else None,
-                                   camera_weights=camera_weights, blend_bands=blend_bands, voronoi_seams=voronoi_seams)
+                                   camera_weights=camera_weights, blend_bands=blend_bands, voronoi_seams=voronoi_seams,
+                                   graphcut_seams=graphcut_seams)
         except PlanUnsupported as e:
             if debugger is not None:
                 debugger.debugger(DEBUG_LEVEL_0, "[STITCHER] {}".format(e), log_type="err")

@@ -17,13 +17,14 @@ MCS_MAX_LAYERS = 16
 MCS_LAYER_COPY = 0
 MCS_LAYER_WARP = 1
 MCS_LAYER_REMAP = 2
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 # every symbol include/mcs.h declares
 EXPORTS = (
     "mcs_abi_version", "mcs_last_error", "mcs_plan_create", "mcs_plan_create_maps", "mcs_plan_destroy",
     "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_set_camera_weights",
     "mcs_plan_set_multiband", "mcs_plan_multiband_bands", "mcs_plan_set_voronoi_seams", "mcs_plan_seam_weights",
+    "mcs_plan_set_graphcut_seams",
     "mcs_plan_last_variant",
     "mcs_plan_force_variant", "mcs_plan_rows_need_padding", "mcs_plan_promise_padded_rows",
     "mcs_plan_tiled_status", "mcs_plan_tiled_ctas_per_sm", "mcs_plan_tiled_stats", "mcs_launch_count",
@@ -117,6 +118,8 @@ def load(build_if_missing=False):
     lib.mcs_plan_set_voronoi_seams.argtypes = [_vp, ctypes.c_int]
     lib.mcs_plan_seam_weights.restype = ctypes.c_int
     lib.mcs_plan_seam_weights.argtypes = [_vp, ctypes.c_int, _vp, ctypes.c_int64]
+    lib.mcs_plan_set_graphcut_seams.restype = ctypes.c_int
+    lib.mcs_plan_set_graphcut_seams.argtypes = [_vp, ctypes.POINTER(_vp), _c_i64p]
     lib.mcs_plan_tiled_ctas_per_sm.restype = ctypes.c_int
     lib.mcs_plan_tiled_ctas_per_sm.argtypes = [_vp]
     lib.mcs_plan_tiled_status.restype = ctypes.c_char_p
@@ -268,6 +271,7 @@ class Plan(object):
         self.multiband = False         # set_multiband is in force
         self.blend_bands = 0           # its effective band count
         self.voronoi_seams = False     # set_voronoi_seams is in force
+        self.graphcut_seams = False    # set_graphcut_seams is in force
 
     def close(self):
         if getattr(self, "_h", None) is not None and _lib is not None:
@@ -360,7 +364,7 @@ class Plan(object):
         or a uint8 array of that layer's source (height, width): the camera-weighted blend (include/mcs.h)."""
         n = self.n_layers
         self.multiband, self.blend_bands = False, 0   # every call switches the multi-band blend off
-        self.voronoi_seams = False
+        self.voronoi_seams = self.graphcut_seams = False
         if weight_maps is None:
             check(_lib.mcs_plan_set_camera_weights(self._h, None, None), "mcs_plan_set_camera_weights")
             self._owned = None
@@ -390,7 +394,7 @@ class Plan(object):
     def set_multiband(self, num_bands):
         """The multi-band blend of the camera weights (include/mcs.h mcs_plan_set_multiband); 0 switches it
         off.  Returns the effective band count."""
-        self.multiband, self.blend_bands, self.voronoi_seams = False, 0, False
+        self.multiband, self.blend_bands, self.voronoi_seams, self.graphcut_seams = False, 0, False, False
         check(_lib.mcs_plan_set_multiband(self._h, int(num_bands)), "mcs_plan_set_multiband")
         self.multiband = int(num_bands) > 0
         self.blend_bands = int(_lib.mcs_plan_multiband_bands(self._h))
@@ -402,9 +406,32 @@ class Plan(object):
         rc = _lib.mcs_plan_set_voronoi_seams(self._h, int(bool(enable)))
         if rc != MCS_ERR_UNSUPPORTED:   # beyond the bound the plan stays as it was
             self.voronoi_seams = bool(enable) and rc == MCS_OK
+            self.graphcut_seams = False
             self.blend_bands = int(_lib.mcs_plan_multiband_bands(self._h))
             self.multiband = self.blend_bands > 0
         check(rc, "mcs_plan_set_voronoi_seams")
+
+    def set_graphcut_seams(self, src_ptrs, src_pitch):
+        """Cut the multi-band blend's masks at graph-cut seams found on one device frame-set (include/mcs.h
+        mcs_plan_set_graphcut_seams): per layer the device pointer and row pitch of its camera's H x W x 3 frame.
+        ``src_ptrs`` None goes back to the full masks.  Synchronous; the frames may be freed afterwards."""
+        if src_ptrs is None:
+            rc = _lib.mcs_plan_set_graphcut_seams(self._h, None, None)
+        else:
+            n = self.n_layers
+            if len(src_ptrs) != n or len(src_pitch) != n:
+                raise ValueError("set_graphcut_seams needs one frame per layer (%d)" % n)
+            ptrs = (_vp * n)(*[int(p) for p in src_ptrs])
+            pitch = (ctypes.c_int64 * n)(*[int(p) for p in src_pitch])
+            rc = _lib.mcs_plan_set_graphcut_seams(self._h, ptrs, pitch)
+        if rc == MCS_OK:   # these seams replace any others
+            self.graphcut_seams, self.voronoi_seams = src_ptrs is not None, False
+        else:              # a refused call leaves the plan as it was; a failed rebuild switches the blend off
+            self.blend_bands = int(_lib.mcs_plan_multiband_bands(self._h))
+            self.multiband = self.blend_bands > 0
+            if not self.multiband:
+                self.graphcut_seams = self.voronoi_seams = False
+        check(rc, "mcs_plan_set_graphcut_seams")
 
     def seam_weights(self, layer):
         """The seam-cut mask of ``layer`` over its visible rectangle clipped to the panorama (uint8 h x w)."""

@@ -8,7 +8,7 @@
 
 #include "mcs.h"
 
-#define MCS_ABI_VERSION 4
+#define MCS_ABI_VERSION 5
 
 // ---- error plumbing -------------------------------------------------------
 void mcs_set_error(const char* fmt, ...);
@@ -172,7 +172,8 @@ struct mcs_plan {
     int mb_on;               // the multi-band blend serves the plan
     int mb_bands;            // its effective band count (clamped like MultiBandBlender::prepare)
     struct McsMultiband* mb; // geometry, weight pyramids and workspace
-    // Voronoi seams of the multi-band blend (mcs_plan_set_voronoi_seams, mcs_seams.cu)
+    // Voronoi or graph-cut seams of the multi-band blend (mcs_plan_set_voronoi_seams, mcs_seams.cu;
+    // mcs_plan_set_graphcut_seams, mcs_seams_graphcut.cu)
     int seams_on;            // the weight pyramids were built from the seam-cut weights
     uint8_t* d_seam[MCS_MAX_LAYERS];   // per fed layer: the seam-cut weights over its clipped rectangle (row pitch =
                              // its width), nullptr for a layer that feeds nothing or while the seams are off
@@ -215,6 +216,14 @@ int mcs_launch_multiband(const mcs_plan* plan, const uint8_t* const* src, const 
 // bound of the uint16 distances; frees the planes.
 int mcs_seams_build(mcs_plan* plan);
 void mcs_seams_free(mcs_plan* plan);
+// Launches seam_fill_kernel: planes[k] (the size of layer k's clipped rectangle) = the weight sample of every fed
+// layer k.
+void mcs_seams_fill(const mcs_plan* plan, uint8_t* const* planes);
+
+// Graph-cut seams (mcs_seams_graphcut.cu): finds the seams of the plan's fed layers from their weight samples and the
+// samples of one frame-set (src / src_pitch per layer, 3 channels) into plan->d_seam (synchronous).  On any failure
+// the plan is unchanged.
+int mcs_graphcut_build(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch);
 
 // Tiled variant (mcs_stitch_tiled.cu): why it cannot serve a call (nullptr = it can), and its launch.
 const char* mcs_tiled_blocker(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,

@@ -593,6 +593,32 @@ extern "C" int mcs_plan_set_voronoi_seams(mcs_plan* plan, int enable) {
     return rc;
 }
 
+extern "C" int mcs_plan_set_graphcut_seams(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch) {
+    MCS_CHECK_ARG(plan != nullptr, "mcs_plan_set_graphcut_seams: plan is NULL");
+    MCS_CHECK_ARG(plan->mb_on, "mcs_plan_set_graphcut_seams: the plan does not blend in bands (mcs_plan_set_multiband)");
+    if (src == nullptr) {
+        if (!plan->seams_on) return MCS_OK;
+        mcs_seams_free(plan);
+    } else {
+        MCS_CHECK_ARG(src_pitch != nullptr, "mcs_plan_set_graphcut_seams: src_pitch is NULL");
+        if (plan->channels != 3) {
+            mcs_set_error("mcs_plan_set_graphcut_seams: the colour cost needs 3 channels, the plan has %d",
+                          plan->channels);
+            return MCS_ERR_UNSUPPORTED;
+        }
+        const int rc = mcs_graphcut_build(plan, src, src_pitch);
+        if (rc != MCS_OK) return rc;   // the plan stays as it was
+    }
+    // the weight pyramids and sums of the cut weights, or of the full ones again
+    const int bands = plan->mb_bands;
+    const int built = mcs_multiband_build(plan, bands);
+    if (built != MCS_OK) {
+        plan->mb_on = 0;
+        mcs_seams_free(plan);
+    }
+    return built;
+}
+
 extern "C" int mcs_plan_seam_weights(const mcs_plan* plan, int layer, uint8_t* host_dst, int64_t dst_pitch) {
     MCS_CHECK_ARG(plan != nullptr && host_dst != nullptr, "mcs_plan_seam_weights: NULL argument");
     MCS_CHECK_ARG(plan->seams_on, "mcs_plan_seam_weights: the plan has no Voronoi seams (mcs_plan_set_voronoi_seams)");

@@ -170,6 +170,29 @@ __global__ void __launch_bounds__(SEAM_COL_THREADS) seam_cols_kernel(const __gri
     }
 }
 
+void mcs_seams_fill(const mcs_plan* plan, uint8_t* const* planes) {
+    SeamFill a;
+    memset(&a, 0, sizeof(a));
+    int n = 0, bw = 0, bh = 0;
+    for (int k = 0; k < plan->n_layers; ++k) {
+        const McsLayer& L = plan->layers[k];
+        a.g[k] = L;
+        a.wmap[k] = plan->d_cwmap[k];
+        a.plane[k] = planes[k];
+        const int x0 = L.rx0 > 0 ? L.rx0 : 0, y0 = L.ry0 > 0 ? L.ry0 : 0;
+        const int x1 = L.rx1 < plan->out_w ? L.rx1 : plan->out_w, y1 = L.ry1 < plan->out_h ? L.ry1 : plan->out_h;
+        a.rect[k] = make_int4(x0, y0, x1, y1);
+        if (x1 > x0 && y1 > y0) {
+            a.layer[n++] = k;
+            bw = x1 - x0 > bw ? x1 - x0 : bw;
+            bh = y1 - y0 > bh ? y1 - y0 : bh;
+        }
+    }
+    if (n == 0) return;
+    seam_fill_kernel<<<dim3((bw + SEAM_BX - 1) / SEAM_BX, (bh + SEAM_BY - 1) / SEAM_BY, n), dim3(SEAM_BX, SEAM_BY, 1)>>>(a);
+    mcs_count_launch(1);
+}
+
 void mcs_seams_free(mcs_plan* plan) {
     for (int k = 0; k < MCS_MAX_LAYERS; ++k) {
         if (plan->d_seam[k]) cudaFree(plan->d_seam[k]);

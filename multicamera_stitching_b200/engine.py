@@ -88,7 +88,7 @@ class CompiledPlan(object):
     """A flattened chain plus its ``mcs_plan`` on one device."""
 
     def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None, blend_bands=0,
-                 voronoi_seams=False):
+                 voronoi_seams=False, graphcut_frames=None):
         self.flat = flat
         self.device = torch.device(device)
         self.feather_log2 = int(feather_log2)
@@ -124,6 +124,8 @@ class CompiledPlan(object):
                         if e.code == _cabi.MCS_ERR_UNSUPPORTED:
                             raise PlanUnsupported(str(e))
                         raise
+                if graphcut_frames is not None:
+                    self._find_graphcut_seams(graphcut_frames)
             # rows that are not a multiple of 4 bytes: run() always passes them through its
             # zero-padded scratch buffers, which is what the tiled kernel needs to serve them
             self.pad_rows = self._tiled() and self.handle.rows_need_padding()
@@ -131,6 +133,26 @@ class CompiledPlan(object):
                 self.handle.promise_padded_rows(True)
         self.cams = [l.cam for l in flat.layers]
         self.out_w, self.out_h, self.channels = flat.out_w, flat.out_h, flat.channels
+
+    def _find_graphcut_seams(self, frames_by_cam):
+        """Upload one host frame-set (``frames_by_cam[c]``: H x W x 3 uint8), find the graph-cut seams on it
+        (include/mcs.h mcs_plan_set_graphcut_seams) and drop the upload."""
+        dev = {}
+        for l in self.flat.layers:
+            f = np.asarray(frames_by_cam[l.cam])
+            want = tuple(l.src_hw) + (3,)
+            if f.dtype != np.uint8 or f.shape != want:
+                raise ValueError("graph-cut seams: camera %d's frame is %s %r, the plan needs uint8 %r"
+                                 % (l.cam, f.dtype, f.shape, want))
+            if l.cam not in dev:
+                dev[l.cam] = torch.from_numpy(np.array(f)).to(self.device)
+        try:
+            self.handle.set_graphcut_seams([dev[l.cam].data_ptr() for l in self.flat.layers],
+                                           [dev[l.cam].stride(0) for l in self.flat.layers])
+        except _cabi.McsError as e:
+            if e.code == _cabi.MCS_ERR_UNSUPPORTED:
+                raise PlanUnsupported(str(e))
+            raise
 
     def _tiled(self):
         """Whether the tiled kernel serves this plan (it does not serve the camera-weighted blends)."""
@@ -289,9 +311,10 @@ class CompositeEngine(object):
         return torch.device(self._device)
 
     def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None, camera_weights=None,
-                 blend_bands=0, voronoi_seams=False):
+                 blend_bands=0, voronoi_seams=False, graphcut_seams=None):
         """Compiled plan for this chain state and these frame shapes, or None
-        when no stage is calibrated (decided on the host, no device needed)."""
+        when no stage is calibrated (decided on the host, no device needed).  ``graphcut_seams``: None or
+        ``(digest, frames by camera)`` of the frame-set the graph-cut seams are found on."""
         shapes = tuple(tuple(int(v) for v in s) for s in cam_shapes)
         sig = tuple(stage_signature(st) for st in stages)
         if all(s is None for s in sig):
@@ -308,7 +331,8 @@ class CompositeEngine(object):
                          for w in camera_weights)
         blend_bands = int(blend_bands or 0)
         voronoi_seams = bool(voronoi_seams)
-        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands, voronoi_seams)
+        gkey = None if graphcut_seams is None else graphcut_seams[0]
+        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands, voronoi_seams, gkey)
         if key in self._plans:
             self._plans[key] = self._plans.pop(key)      # most recently used last
         else:
@@ -316,7 +340,7 @@ class CompositeEngine(object):
             while len(self._plans) >= self.max_plans:     # evict the least recently used, one at a time
                 self._plans.pop(next(iter(self._plans)))
             self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights, blend_bands,
-                                             voronoi_seams)
+                                             voronoi_seams, None if graphcut_seams is None else graphcut_seams[1])
                                 if flat is not None else None)
         return self._plans[key]
 
