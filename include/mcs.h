@@ -349,6 +349,43 @@ int mcs_plan_seam_weights(const mcs_plan* plan, int layer, uint8_t* host_dst, in
  */
 int mcs_plan_set_graphcut_seams(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch);
 
+/*
+ * mcs_plan_estimate_gains - exposure gains of the rig's cameras from one frame-set, as OpenCV's
+ * cv::detail::GainCompensator (ExposureCompensator::createDefault(GAIN)) estimates them: the cameras meter on their own,
+ * so the same wall comes out at different brightness in neighbouring cameras, and multi-band blending or a seam only
+ * spreads or hides that step.  The compensator runs on the layers that feed the blends (non-empty visible rectangle,
+ * innermost first) with their rectangles' corners, the overwrite samples v_k of the frame-set and the weight samples w_k
+ * as masks (the uncut weights: seams do not change the gains).  For every pair i <= j whose rectangles overlap, only
+ * pixels where both masks are exactly 255 count - ramps below 255 and the bilinear rim of a warped camera drop out -
+ * N(i, j) = max(1, their number), I(i, j) = the mean of sqrt(b^2 + g^2 + r^2) of camera i there (a sequential float64
+ * sum in row-major order, as OpenCV adds it); the gains solve OpenCV's normal equations (alpha = 0.01, beta = 100) by
+ * Gaussian elimination with partial pivoting in float64.  A camera that shares no such pixel with another keeps gain 1.
+ * Specification in oracle/exposure_model.py.  The statistics are bit-exact with OpenCV; cv2.solve rounds the same
+ * elimination differently in its SIMD inner loop, so from 3 cameras on the gains agree with OpenCV's to about 1e-15
+ * relative and give the same 256-entry tables on every tested rig.
+ *
+ *   src / src_pitch  one device frame-set laid out as for mcs_plan_set_graphcut_seams (per layer the frame of its
+ *                    camera, H x W x 3 uint8); read only during the call
+ *   host_gains       host float64 [n_layers]: the gain of every layer (1 for a layer that feeds nothing)
+ *   host_N, host_I   host int64 / float64 [n_fed * n_fed] (row-major, fed layers in feed order) or NULL: the
+ *                    statistics (N = 0 where two rectangles do not overlap; I(i, i) = 0)
+ * Needs camera weights (mcs_plan_set_camera_weights), else MCS_ERR_INVALID; a plan of 1 or 4 channels fails with
+ * MCS_ERR_UNSUPPORTED.  It does not change the plan.  Synchronous.
+ *
+ * mcs_plan_set_exposure_gains - compensate every camera of the camera-weighted blend (variant 5) and the multi-band
+ * blend (variant 6) with its gain: each camera's rounded sample v becomes saturate_u8(rint(v * gain)) (rounding half
+ * to even), what GainCompensator::apply does to the warped image before it is blended; gains[k] per layer (host
+ * float64 [n_layers]), for example those of mcs_plan_estimate_gains.  The plan keeps one 256-entry table per layer.
+ * When the plan has gains, mcs_plan_set_graphcut_seams finds its seams on the compensated samples, so set the gains
+ * first.  gains = NULL switches the compensation off.  Needs camera weights, else MCS_ERR_INVALID; a gain that is not
+ * finite or is negative fails with MCS_ERR_INVALID and leaves the plan as it was.  mcs_plan_set_camera_weights, and
+ * clearing the weights, clear the gains.  The overwrite and the stage-wise blend of mcs_plan_set_blend are never
+ * compensated.  Synchronous.
+ */
+int mcs_plan_estimate_gains(const mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch,
+                            double* host_gains, int64_t* host_N, double* host_I);
+int mcs_plan_set_exposure_gains(mcs_plan* plan, const double* gains);
+
 /* Which kernel variant the last mcs_stitch_u8 on this plan launched
  * (diagnostics for tests / bench): 0 = none yet, 1 = gather, 2 = tiled, 3 = overwrite pass +
  * feather band pass, 4 = tiled with the seam bands blended in the same launch, 5 = camera-weighted

@@ -84,6 +84,12 @@ class Stitcher(Debugger):
     # camera order, and its digest, which keys the compiled plans.  Needs ``blend_bands`` > 0, not with
     # ``voronoi_seams``.
     graphcut_seams = None
+    # Optional exposure compensation of the camera-weighted and multi-band blends (extension, include/mcs.h
+    # mcs_plan_set_exposure_gains): None, or {label: gain} - every camera's sample v becomes saturate_u8(rint(v * gain))
+    # before it is blended, as OpenCV's GainCompensator applies its gains; a missing label keeps gain 1.
+    # ``compensate_exposure`` estimates them from a frame-set; they are plain floats, to read, set, pickle and reuse.
+    # Needs ``camera_weights`` or ``blend_bands`` > 0.
+    exposure_gains = None
 
     def __init__(self, images_dic, super_mode=False):
         # labels sorted like np.sort(images_dic.keys()) (reference :61)
@@ -164,7 +170,8 @@ class Stitcher(Debugger):
         out = _composite(self._engine_(), self.stitchers, frames, batched=False, debugger=self,
                          feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
                          camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
-                         voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams())
+                         voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams(),
+                         exposure_gains=self._exposure_gains())
         if draw_descriptors and not _is_tensor(out):
             out = self._draw_overlays(out, frames)
         return out
@@ -209,14 +216,16 @@ class Stitcher(Debugger):
         return _composite(self._engine_(), self.stitchers, frames, batched=True, out=out, debugger=self,
                           feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
                           camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
-                          voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams())
+                          voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams(),
+                          exposure_gains=self._exposure_gains())
 
     def plan(self, img_shapes, device=None):
         """Compiled plan (``engine.CompiledPlan``) for frames of these shapes."""
         return self._engine_().plan_for(self.stitchers, [tuple(s) for s in img_shapes], device,
                                         feather_log2=getattr(self, "feather_log2", 0), blend_weights=self.blend_weights,
                                         camera_weights=self._camera_weight_list(), blend_bands=self._blend_bands(),
-                                        voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams())
+                                        voronoi_seams=self._voronoi_seams(), graphcut_seams=self._graphcut_seams(),
+                                        exposure_gains=self._exposure_gains())
 
     def _blend_bands(self):
         """``blend_bands`` checked: an int in 0..8."""
@@ -243,13 +252,22 @@ class Stitcher(Debugger):
         if images_dic is None:
             self.graphcut_seams = None
             return
+        frames = self._frame_set(images_dic, "find_graphcut_seams")
+        digest = hashlib.sha256()
+        for f in frames:
+            digest.update(repr(f.shape).encode())
+            digest.update(f.data)
+        self.graphcut_seams = (digest.hexdigest(), tuple(frames))
+
+    def _frame_set(self, images_dic, what):
+        """Read-only copies, in camera order, of one frame-set ``{label: H x W x 3 uint8 frame}`` of every camera's
+        calibrated size."""
         labels = [str(l) for l in self.img_labels]
         by_label = {str(k): v for k, v in dict(images_dic).items()}
         missing = sorted(set(labels) - set(by_label))
         if missing:
-            raise ValueError("find_graphcut_seams needs a frame of every camera, missing %r" % (missing,))
+            raise ValueError("%s needs a frame of every camera, missing %r" % (what, missing))
         frames = []
-        digest = hashlib.sha256()
         for i, label in enumerate(labels):
             f = by_label[label]
             if _is_tensor(f):
@@ -259,14 +277,59 @@ class Stitcher(Debugger):
             size = st.BimgSize if i == 0 else st.AimgSize
             want = None if size is None else tuple(size[:2]) + (3,)
             if f.dtype != np.uint8 or f.ndim != 3 or f.shape[2] != 3 or (want is not None and f.shape != want):
-                raise ValueError("find_graphcut_seams: camera %r needs a uint8 frame of its calibrated (h, w, 3) %r, "
-                                 "got %s %r" % (label, want, f.dtype, f.shape))
+                raise ValueError("%s: camera %r needs a uint8 frame of its calibrated (h, w, 3) %r, got %s %r"
+                                 % (what, label, want, f.dtype, f.shape))
             f = np.array(f, np.uint8, order="C", copy=True)
             f.setflags(write=False)
-            digest.update(repr(f.shape).encode())
-            digest.update(f.data)
             frames.append(f)
-        self.graphcut_seams = (digest.hexdigest(), tuple(frames))
+        return frames
+
+    def compensate_exposure(self, images_dic):
+        """Estimate every camera's exposure gain on this frame-set, ``{label: H x W x 3 uint8 frame}`` of every camera's
+        calibrated size, as OpenCV's ``GainCompensator`` does (on the device), store the gains in ``exposure_gains``
+        and return them (``{label: gain}``).  Only pixels where two cameras' weights are both 255 count.  The gains
+        stay until this is called again or with None (no compensation).  Needs ``camera_weights`` or
+        ``blend_bands`` > 0."""
+        if images_dic is None:
+            self.exposure_gains = None
+            return None
+        frames = self._frame_set(images_dic, "compensate_exposure")
+        cw = self._camera_weight_list()
+        if cw is None:
+            raise ValueError("exposure gains compensate the camera-weighted and multi-band blends: set camera_weights "
+                             "or blend_bands > 0 too")
+        # the gains are estimated on the uncut weights and uncompensated samples: a plan without seams or gains
+        plan = self._engine_().plan_for(self.stitchers, [f.shape for f in frames], camera_weights=cw,
+                                        blend_bands=self._blend_bands())
+        if plan is None:
+            raise ValueError("compensate_exposure needs a calibrated chain")
+        by_cam = plan.estimate_gains(frames)
+        self.exposure_gains = {str(label): by_cam.get(i, 1.0) for i, label in enumerate(self.img_labels)}
+        return dict(self.exposure_gains)
+
+    def _exposure_gains(self):
+        """``exposure_gains`` checked and as a tuple of floats in camera order (missing labels 1), or None."""
+        g = self.exposure_gains
+        if g is None:
+            return None
+        if self._camera_weight_list() is None:
+            raise ValueError("exposure gains compensate the camera-weighted and multi-band blends: set camera_weights "
+                             "or blend_bands > 0 too")
+        if not isinstance(g, dict):
+            raise ValueError("exposure_gains must be None or a dict {label: gain}, got %r" % (type(g),))
+        by_label = {str(k): v for k, v in g.items()}
+        labels = [str(l) for l in self.img_labels]
+        unknown = sorted(set(by_label) - set(labels))
+        if unknown:
+            raise ValueError("exposure_gains names unknown cameras %r (cameras: %r)" % (unknown, labels))
+        out = []
+        for label in labels:
+            v = by_label.get(label, 1.0)
+            if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)) or \
+                    not np.isfinite(float(v)) or float(v) < 0:
+                raise ValueError("exposure_gains[%r] must be a finite gain >= 0, got %r" % (label, v))
+            out.append(float(v))
+        return tuple(out)
 
     def _graphcut_seams(self):
         """``graphcut_seams`` checked: None, or ``(digest, frames)`` only with ``blend_bands`` > 0 and without
@@ -632,11 +695,11 @@ def edge_ramp(shape, width=64):
 
 
 def _composite(engine, stages, frames, batched, out=None, debugger=None, feather_log2=0, blend_weights=None,
-               camera_weights=None, blend_bands=0, voronoi_seams=False, graphcut_seams=None):
+               camera_weights=None, blend_bands=0, voronoi_seams=False, graphcut_seams=None, exposure_gains=None):
     """Run the fused kernel for this chain on these frames.  ``camera_weights``: one entry per camera (None or
     a uint8 map) for the camera-weighted blend, or None; ``blend_bands`` > 0 blends them in that many bands, with
     their masks cut at Voronoi seams when ``voronoi_seams`` or at the graph-cut seams of the frame-set
-    ``graphcut_seams = (digest, frames)``."""
+    ``graphcut_seams = (digest, frames)``; ``exposure_gains``: None or a gain per camera."""
     import torch  # local: keeps `import StitcherClass` cheap for calibration-only users
 
     on_device = _is_tensor(frames[0]) and frames[0].is_cuda
@@ -661,7 +724,7 @@ def _composite(engine, stages, frames, batched, out=None, debugger=None, feather
             return engine.plan_for(sub_stages, sub_shapes, device, feather_log2=feather_log2,
                                    blend_weights=[weight_of.get(id(st)) for st in sub_stages] if weight_of else None,
                                    camera_weights=camera_weights, blend_bands=blend_bands, voronoi_seams=voronoi_seams,
-                                   graphcut_seams=graphcut_seams)
+                                   graphcut_seams=graphcut_seams, exposure_gains=exposure_gains)
         except PlanUnsupported as e:
             if debugger is not None:
                 debugger.debugger(DEBUG_LEVEL_0, "[STITCHER] {}".format(e), log_type="err")

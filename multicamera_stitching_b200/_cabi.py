@@ -17,14 +17,14 @@ MCS_MAX_LAYERS = 16
 MCS_LAYER_COPY = 0
 MCS_LAYER_WARP = 1
 MCS_LAYER_REMAP = 2
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 # every symbol include/mcs.h declares
 EXPORTS = (
     "mcs_abi_version", "mcs_last_error", "mcs_plan_create", "mcs_plan_create_maps", "mcs_plan_destroy",
     "mcs_plan_owned_pixels", "mcs_plan_source_windows", "mcs_plan_source_spans", "mcs_copy_window_u8", "mcs_upload_pageable_u8", "mcs_stitch_u8", "mcs_plan_set_feather", "mcs_plan_set_blend", "mcs_plan_set_camera_weights",
     "mcs_plan_set_multiband", "mcs_plan_multiband_bands", "mcs_plan_set_voronoi_seams", "mcs_plan_seam_weights",
-    "mcs_plan_set_graphcut_seams",
+    "mcs_plan_set_graphcut_seams", "mcs_plan_estimate_gains", "mcs_plan_set_exposure_gains",
     "mcs_plan_last_variant",
     "mcs_plan_force_variant", "mcs_plan_rows_need_padding", "mcs_plan_promise_padded_rows",
     "mcs_plan_tiled_status", "mcs_plan_tiled_ctas_per_sm", "mcs_plan_tiled_stats", "mcs_launch_count",
@@ -120,6 +120,10 @@ def load(build_if_missing=False):
     lib.mcs_plan_seam_weights.argtypes = [_vp, ctypes.c_int, _vp, ctypes.c_int64]
     lib.mcs_plan_set_graphcut_seams.restype = ctypes.c_int
     lib.mcs_plan_set_graphcut_seams.argtypes = [_vp, ctypes.POINTER(_vp), _c_i64p]
+    lib.mcs_plan_estimate_gains.restype = ctypes.c_int
+    lib.mcs_plan_estimate_gains.argtypes = [_vp, ctypes.POINTER(_vp), _c_i64p, _c_f64p, _c_i64p, _c_f64p]
+    lib.mcs_plan_set_exposure_gains.restype = ctypes.c_int
+    lib.mcs_plan_set_exposure_gains.argtypes = [_vp, _c_f64p]
     lib.mcs_plan_tiled_ctas_per_sm.restype = ctypes.c_int
     lib.mcs_plan_tiled_ctas_per_sm.argtypes = [_vp]
     lib.mcs_plan_tiled_status.restype = ctypes.c_char_p
@@ -272,6 +276,7 @@ class Plan(object):
         self.blend_bands = 0           # its effective band count
         self.voronoi_seams = False     # set_voronoi_seams is in force
         self.graphcut_seams = False    # set_graphcut_seams is in force
+        self.exposure_gains = None     # set_exposure_gains: the gains per layer in force
 
     def close(self):
         if getattr(self, "_h", None) is not None and _lib is not None:
@@ -365,6 +370,7 @@ class Plan(object):
         n = self.n_layers
         self.multiband, self.blend_bands = False, 0   # every call switches the multi-band blend off
         self.voronoi_seams = self.graphcut_seams = False
+        self.exposure_gains = None                    # and clears the gains
         if weight_maps is None:
             check(_lib.mcs_plan_set_camera_weights(self._h, None, None), "mcs_plan_set_camera_weights")
             self._owned = None
@@ -432,6 +438,41 @@ class Plan(object):
             if not self.multiband:
                 self.graphcut_seams = self.voronoi_seams = False
         check(rc, "mcs_plan_set_graphcut_seams")
+
+    def fed_layers(self):
+        """The layers that feed the blends (non-empty clipped rectangle), in feed order."""
+        return [k for k, (x0, y0, x1, y1) in enumerate(self.rects) if x1 > x0 and y1 > y0]
+
+    def estimate_gains(self, src_ptrs, src_pitch, stats=False):
+        """Exposure gains per layer from one device frame-set (include/mcs.h mcs_plan_estimate_gains): per layer the
+        device pointer and row pitch of its camera's H x W x 3 frame.  Returns float64 [n_layers], or with ``stats``
+        ``(gains, N, I)`` (n_fed x n_fed, fed layers in feed order).  Synchronous; the plan is unchanged."""
+        n = self.n_layers
+        if len(src_ptrs) != n or len(src_pitch) != n:
+            raise ValueError("estimate_gains needs one frame per layer (%d)" % n)
+        m = len(self.fed_layers())
+        gains = np.zeros(n, np.float64)
+        N = np.zeros((m, m), np.int64)
+        I = np.zeros((m, m), np.float64)
+        ptrs = (_vp * n)(*[int(p) for p in src_ptrs])
+        pitch = (ctypes.c_int64 * n)(*[int(p) for p in src_pitch])
+        check(_lib.mcs_plan_estimate_gains(self._h, ptrs, pitch, gains.ctypes.data_as(_c_f64p),
+                                           N.ctypes.data_as(_c_i64p), I.ctypes.data_as(_c_f64p)),
+              "mcs_plan_estimate_gains")
+        return (gains, N, I) if stats else gains
+
+    def set_exposure_gains(self, gains):
+        """Compensate the camera-weighted and multi-band blends with these gains per layer (include/mcs.h
+        mcs_plan_set_exposure_gains); None switches the compensation off."""
+        if gains is None:
+            check(_lib.mcs_plan_set_exposure_gains(self._h, None), "mcs_plan_set_exposure_gains")
+            self.exposure_gains = None
+            return
+        g = np.ascontiguousarray(gains, dtype=np.float64).reshape(-1)
+        if g.size != self.n_layers:
+            raise ValueError("set_exposure_gains needs one gain per layer (%d), got %d" % (self.n_layers, g.size))
+        check(_lib.mcs_plan_set_exposure_gains(self._h, g.ctypes.data_as(_c_f64p)), "mcs_plan_set_exposure_gains")
+        self.exposure_gains = tuple(float(v) for v in g)
 
     def seam_weights(self, layer):
         """The seam-cut mask of ``layer`` over its visible rectangle clipped to the panorama (uint8 h x w)."""

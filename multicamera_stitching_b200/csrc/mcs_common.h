@@ -8,7 +8,7 @@
 
 #include "mcs.h"
 
-#define MCS_ABI_VERSION 5
+#define MCS_ABI_VERSION 6
 
 // ---- error plumbing -------------------------------------------------------
 void mcs_set_error(const char* fmt, ...);
@@ -177,6 +177,10 @@ struct mcs_plan {
     int seams_on;            // the weight pyramids were built from the seam-cut weights
     uint8_t* d_seam[MCS_MAX_LAYERS];   // per fed layer: the seam-cut weights over its clipped rectangle (row pitch =
                              // its width), nullptr for a layer that feeds nothing or while the seams are off
+    // exposure compensation of the camera-weighted and multi-band blends (mcs_plan_set_exposure_gains,
+    // mcs_exposure.cu)
+    int gains_on;            // every camera's rounded sample goes through its layer's table
+    uint8_t* d_gain_lut;     // [MCS_MAX_LAYERS][256]: saturate_u8(rint(v * gain of the layer))
 };
 
 
@@ -224,6 +228,14 @@ void mcs_seams_fill(const mcs_plan* plan, uint8_t* const* planes);
 // samples of one frame-set (src / src_pitch per layer, 3 channels) into plan->d_seam (synchronous).  On any failure
 // the plan is unchanged.
 int mcs_graphcut_build(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch);
+// Launches gc_sample_kernel: img[k] (3 bytes a pixel over layer k's clipped rectangle) = the overwrite sample v_k of
+// every fed layer k, through the plan's gain tables when `gains` (and the plan has them).  Returns the fed layers (in
+// feed order) in fed[] and their count.
+int mcs_graphcut_sample(const mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch, uint8_t* const* img,
+                        bool gains, int* fed);
+
+// Exposure compensation (mcs_exposure.cu): frees the gain tables.
+void mcs_exposure_free(mcs_plan* plan);
 
 // Tiled variant (mcs_stitch_tiled.cu): why it cannot serve a call (nullptr = it can), and its launch.
 const char* mcs_tiled_blocker(const mcs_plan* plan, const uint8_t* const* src, const int64_t* pitch,

@@ -218,6 +218,7 @@ extern "C" int mcs_plan_destroy(mcs_plan* plan) {
     }
     mcs_multiband_free(plan);
     mcs_seams_free(plan);
+    mcs_exposure_free(plan);
     mcs_plan_free_tiles(plan);
     free_maps(plan);
     delete plan;
@@ -508,6 +509,7 @@ static void free_cwmaps(mcs_plan* plan) {
     plan->mb_on = 0;
     mcs_multiband_free(plan);
     mcs_seams_free(plan);
+    mcs_exposure_free(plan);
 }
 
 extern "C" int mcs_plan_set_camera_weights(mcs_plan* plan, const uint8_t* const* weight_maps, const int64_t* map_pitch) {

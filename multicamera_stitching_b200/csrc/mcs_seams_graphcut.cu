@@ -4,7 +4,7 @@
 //
 //   1. seam_fill_kernel (mcs_seams.cu)  every new plane = the weight sample w_k
 //      gc_sample_kernel                 every fed layer's v_k over its clipped rectangle, 3 bytes a pixel (the sample
-//                                       mb_level0_kernel takes)
+//                                       mb_level0_kernel takes, through the exposure tables when the plan has gains)
 //   2. per overlapping pair (i, j), i < j in feed order, on the submask (the overlap ROI grown by MCS_GC_GAP, reading
 //      0 outside each plane), each pair cutting the planes the earlier pairs left:
 //      gc_caps_kernel    D(p) = sum_c (I1_c - I2_c)^2, the grid capacities D(p) + D(q) + 1 (+ MCS_GC_PENALTY where a
@@ -45,6 +45,7 @@ struct GcSample {
     uint8_t* img[MCS_MAX_LAYERS];   // 3 bytes a pixel over the clipped rectangle
     int4 rect[MCS_MAX_LAYERS];      // clipped rectangle {x0, y0, x1, y1}
     int layer[MCS_MAX_LAYERS];      // fed layers in feed order
+    const uint8_t* lut;             // GAIN: per layer the 256-entry exposure table (mcs_exposure.cu)
 };
 
 struct GcPair {
@@ -62,7 +63,9 @@ struct GcPair {
     int* flags;             // MCS_GC_RELAX change flags of a relaxation batch, then the active count
 };
 
-// Plan time: v_k of every fed layer (grid.z = fed layer): the overwrite sample, taps outside the source read 0.
+// Plan time: v_k of every fed layer (grid.z = fed layer): the overwrite sample, taps outside the source read 0;
+// with GAIN its value in the layer's exposure table, the sample the blends then take.
+template <bool GAIN>
 __global__ void __launch_bounds__(GC_BX * GC_BY) gc_sample_kernel(const __grid_constant__ GcSample a) {
     const int k = a.layer[blockIdx.z];
     const int4 r = a.rect[k];
@@ -86,7 +89,7 @@ __global__ void __launch_bounds__(GC_BX * GC_BY) gc_sample_kernel(const __grid_c
         if (y0in && x1in) s += w01 * (int)__ldg(r0 + 3 + ch);
         if (y1in && x0in) s += w10 * (int)__ldg(r0 + pitch + ch);
         if (y1in && x1in) s += w11 * (int)__ldg(r0 + pitch + 3 + ch);
-        out[ch] = (uint8_t)(s >> 15);
+        out[ch] = GAIN ? __ldg(a.lut + k * 256 + (s >> 15)) : (uint8_t)(s >> 15);
     }
 }
 
@@ -331,10 +334,12 @@ static long long gc_global_relabel(const GcPair& p, int* host, int& launches, cu
     }
 }
 
-int mcs_graphcut_build(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch) {
-    GcSample a;
+// The sample table of every layer; returns the fed layers' count, their widest and tallest rectangle in bw, bh.
+static int gc_sample_args(const mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch, GcSample& a,
+                          int& bw, int& bh) {
     memset(&a, 0, sizeof(a));
-    int n = 0, bw = 0, bh = 0;
+    int n = 0;
+    bw = bh = 0;
     for (int k = 0; k < plan->n_layers; ++k) {
         const McsLayer& L = plan->layers[k];
         a.g[k] = L;
@@ -349,6 +354,37 @@ int mcs_graphcut_build(mcs_plan* plan, const uint8_t* const* src, const int64_t*
             bh = y1 - y0 > bh ? y1 - y0 : bh;
         }
     }
+    a.lut = plan->gains_on ? plan->d_gain_lut : nullptr;
+    return n;
+}
+
+static void gc_sample_launch(const GcSample& a, int n, int bw, int bh) {
+    const dim3 grid((bw + GC_BX - 1) / GC_BX, (bh + GC_BY - 1) / GC_BY, n), block(GC_BX, GC_BY, 1);
+    if (a.lut)
+        gc_sample_kernel<true><<<grid, block>>>(a);
+    else
+        gc_sample_kernel<false><<<grid, block>>>(a);
+    mcs_count_launch(1);
+}
+
+int mcs_graphcut_sample(const mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch, uint8_t* const* img,
+                        bool gains, int* fed) {
+    GcSample a;
+    int bw, bh;
+    const int n = gc_sample_args(plan, src, src_pitch, a, bw, bh);
+    if (!gains) a.lut = nullptr;
+    for (int u = 0; u < n; ++u) {
+        fed[u] = a.layer[u];
+        a.img[a.layer[u]] = img[a.layer[u]];
+    }
+    if (n > 0) gc_sample_launch(a, n, bw, bh);
+    return n;
+}
+
+int mcs_graphcut_build(mcs_plan* plan, const uint8_t* const* src, const int64_t* src_pitch) {
+    GcSample a;
+    int bw, bh;
+    const int n = gc_sample_args(plan, src, src_pitch, a, bw, bh);
     for (int u = 0; u < n; ++u)
         MCS_CHECK_ARG(src[a.layer[u]] != nullptr, "mcs_plan_set_graphcut_seams: src[%d] is NULL", a.layer[u]);
     int pi[MCS_MAX_LAYERS * MCS_MAX_LAYERS / 2], pj[MCS_MAX_LAYERS * MCS_MAX_LAYERS / 2];
@@ -381,8 +417,7 @@ int mcs_graphcut_build(mcs_plan* plan, const uint8_t* const* src, const int64_t*
     if (e == cudaSuccess) e = cudaMallocHost(&host, (MCS_GC_RELAX + 1) * sizeof(int));
     if (e == cudaSuccess && n > 0) {
         mcs_seams_fill(plan, planes);
-        gc_sample_kernel<<<dim3((bw + GC_BX - 1) / GC_BX, (bh + GC_BY - 1) / GC_BY, n), dim3(GC_BX, GC_BY, 1)>>>(a);
-        ++launches;
+        gc_sample_launch(a, n, bw, bh);   // compensated when the plan has gains: the cut compares what is blended
         e = cudaGetLastError();
     }
     for (int q = 0; q < np && e == cudaSuccess && rc == MCS_OK; ++q) {

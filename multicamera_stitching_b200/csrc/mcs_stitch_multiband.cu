@@ -57,6 +57,8 @@ struct MbArgs {
     long long dst_pitch, dst_frame_stride;
     // plan time: per layer the seam-cut weights over its rectangle (mcs_seams.cu), nullptr = sample the map
     const uint8_t* seam[MCS_MAX_LAYERS];
+    // per launch, GAIN: per layer the 256-entry exposure table (mcs_exposure.cu)
+    const uint8_t* lut;
 };
 
 struct McsMultiband {
@@ -118,8 +120,9 @@ __device__ __forceinline__ void pyr_up_at(const int16_t* __restrict__ p, int sw,
     for (int c = 0; c < C; ++c) out[c] = clamp16(s[c] >> 6);
 }
 
-// Level 0 of every camera of the sub-batch: grid.z = camera + n_cams * frame.
-template <int C>
+// Level 0 of every camera of the sub-batch: grid.z = camera + n_cams * frame.  GAIN: the rounded sample goes through
+// the layer's exposure table.
+template <int C, bool GAIN>
 __global__ void __launch_bounds__(MB_BX * MB_BY) mb_level0_kernel(const __grid_constant__ MbArgs a) {
     const int j = blockIdx.z % a.n_cams, f = blockIdx.z / a.n_cams;
     const MbCam& c = a.cam[j];
@@ -144,7 +147,7 @@ __global__ void __launch_bounds__(MB_BX * MB_BY) mb_level0_kernel(const __grid_c
         if (y0in && x1in) s += w01 * (int)__ldg(r0 + C + ch);
         if (y1in && x0in) s += w10 * (int)__ldg(r0 + pitch + ch);
         if (y1in && x1in) s += w11 * (int)__ldg(r0 + pitch + C + ch);
-        out[ch] = (int16_t)(s >> 15);
+        out[ch] = GAIN ? (int16_t)__ldg(a.lut + c.k * 256 + (s >> 15)) : (int16_t)(s >> 15);
     }
 }
 
@@ -390,7 +393,10 @@ static void mb_launch_batch(const McsMultiband* m, const MbArgs& a, int nf, cuda
     const dim3 block(MB_BX, MB_BY, 1);
     const int n = a.n_bands;
     if (a.n_cams > 0) {
-        mb_level0_kernel<C><<<mb_grid(m->max_bw, m->max_bh, a.n_cams * nf), block, 0, stream>>>(a);
+        if (a.lut)
+            mb_level0_kernel<C, true><<<mb_grid(m->max_bw, m->max_bh, a.n_cams * nf), block, 0, stream>>>(a);
+        else
+            mb_level0_kernel<C, false><<<mb_grid(m->max_bw, m->max_bh, a.n_cams * nf), block, 0, stream>>>(a);
         for (int i = 0; i < n; ++i)
             mb_pyrdown_kernel<C, false><<<mb_grid(m->max_bw >> (i + 1), m->max_bh >> (i + 1), a.n_cams * nf), block, 0,
                                           stream>>>(a, i);
@@ -408,6 +414,7 @@ int mcs_launch_multiband(const mcs_plan* plan, const uint8_t* const* src, const 
     MbArgs a = m->a;
     a.dst_pitch = dst_pitch;
     a.dst_frame_stride = dst_frame_stride;
+    a.lut = plan->gains_on ? plan->d_gain_lut : nullptr;
     for (int f0 = 0; f0 < n_frames; f0 += MCS_MB_FRAMES) {
         const int nf = n_frames - f0 < MCS_MB_FRAMES ? n_frames - f0 : MCS_MB_FRAMES;
         for (int k = 0; k < plan->n_layers; ++k) {

@@ -30,6 +30,7 @@ struct CwArgs {
     int n_layers;
     int out_w, out_h;
     int n_frames;
+    const uint8_t* lut;   // GAIN: per layer the 256-entry exposure table (mcs_exposure.cu)
 };
 
 #define CW_BX 64
@@ -81,7 +82,8 @@ __device__ __forceinline__ void contrib_sample(const CwArgs& a, const Contrib& q
     for (int c = 0; c < C; ++c) v[c] = (int)(__dp2a_lo(q.wl, p1[c], __dp2a_lo(q.wu, p0[c], 16384u)) >> 15);
 }
 
-template <int C, bool WORDS>
+// GAIN: every camera's rounded sample v_k is replaced by lut_k[v_k] before it is used.
+template <int C, bool WORDS, bool GAIN>
 __global__ void __launch_bounds__(CW_BX * CW_BY)
 mcs_stitch_weighted_kernel(const __grid_constant__ CwArgs a) {
     const int x = blockIdx.x * CW_BX + threadIdx.x;
@@ -136,6 +138,11 @@ mcs_stitch_weighted_kernel(const __grid_constant__ CwArgs a) {
             for (int c = 0; c < C; ++c) r[c] = 0;
         } else if (n == 1) {
             contrib_sample<C, WORDS>(a, q[0], f, r);
+            if (GAIN) {
+                const uint8_t* t = a.lut + ((q[0].meta >> 8) & 0xff) * 256;
+#pragma unroll
+                for (int c = 0; c < C; ++c) r[c] = __ldg(t + r[c]);
+            }
         } else {
             uint32_t acc[C];
 #pragma unroll
@@ -145,6 +152,11 @@ mcs_stitch_weighted_kernel(const __grid_constant__ CwArgs a) {
                 if (j < n) {
                     int v[C];
                     contrib_sample<C, WORDS>(a, q[j], f, v);
+                    if (GAIN) {
+                        const uint8_t* t = a.lut + ((q[j].meta >> 8) & 0xff) * 256;
+#pragma unroll
+                        for (int c = 0; c < C; ++c) v[c] = __ldg(t + v[c]);
+                    }
                     const uint32_t wk = q[j].meta >> 16;
 #pragma unroll
                     for (int c = 0; c < C; ++c) acc[c] += wk * (uint32_t)v[c];
@@ -240,13 +252,25 @@ int mcs_launch_weighted(const mcs_plan* plan, const uint8_t* const* src, const i
     }
     dim3 block(CW_BX, CW_BY, 1);
     dim3 grid((plan->out_w + CW_BX - 1) / CW_BX, (plan->out_h + CW_BY - 1) / CW_BY, (n_frames + CW_FRAMES - 1) / CW_FRAMES);
-    switch (plan->channels * 2 + (words ? 1 : 0)) {
-        case 2: mcs_stitch_weighted_kernel<1, false><<<grid, block, 0, stream>>>(a); break;
-        case 3: mcs_stitch_weighted_kernel<1, true><<<grid, block, 0, stream>>>(a); break;
-        case 6: mcs_stitch_weighted_kernel<3, false><<<grid, block, 0, stream>>>(a); break;
-        case 7: mcs_stitch_weighted_kernel<3, true><<<grid, block, 0, stream>>>(a); break;
-        case 8: mcs_stitch_weighted_kernel<4, false><<<grid, block, 0, stream>>>(a); break;
-        default: mcs_stitch_weighted_kernel<4, true><<<grid, block, 0, stream>>>(a); break;
+    if (plan->gains_on) {
+        a.lut = plan->d_gain_lut;
+        switch (plan->channels * 2 + (words ? 1 : 0)) {
+            case 2: mcs_stitch_weighted_kernel<1, false, true><<<grid, block, 0, stream>>>(a); break;
+            case 3: mcs_stitch_weighted_kernel<1, true, true><<<grid, block, 0, stream>>>(a); break;
+            case 6: mcs_stitch_weighted_kernel<3, false, true><<<grid, block, 0, stream>>>(a); break;
+            case 7: mcs_stitch_weighted_kernel<3, true, true><<<grid, block, 0, stream>>>(a); break;
+            case 8: mcs_stitch_weighted_kernel<4, false, true><<<grid, block, 0, stream>>>(a); break;
+            default: mcs_stitch_weighted_kernel<4, true, true><<<grid, block, 0, stream>>>(a); break;
+        }
+    } else {
+        switch (plan->channels * 2 + (words ? 1 : 0)) {
+            case 2: mcs_stitch_weighted_kernel<1, false, false><<<grid, block, 0, stream>>>(a); break;
+            case 3: mcs_stitch_weighted_kernel<1, true, false><<<grid, block, 0, stream>>>(a); break;
+            case 6: mcs_stitch_weighted_kernel<3, false, false><<<grid, block, 0, stream>>>(a); break;
+            case 7: mcs_stitch_weighted_kernel<3, true, false><<<grid, block, 0, stream>>>(a); break;
+            case 8: mcs_stitch_weighted_kernel<4, false, false><<<grid, block, 0, stream>>>(a); break;
+            default: mcs_stitch_weighted_kernel<4, true, false><<<grid, block, 0, stream>>>(a); break;
+        }
     }
     mcs_count_launch(1);
     MCS_CHECK_CUDA(cudaGetLastError());

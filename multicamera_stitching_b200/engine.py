@@ -88,7 +88,7 @@ class CompiledPlan(object):
     """A flattened chain plus its ``mcs_plan`` on one device."""
 
     def __init__(self, flat, device, feather_log2=0, blend_weights=None, camera_weights=None, blend_bands=0,
-                 voronoi_seams=False, graphcut_frames=None):
+                 voronoi_seams=False, graphcut_frames=None, exposure_gains=None):
         self.flat = flat
         self.device = torch.device(device)
         self.feather_log2 = int(feather_log2)
@@ -124,6 +124,8 @@ class CompiledPlan(object):
                         if e.code == _cabi.MCS_ERR_UNSUPPORTED:
                             raise PlanUnsupported(str(e))
                         raise
+                if exposure_gains is not None:   # before the graph-cut seams: they are found on compensated samples
+                    self.handle.set_exposure_gains([exposure_gains[l.cam] for l in flat.layers])
                 if graphcut_frames is not None:
                     self._find_graphcut_seams(graphcut_frames)
             # rows that are not a multiple of 4 bytes: run() always passes them through its
@@ -134,18 +136,32 @@ class CompiledPlan(object):
         self.cams = [l.cam for l in flat.layers]
         self.out_w, self.out_h, self.channels = flat.out_w, flat.out_h, flat.channels
 
-    def _find_graphcut_seams(self, frames_by_cam):
-        """Upload one host frame-set (``frames_by_cam[c]``: H x W x 3 uint8), find the graph-cut seams on it
-        (include/mcs.h mcs_plan_set_graphcut_seams) and drop the upload."""
+    def _upload_frame_set(self, frames_by_cam, what):
+        """One host frame-set (``frames_by_cam[c]``: H x W x 3 uint8) on the device: ``{cam: tensor}``."""
         dev = {}
         for l in self.flat.layers:
             f = np.asarray(frames_by_cam[l.cam])
             want = tuple(l.src_hw) + (3,)
             if f.dtype != np.uint8 or f.shape != want:
-                raise ValueError("graph-cut seams: camera %d's frame is %s %r, the plan needs uint8 %r"
-                                 % (l.cam, f.dtype, f.shape, want))
+                raise ValueError("%s: camera %d's frame is %s %r, the plan needs uint8 %r"
+                                 % (what, l.cam, f.dtype, f.shape, want))
             if l.cam not in dev:
                 dev[l.cam] = torch.from_numpy(np.array(f)).to(self.device)
+        return dev
+
+    def estimate_gains(self, frames_by_cam):
+        """The exposure gains of one host frame-set (include/mcs.h mcs_plan_estimate_gains), per camera
+        (``{cam: gain}``).  The plan is unchanged."""
+        with torch.cuda.device(self.device):
+            dev = self._upload_frame_set(frames_by_cam, "exposure gains")
+            gains = self.handle.estimate_gains([dev[l.cam].data_ptr() for l in self.flat.layers],
+                                               [dev[l.cam].stride(0) for l in self.flat.layers])
+        return {l.cam: float(g) for l, g in zip(self.flat.layers, gains)}
+
+    def _find_graphcut_seams(self, frames_by_cam):
+        """Upload one host frame-set (``frames_by_cam[c]``: H x W x 3 uint8), find the graph-cut seams on it
+        (include/mcs.h mcs_plan_set_graphcut_seams) and drop the upload."""
+        dev = self._upload_frame_set(frames_by_cam, "graph-cut seams")
         try:
             self.handle.set_graphcut_seams([dev[l.cam].data_ptr() for l in self.flat.layers],
                                            [dev[l.cam].stride(0) for l in self.flat.layers])
@@ -311,10 +327,11 @@ class CompositeEngine(object):
         return torch.device(self._device)
 
     def plan_for(self, stages, cam_shapes, device=None, feather_log2=0, blend_weights=None, camera_weights=None,
-                 blend_bands=0, voronoi_seams=False, graphcut_seams=None):
+                 blend_bands=0, voronoi_seams=False, graphcut_seams=None, exposure_gains=None):
         """Compiled plan for this chain state and these frame shapes, or None
         when no stage is calibrated (decided on the host, no device needed).  ``graphcut_seams``: None or
-        ``(digest, frames by camera)`` of the frame-set the graph-cut seams are found on."""
+        ``(digest, frames by camera)`` of the frame-set the graph-cut seams are found on; ``exposure_gains``: None
+        or a tuple of gains by camera."""
         shapes = tuple(tuple(int(v) for v in s) for s in cam_shapes)
         sig = tuple(stage_signature(st) for st in stages)
         if all(s is None for s in sig):
@@ -332,7 +349,8 @@ class CompositeEngine(object):
         blend_bands = int(blend_bands or 0)
         voronoi_seams = bool(voronoi_seams)
         gkey = None if graphcut_seams is None else graphcut_seams[0]
-        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands, voronoi_seams, gkey)
+        ekey = None if exposure_gains is None else tuple(float(g) for g in exposure_gains)
+        key = (str(device), shapes, sig, feather_log2, wkey, ckey, blend_bands, voronoi_seams, gkey, ekey)
         if key in self._plans:
             self._plans[key] = self._plans.pop(key)      # most recently used last
         else:
@@ -340,7 +358,8 @@ class CompositeEngine(object):
             while len(self._plans) >= self.max_plans:     # evict the least recently used, one at a time
                 self._plans.pop(next(iter(self._plans)))
             self._plans[key] = (CompiledPlan(flat, device, feather_log2, blend_weights, camera_weights, blend_bands,
-                                             voronoi_seams, None if graphcut_seams is None else graphcut_seams[1])
+                                             voronoi_seams, None if graphcut_seams is None else graphcut_seams[1],
+                                             ekey)
                                 if flat is not None else None)
         return self._plans[key]
 
