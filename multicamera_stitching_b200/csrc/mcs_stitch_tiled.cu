@@ -1,16 +1,17 @@
 // Variant 2 ("tiled") of the fused warp + paste kernel (sm_100a).
 //
-// Persistent CTAs of eight warps (two CTAs per SM) walk the plan's tile table.  A work unit is
-// one 128 x 16 output cell of one layer for one frame; a CHUNK is a run of consecutive frames of
-// one cell.
+// Persistent CTAs (two per SM) of eight resampling warps and one producer warpgroup walk the plan's
+// tile table.  A work unit is one 128 x 16 output cell of one layer for one frame; a CHUNK is a run
+// of consecutive frames of one cell.
 //
 //   staging   The bounding box of the source pixels a WARP / COPY cell touches is brought into a
 //             ring of shared-memory buffers by the TMA engine (cp.async.bulk.tensor.3d, zero fill
-//             outside the image = cv2's BORDER_CONSTANT 0), one box per unit, `stages - 2` units
-//             ahead of the consumers.  There is no producer warp: lane 0 of warp 0 issues one box
-//             per unit it consumes, into the slot all warps released two units earlier (full /
-//             empty mbarriers per slot, no CTA-wide barrier anywhere in the loop); its per-unit
-//             cursor is in registers, the chunk walk behind it in shared memory.
+//             outside the image = cv2's BORDER_CONSTANT 0), one box per unit.  One thread of the
+//             producer warpgroup claims the chunks, copies their records and issues every box as
+//             soon as all resampling warps have released its slot (full / empty mbarriers per slot,
+//             no CTA-wide barrier anywhere in the loop), so the ring is kept full whatever warp is
+//             behind.  The producer warpgroup gives its registers to the resampling warps
+//             (setmaxnreg): 32 a thread against 104, which keeps two CTAs per SM.
 //   resample  warp w owns cell rows w and w + 8, lane l the columns l, l+32, l+64, l+96
 //             (consecutive lanes read consecutive source pixels: bank-conflict free).
 //
@@ -37,17 +38,21 @@
 #include <stdlib.h>
 
 #define TILED_WARPS MCS_TILED_WARPS
-#define TILED_THREADS (32 * TILED_WARPS)
+#define TILED_THREADS (32 * TILED_WARPS)            // resampling threads; the producer warpgroup follows them
+#define TILED_CTA_THREADS (TILED_THREADS + 128)
 #define TILED_MIN_CTAS 2
+// setmaxnreg moves registers inside one CTA's pool, which is fixed at launch: 384 threads x 80 registers (two
+// CTAs per SM).  128 x 32 + 256 x 104 fills it exactly; the resampling loops need no spill at 104.
+#define TILED_PRODUCER_REGS 32
+#define TILED_CONSUMER_REGS 104
 #define TILED_PX_BATCH 4   // pixels whose loads are issued before the first store
 #define TILED_SMEM_BUDGET_KB 113   // per CTA, so that TILED_MIN_CTAS CTAs fit an SM
 #define TILED_MAX_STAGES 8
-#define TILED_LOOKAHEAD_SLACK 2   // boxes are issued `stages - TILED_LOOKAHEAD_SLACK` units ahead
 
 struct TiledArgs {
     CUtensorMap tmap[MCS_MAX_LAYERS];   // source of each layer as (row words, rows, frames) of uint32
     const McsTile* tiles;
-    const int4* issue;                  // per tile {layer, bx, by, box bytes}: all the box issuer needs of a tile
+    const int4* issue;                  // per tile {layer, bx, by, box bytes}: all the producer needs of a tile
     const McsLayer* layers;
     const uint32_t* desc;               // plan-time pixel descriptors, 2048 per WARP tile
     uint8_t* dst;
@@ -138,6 +143,17 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, int lin
 #endif
     } while (!done);
 }
+__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {   // mbar_wait without the wait
+    uint32_t done;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(done)
+        : "r"(bar), "r"(parity)
+        : "memory");
+    return done != 0;
+}
 // The box origin must sit on a 16-byte boundary of the source row (c0 * 4 bytes % 16 == 0): the
 // TMA unit raises an illegal-instruction fault otherwise.  mcs_tiles.cu places the boxes so.
 __device__ __forceinline__ void tma_load_3d(uint32_t smem_dst, const CUtensorMap* map, int c0, int c1, int c2,
@@ -155,11 +171,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t smem_dst, const void* src, uin
                  "l"(src), "r"(bytes), "r"(bar)
                  : "memory");
 }
-// 16-byte asynchronous copy global -> shared of the issuing thread (no register in flight).
-__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 // Shared-memory accesses by absolute shared-window address held in a register.  `volatile` keeps
 // them ordered with barriers and with each other; arithmetic is still scheduled across them.
 __device__ __forceinline__ uint32_t lds32(uint32_t addr) {
@@ -229,28 +240,18 @@ __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
 #define MCS_STG128(p, v) __stcs((p), (v))   // streaming: written once, never re-read
 
 // ---- work split --------------------------------------------------------------------------------
-// The scheduler is one thread (lane 0 of warp 0, which also issues the boxes): it claims chunk ids
-// from the global counter, decodes them (once: the decode costs a few integer divisions) and publishes
-// them to the CTA through a small ring in shared memory, by CTA-local sequence number k = 0, 1, 2 ...
-// Consumers look at chunk k once `published > k`; a tile of -1 ends the CTA.  The scheduler stays at most TILED_SCHED_LEAD chunks
-// ahead of its own warp's consumption and every warp within two chunks of warp 0 (the chunk-record
-// buffers see to that), so a ring of TILED_QD entries is never overrun.
+// The scheduler is the producer thread: it claims chunk ids from the global counter, decodes them (once: the
+// decode costs a few integer divisions) and publishes them to the CTA through a small ring in shared memory, by
+// CTA-local sequence number k = 0, 1, 2 ...  Consumers look at chunk k once `published > k`; a tile of -1 ends
+// the CTA.  The producer claims at most two chunks past the one it issues boxes for, and it issues boxes for
+// chunk k only after every warp has taken chunk k - 2's record out of its buffer, so a ring of TILED_QD entries
+// is never overrun.
 #define TILED_QD 32
-#define TILED_SCHED_LEAD 10
 struct SchedMem {
     int published;       // sequence numbers [0, published) have their id in ids[]
-    int pre_k;           // sequence number whose issue record sits in `pre` (-1: none)
-    int pad[2];
-    int4 pre;            // filled by a cp.async issued one chunk earlier
-    int4 pre_ov[MCS_BAND_MAX_OVERLAYS];   // BAND tiles: the records of the overlay boxes, prefetched with `pre`
-    int4 cur_ov[MCS_BAND_MAX_OVERLAYS];   // ... of the chunk the issuer stands in
-    int nl, li;          // boxes per frame of that chunk (1; BAND tiles 2 or 3) / the next one to issue
-    int li0;             // first box of a frame (1 for zero-base BAND tiles, whose owner stages nothing)
-    int pad2;
+    int pad[3];
     int4 chunk[TILED_QD];   // {tile, frame block, first frame, end frame} of sequence number k at [k % QD]; tile -1 = no more work
 };
-static_assert(offsetof(SchedMem, pre) % 16 == 0 && offsetof(SchedMem, pre_ov) % 16 == 0 && offsetof(SchedMem, cur_ov) % 16 == 0,
-              "SchedMem records must be 16-byte aligned");
 
 __device__ __forceinline__ int ld_volatile_shared(uint32_t addr) {
     int v;
@@ -258,36 +259,13 @@ __device__ __forceinline__ int ld_volatile_shared(uint32_t addr) {
     return v;
 }
 
-// Scheduler + box issuer state, in registers of the one thread that uses it.
-struct Issuer {
-    int k;                // sequence number of the chunk whose boxes are being issued
-    int f, f1;            // next frame / end of that chunk
-    int frame0;           // first frame of its block
-    int layer, bx, by;    // its box
-    uint32_t bytes;
-    int slot;
-    uint32_t phase;
+// Claim state, in registers of the producer thread.
+struct Sched {
     int claimed;          // sequence numbers published so far
     int ended;            // the end marker has been published
-    int issued;           // boxes issued so far
-    int zero;             // the chunk the issuer stands in has no boxes (ZERO class)
     int has_pend;         // a claim is in flight: its result is `pend`
     unsigned pend;
 };
-
-__device__ __forceinline__ void issuer_init(SchedMem* sm, Issuer& c, bool writer) {
-    if (writer) {
-        sm->published = 0;
-        sm->pre_k = -1;
-        // nl / li / li0 (BAND tiles) are written whenever the issuer enters a chunk from the BAND-aware path, which is the
-        // only path that reads them
-    }
-    c.k = -1;
-    c.f = c.f1 = c.frame0 = c.layer = c.bx = c.by = c.slot = 0;
-    c.bytes = c.phase = 0;
-    c.claimed = c.ended = c.issued = c.zero = c.has_pend = 0;
-    c.pend = 0u;
-}
 
 // Chunk id -> frame block, tile and frames [f0, f1) of the block.  Inside a block the sweep INTERLEAVES the
 // resampled tiles (FAST, WARP: bound by the SM) evenly with the COPY and ZERO tiles (bound by DRAM): with the
@@ -330,10 +308,10 @@ __device__ __forceinline__ int tile_class(const TiledArgs& a, int t) {
            : t < a.class_first[4] ? MCS_TILE_COPY : MCS_TILE_ZERO;
 }
 
-// Make sure sequence numbers below `upto` are published (or the end marker is).  Scheduler thread.  One claim
+// Make sure sequence numbers below `upto` are published (or the end marker is).  Producer thread.  One claim
 // is kept in flight: the atomic is issued when the previous claim is published and its result read at the
 // next call, a chunk later, so the round trip to the counter is not on the thread's critical path.
-__device__ __forceinline__ void sched_ensure(const TiledArgs& a, SchedMem* sm, Issuer& c, int upto) {
+__device__ __forceinline__ void sched_ensure(const TiledArgs& a, SchedMem* sm, Sched& c, int upto) {
     while (!c.ended && c.claimed < upto) {
         unsigned g0;
         if (c.has_pend) {
@@ -357,107 +335,6 @@ __device__ __forceinline__ void sched_ensure(const TiledArgs& a, SchedMem* sm, I
         c.pend = atomicAdd(a.work, (unsigned)a.claim);
         c.has_pend = 1;
     }
-}
-
-// Called by the scheduler thread once per unit its warp consumes (`k_cons` = the chunk that warp is in,
-// `consumed` = the boxes it has consumed so far): issue the box of the next unit, if any, unless stages - 1
-// boxes are in flight already (the thread must never wait for a slot its own warp still has to release).  At a chunk boundary at most ONE new chunk is entered per call
-// (ZERO chunks have no boxes), which bounds the scheduler's lead.  The tile's issue record comes from shared
-// memory, where a cp.async started one chunk earlier has put it (a dependent global load here would stall
-// the issuing warp, and with it the CTA, for a DRAM round trip per chunk).
-// BANDS: the plan has BAND tiles (feather mode), whose units stage more than one box.  The issuing thread's path
-// sets the pace of its CTA - a handful of extra instructions and two more live registers on it cost the overwrite
-// mode 13 % when they were unconditional - so the multi-box logic exists only in the INBAND instantiation, which
-// the frame loop of the BAND tiles (and the prologue) calls, with its cursor (boxes per frame, next box) in shared
-// memory.  Everywhere else the issuer does not look ahead INTO a BAND chunk: it stops at its boundary until the
-// consumers get there (BAND tiles sit together at the start of the sweep, so that is one short bubble per CTA and
-// frame block), and inside any other chunk a unit is one box, as in the overwrite mode.
-template <bool BANDS, bool INBAND>
-__device__ __forceinline__ void issuer_step(const TiledArgs& a, SchedMem* sm, Issuer& c, int k_cons, int consumed,
-                                            uint32_t s_base, uint32_t s_full, uint32_t s_empty) {
-    if (c.issued - consumed >= a.stages - 1) return;
-    if (c.f == c.f1) {
-        const int kn = c.k + 1;
-        // through a run of ZERO chunks the issuer only keeps pace with the consumers: claiming ahead there
-        // would just take cheap chunks away from CTAs that have nothing else left
-        if (kn > k_cons + (c.zero ? 1 : TILED_SCHED_LEAD)) return;
-        sched_ensure(a, sm, c, kn + 1);
-        if (kn >= c.claimed) return;                 // past the end marker
-        const int4 e = sm->chunk[kn % TILED_QD];
-        if (e.x < 0) return;
-        // A BAND chunk is entered from a BAND frame loop only, and only when it is the chunk the consumers are in or
-        // the very next one: between two BAND chunks that are further apart the consumers run ordinary frame loops,
-        // whose issuer calls know nothing of multi-box units.
-        if (BANDS && e.x < a.class_first[1] && !(INBAND && kn <= k_cons + 1)) return;
-        c.k = kn;
-        const int t = e.x, blk = e.y, f0 = e.z, f1 = e.w;
-        c.zero = t >= a.class_first[MCS_N_CLASSES - 1];
-        if (c.zero || f0 == f1) return;   // ZERO chunk (or no frames): nothing to stage
-        c.f = f0;
-        c.f1 = f1;
-        c.frame0 = blk * a.frame_block;
-        int4 rec;
-        if (sm->pre_k == kn) {
-            cp_async_wait_all();
-            const uint4 r = lds128(smem_u32(&sm->pre));
-            rec = make_int4((int)r.x, (int)r.y, (int)r.z, (int)r.w);
-        } else {
-            rec = __ldg(a.issue + t);
-        }
-        c.layer = rec.x;
-        c.bx = rec.y;
-        c.by = rec.z;
-        c.bytes = (uint32_t)rec.w & 0xffffffu;
-        if (BANDS && INBAND) {
-            sm->nl = 1 + ((rec.w >> 24) & 15);
-            sm->li0 = (rec.w >> 28) & 1;   // zero-base BAND tile: no box of the owner, the unit starts at its first overlay
-            sm->li = sm->li0;
-            if ((rec.w >> 24) & 15) {   // BAND tile: the records of its overlay boxes
-#pragma unroll
-                for (int o = 0; o < MCS_BAND_MAX_OVERLAYS; ++o)
-                    sm->cur_ov[o] = sm->pre_k == kn ? sm->pre_ov[o] : __ldg(a.band_issue + t * (1 + MCS_BAND_MAX_OVERLAYS) + 1 + o);
-            }
-        }
-        sm->pre_k = -1;
-        if (kn + 1 < c.claimed) {                    // request the record of the chunk after this one
-            const int t2 = sm->chunk[(kn + 1) % TILED_QD].x;
-            if (t2 >= 0) {
-                if (t2 < a.class_first[MCS_N_CLASSES - 1]) {
-                    cp_async16(smem_u32(&sm->pre), a.issue + t2);
-                    if (BANDS && t2 < a.class_first[1]) {
-#pragma unroll
-                        for (int o = 0; o < MCS_BAND_MAX_OVERLAYS; ++o)
-                            cp_async16(smem_u32(&sm->pre_ov[o]), a.band_issue + t2 * (1 + MCS_BAND_MAX_OVERLAYS) + 1 + o);
-                    }
-                    sm->pre_k = kn + 1;
-                }
-            }
-        }
-    }
-    int layer = c.layer, bx = c.bx, by = c.by;
-    uint32_t bytes = c.bytes;
-    int li = 0;
-    if (BANDS && INBAND) {
-        li = sm->li;
-        if (li > 0) {
-            const int4 r = sm->cur_ov[li - 1];
-            layer = r.x; bx = r.y; by = r.z; bytes = (uint32_t)r.w;
-        }
-    }
-    mbar_wait(s_empty + 8 * c.slot, c.phase ^ 1, __LINE__);   // first trip round the ring: passes at once
-    mbar_expect_tx(s_full + 8 * c.slot, bytes);
-    tma_load_3d(s_base + c.slot * a.box_bytes, &a.tmap[layer], bx, by, c.frame0 + c.f, s_full + 8 * c.slot);
-    if (BANDS && INBAND) {
-        if (++li == sm->nl) {
-            li = sm->li0;
-            ++c.f;
-        }
-        sm->li = li;
-    } else {
-        ++c.f;
-    }
-    ++c.issued;
-    if (++c.slot == a.stages) { c.slot = 0; c.phase ^= 1; }
 }
 
 // ---- resampling ----------------------------------------------------------------------------------
@@ -663,7 +540,7 @@ struct Smem {
     uint32_t dbuf;      // two chunk-record buffers of TILED_DESC_BUF_BYTES
     uint32_t ov;        // BAND tiles: overlay descriptors of the chunk being processed (MCS_BAND_MAX_OVERLAYS slabs),
                         // behind them its full barrier (+0) and its empty barrier (+8)
-    SchedMem* issuer;   // chunk ids claimed by the scheduler
+    SchedMem* sched;    // chunk ids claimed by the producer
 };
 
 // Start the copy of the record of chunk e = {tile, frame block, first frame, end frame} into buffer b, and
@@ -689,21 +566,74 @@ __device__ __forceinline__ void prefetch_chunk(const TiledArgs& a, const Smem& s
     }
 }
 
+// The producer: one thread, lane 0 of the first warp behind the resampling warps.  Per chunk in claim order
+// it issues the chunk's boxes, one per frame (BAND tiles: one per layer involved and frame, the owner's first
+// unless the tile is zero-base), each as soon as its slot is released; in between it starts the copy of the
+// NEXT chunk's record once every warp is done with the buffer, and waits for that buffer only when all boxes
+// of the chunk are out.  Both waits are deadlock-free: a warp that holds a slot or a record buffer is in a
+// chunk whose boxes and record are already on their way.  tests/test_producer_protocol.py restates this.
+template <bool BANDS>
+__device__ __forceinline__ void produce(const TiledArgs& a, const Smem& sm) {
+    SchedMem* const q = sm.sched;
+    Sched c{0, 0, 0, 0u};
+    sched_ensure(a, q, c, 1);
+    if (q->chunk[0].x >= 0) prefetch_chunk(a, sm, 0, q->chunk[0]);
+    int slot = 0;
+    uint32_t phase = 0;
+    for (int k = 0;; ++k) {
+        sched_ensure(a, q, c, k + 2);
+        const int4 e = q->chunk[k % TILED_QD];
+        if (e.x < 0) break;
+        // the record of chunk k + 1 (published: e is not the end marker) still has to be copied; its buffer last
+        // held chunk k - 1 (none for k == 0)
+        bool rec_todo = q->chunk[(k + 1) % TILED_QD].x >= 0;
+        const uint32_t rel = sm.dbar + 16 + 8 * ((k + 1) & 1), rel_par = (uint32_t)(((k - 1) >> 1) & 1);
+        if (e.x < a.class_first[MCS_N_CLASSES - 1]) {   // ZERO chunks stage nothing
+            // the box records are re-read per box (L1 hits) rather than held in the producer's 32 registers
+            const int w = __ldg(&a.issue[e.x].w);
+            const int nl = BANDS ? 1 + ((w >> 24) & 15) : 1, li0 = BANDS ? (w >> 28) & 1 : 0;
+            const int frame0 = e.y * a.frame_block;
+            for (int f = e.z; f < e.w; ++f) {
+                for (int li = li0; li < nl; ++li) {
+                    int4 r = __ldg(BANDS && li > 0 ? a.band_issue + e.x * (1 + MCS_BAND_MAX_OVERLAYS) + li : a.issue + e.x);
+                    if (!(BANDS && li > 0)) r.w &= 0xffffff;
+                    if (rec_todo && (k == 0 || mbar_test(rel, rel_par))) {
+                        prefetch_chunk(a, sm, (k + 1) & 1, q->chunk[(k + 1) % TILED_QD]);
+                        rec_todo = false;
+                    }
+                    mbar_wait(sm.empty + 8 * slot, phase ^ 1, __LINE__);   // first trip round the ring: passes at once
+                    mbar_expect_tx(sm.full + 8 * slot, (uint32_t)r.w);
+                    tma_load_3d(sm.base + slot * a.box_bytes, &a.tmap[r.x], r.y, r.z, frame0 + f, sm.full + 8 * slot);
+                    if (++slot == a.stages) { slot = 0; phase ^= 1; }
+                }
+            }
+        }
+        if (rec_todo) {
+            if (k >= 1) mbar_wait(rel, rel_par, __LINE__);
+            prefetch_chunk(a, sm, (k + 1) & 1, q->chunk[(k + 1) % TILED_QD]);
+        }
+    }
+    // every CTA ends on a claim past the last chunk; the last CTA out rewinds the counters for the next launch
+    __threadfence();
+    if (atomicAdd(a.work + 1, 1u) == gridDim.x - 1) {
+        a.work[0] = 0u;
+        a.work[1] = 0u;
+        __threadfence();
+    }
+}
+
 // The n_fr frames of one WARP chunk for one warp: per frame wait for the staged box, resample
 // this thread's (up to) 8 pixels into the warp's two staging rows, release the box, stream the
 // rows out.  `groups` has bit j set when pixel group j of this warp (row j>>2, columns
 // 32*(j&3) .. +31) contains owned pixels; it is warp-uniform.  frame = first output frame,
 // g_row0 = frame offset of column 0 of cell row `warp`.
-// ISS: this warp is warp 0, whose lane 0 is the scheduler / box issuer.  The role is a template parameter so
-// that the other seven warps carry no trace of the issuer in their frame loop (as a per-frame test it cost every
-// warp a dozen instructions and two branch resolutions per frame, 10 % of all stall samples).
 // BAND: the tile blends with n_ov outer layers (feather mode): after the owner's pixels are staged, each overlay
 // box is waited for in turn and the pixels its descriptors mark (sm.ov, slab o; box pitch ov_sp[o]) are resampled
 // from it and blended into the staged values - value = (a * value + (F - a) * sample + F/2) >> feather_log2 -
 // before the rows go out.
-template <int C, int SP, bool ISS, bool BAND, bool BANDS>
+template <int C, int SP, bool BAND>
 __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d)[8], uint32_t groups, uint32_t sp,
-                                            const Smem& sm, RingPos& ring, Issuer& issuer, int k_cons, uint8_t* frame,
+                                            const Smem& sm, RingPos& ring, uint8_t* frame,
                                             uint32_t g_row0, int n_fr, int c0, int nbytes, int h, int warp,
                                             int lane, int n_ov = 0, uint32_t ov_sp0 = 0, uint32_t ov_sp1 = 0,
                                             bool zero_base = false) {
@@ -738,7 +668,6 @@ __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d
     bool ragged = __any_sync(0xffffffffu, r0.do_byte || r1.do_byte);
 
     for (int i = 0; i < n_fr; ++i, frame += a.dst_frame_stride) {
-        if (ISS && lane == 0) issuer_step<BANDS, BAND>(a, sm.issuer, issuer, k_cons, ring.n, sm.base, sm.full, sm.empty);
         if (phase_moves && i != 0) {
             ph0 = ((uint32_t)reinterpret_cast<uintptr_t>(frame) + g_row0) & 15u;
             ph1 = ((uint32_t)reinterpret_cast<uintptr_t>(frame) + g_row1) & 15u;
@@ -808,7 +737,6 @@ __device__ __forceinline__ void warp_frames(const TiledArgs& a, const PxDesc (&d
             const uint32_t F = 1u << a.feather_log2;
 #pragma unroll 1
             for (int o = 0; o < n_ov; ++o) {
-                if (ISS && lane == 0) issuer_step<BANDS, BAND>(a, sm.issuer, issuer, k_cons, ring.n, sm.base, sm.full, sm.empty);
                 mbar_wait(sm.full + 8 * ring.slot, ring.phase, __LINE__);
                 const uint32_t obox = order_after_wait(sm.base + ring.slot * a.box_bytes);
                 const uint32_t osp = o == 0 ? ov_sp0 : ov_sp1;
@@ -945,10 +873,10 @@ __device__ __forceinline__ GenDesc expand_gen(uint2 e, int lane) {
 
 // The n_fr frames of one FAST chunk for one warp (the group-path counterpart of warp_frames).  The
 // caller passes single frames when the rows' 16-byte phase differs from frame to frame.
-template <int SP, bool ISS, bool BANDS>
+template <int SP>
 __device__ __forceinline__ void fast_frames(const TiledArgs& a, const GroupDesc& g0, const GroupDesc& g1,
                                             const GenDesc (&gen)[MCS_FAST_MAX_PASSES], int n_pass, uint32_t sp,
-                                            const Smem& sm, RingPos& ring, Issuer& issuer, int k_cons, uint8_t* frame,
+                                            const Smem& sm, RingPos& ring, uint8_t* frame,
                                             uint32_t g_row0, int n_fr, int c0, int nbytes, int h, int warp,
                                             int lane) {
     constexpr int C = 3;
@@ -972,7 +900,6 @@ __device__ __forceinline__ void fast_frames(const TiledArgs& a, const GroupDesc&
         ragged = __any_sync(0xffffffffu, r0.do_byte || r1.do_byte);
     }
     for (int i = 0; i < n_fr; ++i, frame += a.dst_frame_stride) {
-        if (ISS && lane == 0) issuer_step<BANDS, false>(a, sm.issuer, issuer, k_cons, ring.n, sm.base, sm.full, sm.empty);
         mbar_wait(sm.full + 8 * ring.slot, ring.phase, __LINE__);
         const uint32_t box = order_after_wait(sm.base + ring.slot * a.box_bytes);
         {
@@ -1008,10 +935,10 @@ __device__ __forceinline__ void fast_frames(const TiledArgs& a, const GroupDesc&
 }
 
 template <int C, bool BANDS>
-__global__ void __launch_bounds__(TILED_THREADS, TILED_MIN_CTAS)
+__global__ void __launch_bounds__(TILED_CTA_THREADS, TILED_MIN_CTAS)
 mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
     constexpr int OUT_PITCH = MCS_CELL_W * C + 16;
-    // layout: [ring of `stages` boxes][full barriers][empty barriers][issuer cursor][chunk-record barriers]
+    // layout: [ring of `stages` boxes][full barriers][empty barriers][chunk ids][chunk-record barriers]
     //         [staging 16 x OUT_PITCH][two chunk-record buffers][slack]
     // (slack: the unpredicated 16-byte loads of write_out start up to 15 + 127 C + 15 + 496 bytes
     // past the start of a staging row, i.e. up to ~1 KB past the start of the last row)
@@ -1020,19 +947,14 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
     sm.base = smem_u32(smem);
     sm.full = sm.base + stages * a.box_bytes;
     sm.empty = sm.full + 8 * TILED_MAX_STAGES;
-    sm.issuer = reinterpret_cast<SchedMem*>(smem + stages * a.box_bytes + 16 * TILED_MAX_STAGES);
+    sm.sched = reinterpret_cast<SchedMem*>(smem + stages * a.box_bytes + 16 * TILED_MAX_STAGES);
     sm.dbar = sm.empty + 8 * TILED_MAX_STAGES + TILED_SCHED_BYTES;
     sm.out = sm.dbar + 64;
     sm.dbuf = (sm.out + MCS_CELL_H * OUT_PITCH + 15u) & ~15u;
     sm.ov = sm.dbuf + 2 * TILED_DESC_BUF_BYTES + 1024;   // behind the slack of the write-out loads
-    // keep the shared-window addresses in registers: left alone, the compiler rematerialises them
-    // in the frame loop from SR_CgaCtaId and the kernel parameters
-    asm volatile("" : "+r"(sm.base), "+r"(sm.full), "+r"(sm.empty), "+r"(sm.out));
-
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    Issuer issuer;
-    issuer_init(sm.issuer, issuer, tid == 0);
     if (tid == 0) {
+        sm.sched->published = 0;
         for (int s = 0; s < stages; ++s) {
             mbar_init(sm.full + 8 * s, 1);
             mbar_init(sm.empty + 8 * s, TILED_WARPS);
@@ -1050,35 +972,24 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
     }
     __syncthreads();
 
-    if (tid == 0) {
-        // the first chunks, the record of the very first one, the first boxes
-        sched_ensure(a, sm.issuer, issuer, 2);
-        const int4 e0 = sm.issuer->chunk[0];
-        if (e0.x >= 0) prefetch_chunk(a, sm, 0, e0);
-        // (BAND-aware: the prologue may enter chunk 0 whatever it is, but not run ahead into a BAND chunk 1 - the
-        // consumers will drive chunk 0 with the calls of ITS frame loop)
-        for (int i = 0; i < stages - TILED_LOOKAHEAD_SLACK; ++i)
-            issuer_step<BANDS, BANDS>(a, sm.issuer, issuer, BANDS ? -1 : 0, -1, sm.base, sm.full, sm.empty);
+    if (warp >= TILED_WARPS) {   // the producer warpgroup
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(TILED_PRODUCER_REGS));
+        if (tid == TILED_THREADS) produce<BANDS>(a, sm);
+        return;
     }
+    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(TILED_CONSUMER_REGS));
+    // keep the shared-window addresses in registers: left alone, the compiler rematerialises them
+    // in the frame loop from SR_CgaCtaId and the kernel parameters
+    asm volatile("" : "+r"(sm.base), "+r"(sm.full), "+r"(sm.empty), "+r"(sm.out));
 
     RingPos ring{0, 0u, 0};
     if (BANDS && lane == 0) sts32(sm.ov + a.ov_bytes + 16 + 4 * warp, 0u);   // BAND chunks this warp has processed (phase of the overlay buffer's barriers; own warp only)
-    const uint32_t s_published = smem_u32(&sm.issuer->published), s_ids = smem_u32(&sm.issuer->chunk[0]);
+    const uint32_t s_published = smem_u32(&sm.sched->published), s_ids = smem_u32(&sm.sched->chunk[0]);
     for (int k_cons = 0;; ++k_cons) {
-        // ---- chunk record: start the copy of the next chunk's, wait for this chunk's ----
+        // ---- chunk record: wait for this chunk's ----
         const int cb = k_cons & 1;
         const uint32_t rec = sm.dbuf + cb * TILED_DESC_BUF_BYTES;
         const uint32_t rec_release = sm.dbar + 16 + 8 * cb;
-        if (tid == 0) {
-            sched_ensure(a, sm.issuer, issuer, k_cons + 2);
-            int4 e2 = make_int4(-1, 0, 0, 0);
-            if (k_cons + 1 < issuer.claimed) e2 = sm.issuer->chunk[(k_cons + 1) % TILED_QD];
-            if (e2.x >= 0) {
-                // buffer cb ^ 1 held chunk k_cons - 1: every warp has copied what it needs out of it
-                if (k_cons >= 1) mbar_wait(sm.dbar + 16 + 8 * (cb ^ 1), (uint32_t)(((k_cons - 1) >> 1) & 1), __LINE__);
-                prefetch_chunk(a, sm, cb ^ 1, e2);
-            }
-        }
         {
 #ifdef TILED_DEBUG_HANG
             unsigned spins = 0;
@@ -1125,7 +1036,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             uint8_t* frame = frame0;
             RowOut r0, r1;
             for (int i = 0; i < n_fr; ++i, frame += a.dst_frame_stride) {
-                if (warp == 0 && lane == 0) issuer_step<BANDS, false>(a, sm.issuer, issuer, k_cons, ring.n, sm.base, sm.full, sm.empty);
                 if (i == 0 || phase_moves) {
                     const uint32_t fp = (uint32_t)reinterpret_cast<uintptr_t>(frame);
                     r0 = row_split(0, g_first0, (fp + g_first0) & 15u, warp < h, nbytes, lane);
@@ -1150,7 +1060,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             RowOut r0, r1;
             bool ragged = false;
             for (int i = 0; i < n_fr; ++i, frame += a.dst_frame_stride) {
-                if (warp == 0 && lane == 0) issuer_step<BANDS, false>(a, sm.issuer, issuer, k_cons, ring.n, sm.base, sm.full, sm.empty);
                 if (i == 0 || phase_moves) {
                     const uint32_t fp = (uint32_t)reinterpret_cast<uintptr_t>(frame);
                     r0 = row_split(s_off + warp * sp, g_first0, (fp + g_first0) & 15u, warp < h, nbytes, lane);
@@ -1191,11 +1100,6 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             const int4 r1 = __ldg(a.band_issue + id * (1 + MCS_BAND_MAX_OVERLAYS) + 2);
             ov_sp0 = (uint32_t)a.layer_sp[r0.x];
             ov_sp1 = r1.x >= 0 ? (uint32_t)a.layer_sp[r1.x] : 0u;
-            // the issuer does not look ahead into a BAND chunk from an ordinary one: refill the ring now, while the
-            // overlay descriptors are on their way (every call returns at once when the ring is full)
-            if (tid == 0)
-                for (int i = 0; i < stages - TILED_LOOKAHEAD_SLACK; ++i)
-                    issuer_step<BANDS, BANDS>(a, sm.issuer, issuer, k_cons, ring.n, sm.base, sm.full, sm.empty);
             mbar_wait(ov_full, (uint32_t)(band_seq & 1), __LINE__);
             __syncwarp();
             if (lane == 0) sts32(ov_full + 16 + 4 * warp, (uint32_t)(band_seq + 1));
@@ -1218,15 +1122,11 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
             const GroupDesc g0 = expand_group(w0), g1 = expand_group(w1);
             // one call per frame when the frame stride moves the rows' 16-byte phase
             const int n_call = phase_moves ? n_fr : 1, fr_call = phase_moves ? 1 : n_fr;
-#define MCS_FAST_FRAMES(SP_, ISS_)                                                                                  \
+#define MCS_FAST_FRAMES(SP_)                                                                                        \
     for (int q = 0; q < n_call; ++q)                                                                                  \
-        fast_frames<SP_, ISS_, BANDS>(a, g0, g1, gen, n_pass, sp, sm, ring, issuer, k_cons,                                 \
-                               frame0 + (long long)q * a.dst_frame_stride, g_row0, fr_call, c0, nbytes, h, warp, lane)
-            if (warp == 0) {
-                if (sp == 512) MCS_FAST_FRAMES(512, true); else MCS_FAST_FRAMES(0, true);
-            } else {
-                if (sp == 512) MCS_FAST_FRAMES(512, false); else MCS_FAST_FRAMES(0, false);
-            }
+        fast_frames<SP_>(a, g0, g1, gen, n_pass, sp, sm, ring, frame0 + (long long)q * a.dst_frame_stride, g_row0,     \
+                         fr_call, c0, nbytes, h, warp, lane)
+            if (sp == 512) MCS_FAST_FRAMES(512); else MCS_FAST_FRAMES(0);
 #undef MCS_FAST_FRAMES
             continue;
         }
@@ -1251,28 +1151,17 @@ mcs_stitch_tiled_kernel(const __grid_constant__ TiledArgs a) {
         }
         // the common box pitch of this channel count at compile time (128 columns at about unit scale), any other at run time
         constexpr int SP_MAIN = C == 1 ? 256 : C == 3 ? 512 : 640;
-#define MCS_WARP_FRAMES(SP_, ISS_, BAND_)                                                                           \
-    warp_frames<C, SP_, ISS_, BAND_, BANDS>(a, d, groups, sp, sm, ring, issuer, k_cons, frame0, g_row0, n_fr, c0, nbytes, h, \
-                                     warp, lane, n_ov, ov_sp0, ov_sp1, zero_base)
+#define MCS_WARP_FRAMES(SP_, BAND_)                                                                                 \
+    warp_frames<C, SP_, BAND_>(a, d, groups, sp, sm, ring, frame0, g_row0, n_fr, c0, nbytes, h, warp, lane, n_ov,     \
+                               ov_sp0, ov_sp1, zero_base)
         if (BANDS && tile.cls == MCS_TILE_BAND) {
-            if (warp == 0) MCS_WARP_FRAMES(0, true, BANDS); else MCS_WARP_FRAMES(0, false, BANDS);
+            MCS_WARP_FRAMES(0, BANDS);
             __syncwarp();
             if (lane == 0) mbar_arrive(sm.ov + a.ov_bytes + 8);   // done with the overlay descriptors
-        } else if (warp == 0) {
-            if (sp == SP_MAIN) MCS_WARP_FRAMES(SP_MAIN, true, false); else MCS_WARP_FRAMES(0, true, false);
         } else {
-            if (sp == SP_MAIN) MCS_WARP_FRAMES(SP_MAIN, false, false); else MCS_WARP_FRAMES(0, false, false);
+            if (sp == SP_MAIN) MCS_WARP_FRAMES(SP_MAIN, false); else MCS_WARP_FRAMES(0, false);
         }
 #undef MCS_WARP_FRAMES
-    }
-    // every CTA ends on a claim past the last chunk; the last CTA out rewinds the counters for the next launch
-    if (tid == 0) {
-        __threadfence();
-        if (atomicAdd(a.work + 1, 1u) == gridDim.x - 1) {
-            a.work[0] = 0u;
-            a.work[1] = 0u;
-            __threadfence();
-        }
     }
 }
 
@@ -1406,7 +1295,7 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
         int per_sm = 0, n_sm = 0, dev = 0;
         MCS_CHECK_CUDA(cudaGetDevice(&dev));
         MCS_CHECK_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
-        MCS_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, TILED_THREADS, smem));
+        MCS_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, TILED_CTA_THREADS, smem));
         if (per_sm < 1) {
             mcs_set_error("mcs_stitch_u8: tiled kernel does not fit (smem %zu bytes)", smem);
             return MCS_ERR_UNSUPPORTED;
@@ -1434,9 +1323,8 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
         const char* env = getenv("MCS_TILED_SPLIT");   // tests: split factor (0 / 1 = no split)
         if (env) a.split = atoi(env) > 1 && fb >= atoi(env) ? atoi(env) : 1;
     }
-    // A last frame block shorter than the split factor would cut its split tiles into chunks WITHOUT frames.  The box
-    // issuer spends one of its calls on stepping over such a chunk and its consumers make none in it, so every one of
-    // them eats a unit of look-ahead for good (tests/test_issuer_protocol.py shows the hang that ends in): no split then.
+    // A last frame block shorter than the split factor would cut its split tiles into chunks WITHOUT frames, each a
+    // claim and a record copy for no work: no split then.
     if (a.split > 1 && a.nf_last < a.split) a.split = 1;
     a.split_first = a.split > 1 ? (a.split_end > split_tiles ? a.split_end - split_tiles : 0) : a.split_end;
     a.chunks_per_block = plan->n_tiles + (a.split_end - a.split_first) * (a.split - 1);
@@ -1456,7 +1344,7 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
     }
     a.n_chunks = a.n_blocks * a.chunks_per_block;
     // chunks per claim: short chunks (few frames per launch) are claimed several at a time, so that a claim - one
-    // atomic round trip of the scheduler thread - covers about 32 units of work, but never so many that the
+    // atomic round trip of the producer thread - covers about 32 units of work, but never so many that the
     // CTAs could not all be served
     {
         int claim = 32 / fb;
@@ -1477,7 +1365,7 @@ int mcs_launch_tiled(mcs_plan* plan, const uint8_t* const* src, const int64_t* p
     // output rows: every output row of every frame must start on a 4-byte boundary
     a.use_fast = plan->d_fast != nullptr && (reinterpret_cast<uintptr_t>(dst) & 3) == 0 && (dst_pitch & 3) == 0 &&
                  (n_frames == 1 || (dst_frame_stride & 3) == 0);
-    kern<<<(unsigned)grid, TILED_THREADS, smem, stream>>>(a);
+    kern<<<(unsigned)grid, TILED_CTA_THREADS, smem, stream>>>(a);
     mcs_count_launch(1);
     MCS_CHECK_CUDA(cudaGetLastError());
     return MCS_OK;
